@@ -26,8 +26,14 @@ the one-profile-at-a-time order of the reference's query loop is timed beside it
 tables compared byte for byte (search.checks.hits_identical_to_1gpu); at N = 1 the GPU search of the CPU-baseline prefix
 is compared with the CPU-oracle pipeline's table field by field (search.checks.hits_identical_to_cpu_prefix, rule in
 search.checks.cpu_prefix_rule; byte identity per profile beside it).
+
+--steps sets the timed steps of the Forward legs and the timed passes of the search.  --dump-outputs DIR writes what the last of
+them computed: fs_fwd_scores / fs_fwd_status (one value per window) and search_hits_<profile> (one row per hit of the merged list,
+columns SEARCH_HIT_FIELDS).  Every input is generated from a fixed seed, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -39,6 +45,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the benchmark writes nothing in the tree it runs from (no __pycache__ either)
 
 HMM_FILE = os.path.join(ROOT, "tests", "golden", "tRNA-synthetases.bhmm")
 HMM_INDEX = 1
@@ -62,7 +69,38 @@ def parse_args():
     ap.add_argument("--contexts-per-gpu", type=int, default=0,
                     help="device contexts per profile and GPU in the search leg (0: 4 on one or two GPUs, 2 on four, 1 on eight -- the three "
                          "profiles run at the same time and every context has a host thread of its own: 12-24 of them in all)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (Forward scores and status per window, the search's hit lists) to "
+                         "DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs: use it with --impl ours")
+    return args
+
+
+# ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 << 20             # all files of --dump-outputs together stay under 64 MB, .npy headers included
+SEARCH_HIT_FIELDS = ("seqidx", "strand", "ali_from", "ali_to", "env_from", "env_to", "sq_len", "hmm_from", "hmm_to", "evalue", "lnP",
+                     "score", "bias", "pre_score", "envsc", "oasc", "pid", "shifts", "stops", "trace_len")
+
+
+def dump_arrays(outdir, arrays, budget):
+    """Writes each array of {name: array} as outdir/<name>.npy (float32 stays float32, everything else becomes float64, exact for the
+    integers written here).  An array larger than `budget` bytes is cut to a sample of its rows -- the same rows for arrays of the same
+    length, drawn from a fixed seed -- whose row numbers go to <name>_rows.npy."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        row_bytes = a.itemsize * (a.size // max(len(a), 1))
+        if a.nbytes > budget:
+            keep = budget // (row_bytes + 8)
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            a = a[rows]
+            np.save(os.path.join(outdir, name + "_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(outdir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -83,8 +121,13 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.index), f"--query-gpu={self.Q}",
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(self._kill)            # a run that fails before stop() leaves no sampler running
         except Exception:
             self.proc = None
+
+    def _kill(self):
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.kill()
 
     def stop(self):
         out = {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
@@ -351,11 +394,12 @@ def recovered(hits_per_model, contigs, plants):
     return found
 
 
-def search_leg(devices, per_gpu, mbp, cpu_mbp, with_cpu):
+def search_leg(devices, per_gpu, mbp, cpu_mbp, with_cpu, steps):
     """BASELINE.json's second metric on rank 0: bathsearch --fs end to end (ORF translation, MSV/bias/Viterbi/Forward filters, DNA
     windows, frameshift Forward/Backward, domain definition, rescoring, merged hit list) through the host pipeline
     (bath_b200/host/pipeline.cpp) and the C ABI, host buffers in, hit records out, for each of the three profiles.  Mbp/s = target
-    nucleotides x profiles (one strand counted, both searched) / wall seconds."""
+    nucleotides x profiles (one strand counted, both searched) / wall seconds of one of `steps` timed passes.  Returns the JSON
+    record and the hit lists of the last timed pass, one per profile."""
     from bath_b200 import capi, hostapi
     models, contigs, plants = search_target(mbp)
     pinned = []
@@ -373,7 +417,7 @@ def search_leg(devices, per_gpu, mbp, cpu_mbp, with_cpu):
     cold = time.perf_counter() - t0
     run_search_together(models, pinned, sets)                  # second untimed pass: with the searches running at the same time, buffers change hands between passes
     passes = []
-    for _ in range(3):                                         # three timed passes; the metric is the target searched three times / their total time
+    for _ in range(steps):                                     # --steps timed passes; the metric is the target searched that often / their total time
         dt_k, tables, stats, hits = run_search_together(models, pinned, sets)
         passes.append(dt_k)
     dt = sum(passes) / len(passes)
@@ -427,7 +471,7 @@ def search_leg(devices, per_gpu, mbp, cpu_mbp, with_cpu):
     for cs in sets:
         for c in cs:
             c.close()
-    return out
+    return out, hits
 
 
 def search_leg_cpu(mbp, nthreads, target_mbp):
@@ -577,6 +621,10 @@ def main():
     wall_ms = (time.perf_counter() - t_wall0) * 1e3
     dev_ms = max_over_ranks(dev_ms)
     sc_dev, st_dev = ctx.fetch_scores(nwin)
+    dump_budget = DUMP_BYTES // (2 * world + len(SEARCH_MODELS))          # per file: every rank's two, rank 0's hit lists
+    if args.dump_outputs:
+        sfx = f"_rank{rank}" if world > 1 else ""
+        dump_arrays(args.dump_outputs, {"fs_fwd_scores" + sfx: sc_dev, "fs_fwd_status" + sfx: st_dev.astype(np.float32)}, dump_budget)
 
     # ---- end to end through the C ABI with host buffers -------------------------------------
     sc = capi.pinned_array((nwin,), np.float32)
@@ -640,7 +688,11 @@ def main():
         devices = ranks.search_devices(rank, world, torch.cuda.device_count())
         if devices:
             per_gpu = args.contexts_per_gpu if args.contexts_per_gpu > 0 else max(1, min(4, 8 // len(devices)))
-            search = search_leg(devices, per_gpu, args.search_mbp, args.search_cpu_mbp, world == 1 and not args.no_cpu_baseline)
+            search, hits = search_leg(devices, per_gpu, args.search_mbp, args.search_cpu_mbp, world == 1 and not args.no_cpu_baseline,
+                                      args.steps)
+            if args.dump_outputs:                                 # one row per hit in the merged list, columns SEARCH_HIT_FIELDS
+                dump_arrays(args.dump_outputs, {f"search_hits_{k}": np.array([[h[f] for f in SEARCH_HIT_FIELDS] for h in hk], np.float64)
+                                                .reshape(-1, len(SEARCH_HIT_FIELDS)) for k, hk in zip(SEARCH_MODELS, hits)}, dump_budget)
         cpu_barrier()
 
     if rank != 0:

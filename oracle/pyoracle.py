@@ -6,6 +6,7 @@ cpu_baseline / --impl reference legs of bench.py.  The product never imports it.
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -102,17 +103,23 @@ def build(force=False):
     return so
 
 
-def build_native():
-    """Host-tuned build (-O3 -march=native) for the CPU-baseline legs of bench.py; built on the box that runs it."""
-    subprocess.check_call(["make", "-s", "-B", "-C", _HERE, "native"])   # -B: never trust a copy built on another host
-    return os.path.join(_HERE, "liboracle_native.so")
+def build_native(outdir):
+    """Host-tuned build (-O3 -march=native) for the CPU-baseline legs of bench.py; built on the box that runs it, into outdir
+    (bench.py writes nothing in the source tree, which may be read-only)."""
+    so = os.path.join(outdir, "liboracle_native.so")
+    subprocess.check_call(["make", "-s", "-B", "-C", _HERE, "native", f"NATIVE={so}"])   # -B: never trust a copy built on another host
+    return so
 
 
 def lib(native=False):
     global _LIB
     if _LIB is not None:
         return _LIB
-    L = C.CDLL(build_native() if native else build())
+    if native:
+        with tempfile.TemporaryDirectory(prefix="bath_oracle_native_") as d:
+            L = C.CDLL(build_native(d))          # the loaded mapping outlives the file
+    else:
+        L = C.CDLL(build())
     P = C.POINTER
     u8p, fp = P(C.c_uint8), P(C.c_float)
     sig = {
