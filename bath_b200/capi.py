@@ -22,7 +22,7 @@ EXPORTS = [
     "bathgpu_orfs_msv_screen", "bathgpu_orfs_fetch", "bathgpu_revcomp_slot", "bathgpu_fs_fwd_block", "bathgpu_fs_forward_matrices",
     "bathgpu_bias_forward", "bathgpu_orfs_stage_breakdown", "bathgpu_measure_int16_peak", "bathgpu_orf_forward_matrices",
     "bathgpu_packed4_bytes", "bathgpu_pack_dna4", "bathgpu_upload_block_packed4", "bathgpu_fs_fwd_block_packed4",
-    "bathgpu_upload_block_segments",
+    "bathgpu_upload_block_segments", "bathgpu_load_fs_profile_set", "bathgpu_fs_set_scores",
 ]
 
 
@@ -33,6 +33,7 @@ class Window(C.Structure):
 Envelope = Window
 
 window_dtype = np.dtype([("start", "<i8"), ("L", "<i4"), ("pmove", "<f4"), ("ploop", "<f4")], align=True)
+set_window_dtype = np.dtype([("start", "<i8"), ("L", "<i4"), ("pmove", "<f4"), ("ploop", "<f4"), ("profile", "<i4")], align=True)
 trace_dtype = np.dtype([("i", "<i4"), ("k", "<i2"), ("st", "u1"), ("c", "u1"), ("pp", "<f4")], align=True)
 domain_dtype = np.dtype([("envsc", "<f4"), ("bcksc", "<f4"), ("oasc", "<f4"), ("status", "<i4"),
                          ("trace_offset", "<i4"), ("trace_len", "<i4"), ("null2", "<f4", (KP,))], align=True)
@@ -156,6 +157,10 @@ def load():
     L.bathgpu_orfs_stage_breakdown.argtypes = [vp, fp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     L.bathgpu_bias_forward.restype = C.c_int
     L.bathgpu_bias_forward.argtypes = [vp, C.c_int, vp, C.c_int, fp, C.c_int, C.c_float, C.c_float, C.POINTER(C.c_uint8), fp]
+    L.bathgpu_load_fs_profile_set.restype = C.c_int
+    L.bathgpu_load_fs_profile_set.argtypes = [vp, C.c_int, C.c_int, ip, ip, C.POINTER(fp), C.POINTER(fp)]
+    L.bathgpu_fs_set_scores.restype = C.c_int
+    L.bathgpu_fs_set_scores.argtypes = [vp, C.c_int, vp, C.c_int, fp, fp, ip]
     L.bathgpu_host_alloc.restype = vp
     L.bathgpu_host_alloc.argtypes = [C.c_size_t]
     L.bathgpu_host_free.restype = None
@@ -234,6 +239,37 @@ class Context:
         nrows, ld = rfv.shape
         assert tfv.shape == (8, ld)
         self._check(self.lib.bathgpu_load_fs_profile(self.h, which, ld - 1, nrows, _f(rfv), _f(tfv)))
+
+    def load_fs_profile_set(self, which, profiles):
+        """bathgpu_load_fs_profile_set: profiles = [(rfv [nrows][M+1], tfv [8][M+1]), ...] of one codon length"""
+        rf = [np.ascontiguousarray(r, dtype=np.float32) for r, _ in profiles]
+        tf = [np.ascontiguousarray(t, dtype=np.float32) for _, t in profiles]
+        n = len(rf)
+        assert all(t.shape == (8, r.shape[1]) for r, t in zip(rf, tf))
+        M = np.array([r.shape[1] - 1 for r in rf], np.int32)
+        nrows = np.array([r.shape[0] for r in rf], np.int32)
+        fp = C.POINTER(C.c_float)
+        self._check(self.lib.bathgpu_load_fs_profile_set(self.h, which, n, _i(M), _i(nrows), (fp * n)(*[_f(r) for r in rf]),
+                                                         (fp * n)(*[_f(t) for t in tf])))
+
+    @staticmethod
+    def make_set_windows(starts, lengths, profiles, nj=1.0):
+        """bathgpu_set_window descriptors: make_windows' length model, window w scored with profile profiles[w] of the set"""
+        w = np.zeros(len(starts), dtype=set_window_dtype)
+        base = Context.make_windows(starts, lengths, nj)
+        for f in ("start", "L", "pmove", "ploop"):
+            w[f] = base[f]
+        w["profile"] = profiles
+        return w
+
+    def fs_set_scores(self, which, wins, xfE):
+        """bathgpu_fs_set_scores over the loaded set of this codon length: xfE [n_profiles][2]; returns (scores, status)"""
+        wins = np.ascontiguousarray(wins, set_window_dtype)
+        n = len(wins)
+        sc, st = np.empty(n, np.float32), np.empty(n, np.int32)
+        xf = np.ascontiguousarray(xfE, np.float32)
+        self._check(self.lib.bathgpu_fs_set_scores(self.h, which, wins.ctypes.data, n, _f(xf), _f(sc), _i(st)))
+        return sc, st
 
     def select_slot(self, slot):
         self._check(self.lib.bathgpu_select_slot(self.h, slot))

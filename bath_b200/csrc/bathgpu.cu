@@ -87,6 +87,14 @@ struct FsProfileImage {
   bool  loaded = false;
 };
 
+// bathgpu_load_fs_profile_set: n profile images of one codon length in one device block, beside the context's own profile
+struct FsProfileSet {
+  int n = 0;
+  std::vector<int> J, scan_steps, mw_scan_steps;     // per profile: what picks the kernel (bathgpu_fs_set_scores groups by it)
+  std::vector<FsSetProfile> table;                   // device pointers into arena; tEM / tEL are set per call
+  DevBuf arena, dtable, dwins, dwprof, dsc, dst, dcounter;
+};
+
 }  // namespace
 
 struct TargetSlot {          // one resident target: packed DNA + codon classes + survivor residues (e.g. one strand of one chunk of the target)
@@ -106,6 +114,7 @@ struct bathgpu_ctx {
   cudaEvent_t   sync_ev = nullptr;                    // blocking-sync event: a host thread waiting for its stream sleeps instead of spinning
   std::string   err;
   FsProfileImage fs3, fs5;
+  FsProfileSet  set3, set5;
   std::vector<std::unique_ptr<TargetSlot>> slot;      // grows on demand (bathgpu_select_slot)
   int           cur = 0;
   TargetSlot   &S() { return *slot[cur]; }
@@ -399,7 +408,24 @@ static inline int perm_index(int kk, int J)   // position of node k=kk+1 inside 
   return (j / VEC) * (32 * VEC) + lane * VEC + (j % VEC);
 }
 
-extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int nrows, const float *rfv, const float *tfv)
+namespace {
+enum { tBM = 0, tMM, tIM, tDM, tMD, tMI, tII, tDD };
+
+// What every device image of a profile is folded with (all in double, rounded once):
+//   s(k) = tBM(k-1): entry odds of node k.  The kernels carry V(k)/s(k), so s(k) must be positive
+//          (true for every local-mode profile: occ(k) > 0, src/modelconfig.c:90-97).
+//   Z(k) = 1 + tMD(k) * sum_{k'>k} prod_{m=k+1}^{k'-1} tDD(m): E(i) = sum_k M(i,k) Z(k).
+struct Fold {
+  int M = 0, J = 0, mpad = 0, ld = 0;
+  const float *tfv = nullptr;
+  std::vector<double> sK, zK;
+  // per-node transition odds, source-node indexed; zero beyond M
+  double T(int t, int k) const { return (k >= 0 && k <= M) ? (double)tfv[(size_t)t * ld + k] : 0.0; }
+};
+}  // namespace
+
+// The argument checks of bathgpu_load_fs_profile and the folding constants of one profile.  f.J is set once the arguments passed.
+static int fold_profile(bathgpu_ctx *ctx, int which, int M, int nrows, const float *rfv, const float *tfv, Fold &f)
 {
   if (!ctx || !rfv || !tfv || M < 1) return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_load_fs_profile");
   if (which != 3 && which != 5)     return fail(ctx, BATHGPU_EINVAL, "codon_lengths must be 3 or 5");
@@ -407,22 +433,12 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
   if (nrows != want_rows)           return fail(ctx, BATHGPU_EINVAL, "nrows %d != %d for %d codon lengths", nrows, want_rows, which);
   const int J = choose_J(M);
   if (J == 0) return fail(ctx, BATHGPU_EINVAL, "model length %d exceeds the single-warp kernels' limit (%d)", M, 32 * 32);
-  CUDA_TRY(ctx, enter(ctx));
-
-  FsProfileImage &im = (which == 3) ? ctx->fs3 : ctx->fs5;
-  im.loaded = false;
-  im.which = which; im.M = M; im.nrows = nrows; im.J = J; im.mpad = 32 * J;
-  const int mpad = im.mpad, ld = M + 1;
-
-  // per-node transition odds, source-node indexed; zero beyond M
-  auto T = [&](int t, int k) -> double { return (k >= 0 && k <= M) ? (double)tfv[(size_t)t * ld + k] : 0.0; };
-  enum { tBM = 0, tMM, tIM, tDM, tMD, tMI, tII, tDD };
-
-  // Folding constants (all in double, rounded once):
-  //   s(k) = tBM(k-1): entry odds of node k.  The kernels carry V(k)/s(k), so s(k) must be positive
-  //          (true for every local-mode profile: occ(k) > 0, src/modelconfig.c:90-97).
-  //   Z(k) = 1 + tMD(k) * sum_{k'>k} prod_{m=k+1}^{k'-1} tDD(m): E(i) = sum_k M(i,k) Z(k).
-  std::vector<double> sK(mpad + 2, 1.0), zK(mpad + 2, 0.0), Tsum(mpad + 2, 0.0);
+  f.M = M; f.J = J; f.mpad = 32 * J; f.ld = M + 1; f.tfv = tfv;
+  const int mpad = f.mpad;
+  auto T = [&](int t, int k) -> double { return f.T(t, k); };
+  std::vector<double> &sK = f.sK, &zK = f.zK;
+  std::vector<double> Tsum(mpad + 2, 0.0);
+  sK.assign(mpad + 2, 1.0); zK.assign(mpad + 2, 0.0);
   for (int k = 1; k <= M; ++k) {
     sK[k] = T(tBM, k - 1);
     if (!(sK[k] > 0.0) || !std::isfinite(sK[k]))
@@ -430,16 +446,29 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
   }
   for (int k = M - 1; k >= 1; --k) Tsum[k] = 1.0 + T(tDD, k + 1) * Tsum[k + 1];
   for (int k = 1; k <= M; ++k) zK[k] = 1.0 + T(tMD, k) * Tsum[k];
+  return BATHGPU_OK;
+}
 
-  // emission table, permuted [c][J/VEC][lane][VEC], scaled by s(k) Z(k)
-  std::vector<float> emis((size_t)nrows * mpad, 0.0f);
+// emission table, permuted [c][J/VEC][lane][VEC], scaled by s(k) Z(k)
+static void emission_table(const Fold &f, int nrows, const float *rfv, std::vector<float> &emis)
+{
+  const int M = f.M, J = f.J, mpad = f.mpad, ld = f.ld;
+  emis.assign((size_t)nrows * mpad, 0.0f);
   for (int c = 0; c < nrows; ++c)
     for (int k = 1; k <= M; ++k)
-      emis[(size_t)c * mpad + perm_index(k - 1, J)] = (float)((double)rfv[(size_t)c * ld + k] * sK[k] * zK[k]);
+      emis[(size_t)c * mpad + perm_index(k - 1, J)] = (float)((double)rfv[(size_t)c * ld + k] * f.sK[k] * f.zK[k]);
+}
 
-  // ---- forward constants
+// The Forward parsers' table copy ef, lane constants cc, the multi-warp kernel's constants mw (3 codon lengths, J >= 16; else empty)
+// and the D->D scan steps they need
+static void forward3_tables(const Fold &f, int which, int nrows, const float *rfv, std::vector<float> &ef, std::vector<float> &cc,
+                            std::vector<float> &mw, int &scan_steps, int &mw_scan_steps)
+{
+  const int M = f.M, J = f.J, mpad = f.mpad, ld = f.ld;
+  const std::vector<double> &sK = f.sK, &zK = f.zK;
+  auto T = [&](int t, int k) -> double { return f.T(t, k); };
   {
-    std::vector<float> cc((size_t)(FC_COUNT * J + FL_COUNT) * 32, 0.0f);
+    cc.assign((size_t)(FC_COUNT * J + FL_COUNT) * 32, 0.0f);
     auto C = [&](int which_c, int j, int lane) -> float & { return cc[(size_t)(which_c * J + j) * 32 + lane]; };
     // Scaled forms of the Forward parsers (fs_parser.cuh, FwdConsts): the table copy they read carries mm(k) too, and the
     // delete and insert chains are divided by g(k) and hi(k) so that the match value enters every chain with coefficient 1.
@@ -455,13 +484,10 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
     // node 1 has no delete state (D(i,1) = 0): its dd and dm are 0, which also cancels whatever lane 0 is handed as inflow
     auto ddS = [&](int k) -> double { return (k >= 2 && k < M) ? gK(k) * T(tDD, k) / mdK(k) : 0.0; };
     std::vector<double> bfull(32, 1.0), bscaled(32, 1.0);
-    std::vector<float> ef((size_t)nrows * mpad, 0.0f);
+    ef.assign((size_t)nrows * mpad, 0.0f);
     for (int c = 0; c < nrows; ++c)
       for (int k = 1; k <= M; ++k)
         ef[(size_t)c * mpad + perm_index(k - 1, J)] = (float)((double)rfv[(size_t)c * ld + k] * sK[k] * zK[k] * mmK(k));
-    if (im.emis_fwd.reserve(ef.size() * sizeof(float)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
-    CUDA_TRY(ctx, cudaMemcpyAsync(im.emis_fwd.p, ef.data(), ef.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(ctx, wait_stream(ctx));
     for (int lane = 0; lane < 32; ++lane) {
       double pp = 1.0, ps = 1.0;
       for (int j = 0; j < J; ++j) {
@@ -481,7 +507,7 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
       bfull[lane] = pp; bscaled[lane] = ps;
     }
     std::vector<double> b(bfull), bs(bscaled);
-    im.scan_steps = 5;
+    scan_steps = 5;
     for (int s = 0; s < 5; ++s) {
       int d = 1 << s;
       std::vector<double> nb(b), nbs(bs);
@@ -493,14 +519,14 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
       bs.swap(nbs);
       // step s carries D in from 2^s lanes away with these multipliers: below 1e-9 everywhere it (and every later step) changes
       // nothing at float resolution -- the cut-off the reference's own D->D passes apply (fwdback_fs.c:415-453)
-      if (biggest < 1.0e-9 && im.scan_steps == 5) im.scan_steps = std::max(s, 2);
+      if (biggest < 1.0e-9 && scan_steps == 5) scan_steps = std::max(s, 2);
       b.swap(nb);
     }
     if (which == 3 && J >= 16) {
       // multi-warp Forward kernel (fs_parser_mw.cuh): JW nodes per lane, NW = J/JW warps, virtual lane v = 32 w + lane owns nodes
       // JW v + 1 .. JW v + JW
       const int JW = kMwNodesPerLane, NW = J / JW, VL = 32 * NW;
-      std::vector<float> mw((size_t)(5 * JW + 6) * VL + NW, 0.0f);
+      mw.assign((size_t)(5 * JW + 6) * VL + NW, 0.0f);
       std::vector<double> lp(VL, 1.0), lpfull(VL, 1.0);
       for (int v = 0; v < VL; ++v)
         for (int j = 0; j < JW; ++j) {
@@ -515,7 +541,7 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
           }
           lp[v] *= ddS(k); lpfull[v] *= T(tDD, k);
         }
-      im.mw_scan_steps = 3;
+      mw_scan_steps = 3;
       for (int w = 0; w < NW; ++w) {
         std::vector<double> bsw(lp.begin() + 32 * w, lp.begin() + 32 * w + 32), bw(lpfull.begin() + 32 * w, lpfull.begin() + 32 * w + 32);
         double q = 1.0;
@@ -533,14 +559,85 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
           bsw.swap(nbs); bw.swap(nb);
           if (biggest < 1.0e-9 && need == 5) need = std::max(s2, 3);
         }
-        im.mw_scan_steps = std::max(im.mw_scan_steps, need);
+        mw_scan_steps = std::max(mw_scan_steps, need);
       }
-      if (getenv("BATHGPU_FULL_SCAN")) im.mw_scan_steps = 5;
+      if (getenv("BATHGPU_FULL_SCAN")) mw_scan_steps = 5;
+    } else mw.clear();
+    if (getenv("BATHGPU_FULL_SCAN")) scan_steps = 5;
+  }
+}
+
+// the full-matrix 5-codon Forward lane constants (fs_domain.cuh, Fwd5Const)
+static void fs5_forward_consts(const Fold &f, std::vector<float> &cc)
+{
+  const int M = f.M, J = f.J;
+  const std::vector<double> &sK = f.sK, &zK = f.zK;
+  auto T = [&](int t, int k) -> double { return f.T(t, k); };
+  cc.assign((size_t)(F5_COUNT * J + 5) * 32, 0.0f);
+  auto C = [&](int which_c, int j, int lane) -> float & { return cc[(size_t)(which_c * J + j) * 32 + lane]; };
+  std::vector<double> bfull(32, 1.0);
+  for (int lane = 0; lane < 32; ++lane) {
+    double pp = 1.0;
+    for (int j = 0; j < J; ++j) {
+      int k = lane * J + j + 1;
+      if (k <= M) {
+        double sn = sK[k + 1];
+        C(F5_MM, j, lane) = (float)(T(tMM, k) / (zK[k] * sn));
+        C(F5_IM, j, lane) = (float)(T(tIM, k) / sn);
+        C(F5_DM, j, lane) = (float)(T(tDM, k) / sn);
+        C(F5_MD, j, lane) = (float)(T(tMD, k) / zK[k]);
+        C(F5_DD, j, lane) = (float)T(tDD, k);
+        C(F5_MI, j, lane) = (float)(T(tMI, k) / zK[k]);
+        C(F5_II, j, lane) = (float)T(tII, k);
+      }
+      pp *= T(tDD, k);
+    }
+    bfull[lane] = pp;
+  }
+  std::vector<double> b(bfull);
+  for (int s = 0; s < 5; ++s) {
+    int d = 1 << s;
+    std::vector<double> nb(b);
+    for (int lane = 0; lane < 32; ++lane) {
+      cc[(size_t)(F5_COUNT * J + s) * 32 + lane] = (lane >= d) ? (float)b[lane] : 0.0f;
+      if (lane >= d) nb[lane] = b[lane] * b[lane - d];
+    }
+    b.swap(nb);
+  }
+}
+
+extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int nrows, const float *rfv, const float *tfv)
+{
+  Fold f;
+  const int fst = fold_profile(ctx, which, M, nrows, rfv, tfv, f);
+  if (fst != BATHGPU_OK) {
+    if (f.J) (which == 3 ? ctx->fs3 : ctx->fs5).loaded = false;      // a profile refused past the argument checks leaves no image behind
+    return fst;
+  }
+  CUDA_TRY(ctx, enter(ctx));
+
+  FsProfileImage &im = (which == 3) ? ctx->fs3 : ctx->fs5;
+  im.loaded = false;
+  const int J = f.J;
+  im.which = which; im.M = M; im.nrows = nrows; im.J = J; im.mpad = f.mpad;
+  const int mpad = im.mpad, ld = M + 1;
+  auto T = [&](int t, int k) -> double { return f.T(t, k); };
+  const std::vector<double> &sK = f.sK, &zK = f.zK;
+  std::vector<float> emis;
+  emission_table(f, nrows, rfv, emis);
+
+  // ---- forward constants
+  {
+    std::vector<float> ef, cc, mw;
+    forward3_tables(f, which, nrows, rfv, ef, cc, mw, im.scan_steps, im.mw_scan_steps);
+    if (im.emis_fwd.reserve(ef.size() * sizeof(float)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
+    CUDA_TRY(ctx, cudaMemcpyAsync(im.emis_fwd.p, ef.data(), ef.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, wait_stream(ctx));
+    if (!mw.empty()) {
       if (im.cellmw.reserve(mw.size() * sizeof(float)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
       CUDA_TRY(ctx, cudaMemcpyAsync(im.cellmw.p, mw.data(), mw.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
       CUDA_TRY(ctx, wait_stream(ctx));
     } else im.cellmw.release();
-    if (getenv("BATHGPU_FULL_SCAN")) im.scan_steps = 5;
     if (im.cellc.reserve(cc.size() * sizeof(float)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
     CUDA_TRY(ctx, cudaMemcpyAsync(im.cellc.p, cc.data(), cc.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(ctx, wait_stream(ctx));
@@ -678,37 +775,8 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
 
   // ---- full-matrix Forward constants, null2 amino rows, optimal-accuracy masks, raw transitions (fs_domain.cuh)
   {
-    std::vector<float> cc((size_t)(F5_COUNT * J + 5) * 32, 0.0f);
-    auto C = [&](int which_c, int j, int lane) -> float & { return cc[(size_t)(which_c * J + j) * 32 + lane]; };
-    std::vector<double> bfull(32, 1.0);
-    for (int lane = 0; lane < 32; ++lane) {
-      double pp = 1.0;
-      for (int j = 0; j < J; ++j) {
-        int k = lane * J + j + 1;
-        if (k <= M) {
-          double sn = sK[k + 1];
-          C(F5_MM, j, lane) = (float)(T(tMM, k) / (zK[k] * sn));
-          C(F5_IM, j, lane) = (float)(T(tIM, k) / sn);
-          C(F5_DM, j, lane) = (float)(T(tDM, k) / sn);
-          C(F5_MD, j, lane) = (float)(T(tMD, k) / zK[k]);
-          C(F5_DD, j, lane) = (float)T(tDD, k);
-          C(F5_MI, j, lane) = (float)(T(tMI, k) / zK[k]);
-          C(F5_II, j, lane) = (float)T(tII, k);
-        }
-        pp *= T(tDD, k);
-      }
-      bfull[lane] = pp;
-    }
-    std::vector<double> b(bfull);
-    for (int s = 0; s < 5; ++s) {
-      int d = 1 << s;
-      std::vector<double> nb(b);
-      for (int lane = 0; lane < 32; ++lane) {
-        cc[(size_t)(F5_COUNT * J + s) * 32 + lane] = (lane >= d) ? (float)b[lane] : 0.0f;
-        if (lane >= d) nb[lane] = b[lane] * b[lane - d];
-      }
-      b.swap(nb);
-    }
+    std::vector<float> cc;
+    fs5_forward_consts(f, cc);
     const int amino0 = nrows - BATHGPU_KP;
     std::vector<float> am((size_t)20 * mpad, 0.0f);
     for (int x = 0; x < 20; ++x)
@@ -1579,6 +1647,172 @@ extern "C" int bathgpu_fs_forward_matrices(bathgpu_ctx *ctx, const bathgpu_envel
     e0 = e1;
   }
   ctx->dom_L.clear(); ctx->dom_xoff.clear();           // the posterior matrices of the last bathgpu_fs_domains call are gone
+  return BATHGPU_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Profile sets: the frameshift Forward parsers over windows that each name their profile (the calibration of many models at once)
+extern "C" int bathgpu_load_fs_profile_set(bathgpu_ctx *ctx, int which, int n, const int *M, const int *nrows,
+                                           const float *const *rfv, const float *const *tfv)
+{
+  if (!ctx || n < 1 || !M || !nrows || !rfv || !tfv) return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_load_fs_profile_set");
+  if (which != 3 && which != 5) return fail(ctx, BATHGPU_EINVAL, "codon_lengths must be 3 or 5");
+  FsProfileSet &ps = (which == 3) ? ctx->set3 : ctx->set5;
+  ps.n = 0;
+  // every table starts on a 256-byte boundary of the block (the kernels read them with 16-byte vector loads)
+  std::vector<float> host;
+  std::vector<size_t> off_emis(n), off_cc(n), off_mw(n);
+  ps.J.assign(n, 0); ps.scan_steps.assign(n, 5); ps.mw_scan_steps.assign(n, 5);
+  std::vector<float> tab, cc, mw;
+  auto append = [&](const std::vector<float> &v) -> size_t {
+    const size_t at = (host.size() + 63) & ~(size_t)63;
+    host.resize(at + v.size(), 0.0f);
+    std::copy(v.begin(), v.end(), host.begin() + at);
+    return at;
+  };
+  for (int p = 0; p < n; ++p) {
+    Fold f;
+    const int st = fold_profile(ctx, which, M[p], nrows[p], rfv[p], tfv[p], f);
+    if (st != BATHGPU_OK) return fail(ctx, st, "profile %d of the set: %s", p, std::string(ctx->err).c_str());
+    if (which == 3) forward3_tables(f, 3, nrows[p], rfv[p], tab, cc, mw, ps.scan_steps[p], ps.mw_scan_steps[p]);
+    else { emission_table(f, nrows[p], rfv[p], tab); fs5_forward_consts(f, cc); mw.clear(); }
+    ps.J[p] = f.J;
+    off_emis[p] = append(tab);
+    off_cc[p] = append(cc);
+    off_mw[p] = mw.empty() ? (size_t)-1 : append(mw);
+  }
+  CUDA_TRY(ctx, enter(ctx));
+  if (ps.arena.reserve(host.size() * sizeof(float)) != BATHGPU_OK || ps.dtable.reserve((size_t)n * sizeof(FsSetProfile)) != BATHGPU_OK)
+    return fail(ctx, BATHGPU_EMEM, "device allocation failed for a set of %d profiles (%zu bytes)", n, host.size() * sizeof(float));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ps.arena.p, host.data(), host.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, wait_stream(ctx));
+  const float *base = ps.arena.as<float>();
+  ps.table.assign(n, FsSetProfile{});
+  for (int p = 0; p < n; ++p) {
+    ps.table[p].emis = base + off_emis[p];
+    ps.table[p].cellc = base + off_cc[p];
+    ps.table[p].cellmw = (off_mw[p] == (size_t)-1) ? nullptr : base + off_mw[p];
+  }
+  ps.n = n;
+#define X(S) preload_fwd_##S(ps.J[0]); preload_fs5_##S(ps.J[0]);
+  BATHGPU_FOR_EACH_SET(X)
+#undef X
+  return BATHGPU_OK;
+}
+
+static cudaError_t dispatch_fwd_set(int J, const FsParserArgs &a, int sms, cudaStream_t s)
+{
+  cudaError_t e = cudaErrorInvalidValue;
+  const int v = fwd_version(J);
+#define X(S) if (launch_fs3_forward_set_##S(J, v, a, sms, s, &e)) return e;
+  BATHGPU_FOR_EACH_SET(X)
+#undef X
+  return cudaErrorInvalidValue;
+}
+
+static cudaError_t dispatch_fs5_set(int J, const DomainArgs &a, int sms, cudaStream_t s)
+{
+  cudaError_t e = cudaErrorInvalidValue;
+#define X(S) if (launch_fs5_forward_set_##S(J, a, sms, s, &e)) return e;
+  BATHGPU_FOR_EACH_SET(X)
+#undef X
+  return cudaErrorInvalidValue;
+}
+
+extern "C" int bathgpu_fs_set_scores(bathgpu_ctx *ctx, int which, const bathgpu_set_window *wins, int n, const float *xfE,
+                                     float *fwdsc, int32_t *status)
+{
+  if (!ctx || !wins || n < 1 || !xfE || !fwdsc || !status) return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_fs_set_scores");
+  if (which != 3 && which != 5) return fail(ctx, BATHGPU_EINVAL, "codon_lengths must be 3 or 5");
+  FsProfileSet &ps = (which == 3) ? ctx->set3 : ctx->set5;
+  if (ps.n < 1)              return fail(ctx, BATHGPU_EINVAL, "no %d-codon profile set loaded", which);
+  if (ctx->S().block_n == 0) return fail(ctx, BATHGPU_EINVAL, "no block uploaded");
+  const int minL = (which == 3) ? 3 : 6;
+  for (int w = 0; w < n; ++w) {
+    if (wins[w].profile < 0 || wins[w].profile >= ps.n)
+      return fail(ctx, BATHGPU_EINVAL, "window %d names profile %d of a set of %d", w, wins[w].profile, ps.n);
+    if (wins[w].L < minL || wins[w].start < 1 || wins[w].start + wins[w].L - 1 > ctx->S().block_n)
+      return fail(ctx, BATHGPU_EINVAL, "window %d (start %lld, L %d) is outside the uploaded block (n=%lld) or shorter than %d",
+                  w, (long long)wins[w].start, wins[w].L, (long long)ctx->S().block_n, minL);
+  }
+  CUDA_TRY(ctx, enter(ctx));
+  // one launch per kernel the single-profile dispatch would pick: node count per lane J and, on the 3-codon side, the D->D scan
+  // steps the kernel is instantiated for; windows of one profile stay together and in call order
+  auto key = [&](int p) -> long long { return which == 3 ? ((long long)ps.J[p] * 8 + ps.scan_steps[p]) * 8 + ps.mw_scan_steps[p] : ps.J[p]; };
+  std::vector<int> order(n);
+  for (int w = 0; w < n; ++w) order[w] = w;
+  std::stable_sort(order.begin(), order.end(), [&](int x, int y) {
+    const int px = wins[x].profile, py = wins[y].profile;
+    const long long kx = key(px), ky = key(py);
+    return kx != ky ? kx < ky : px < py;
+  });
+  static_assert(sizeof(WindowDesc) == sizeof(EnvelopeDesc), "descriptor layouts must agree");
+  std::vector<WindowDesc> hw(n);
+  std::vector<int> hp(n), grp;
+  for (int z = 0; z < n; ++z) {
+    const bathgpu_set_window &sw = wins[order[z]];
+    hw[z].start = sw.start; hw[z].L = sw.L; hw[z].pmove = sw.pmove; hw[z].ploop = sw.ploop;
+    hp[z] = sw.profile;
+    if (z == 0 || key(hp[z]) != key(hp[z - 1])) grp.push_back(z);
+  }
+  const int ng = (int)grp.size();
+  grp.push_back(n);
+  std::vector<FsSetProfile> table(ps.table);
+  for (int p = 0; p < ps.n; ++p) { table[p].tEM = xfE[2 * p]; table[p].tEL = xfE[2 * p + 1]; }
+  if (ps.dwins.reserve((size_t)n * sizeof(WindowDesc)) != BATHGPU_OK || ps.dwprof.reserve((size_t)n * 4) != BATHGPU_OK ||
+      ps.dsc.reserve((size_t)n * 4) != BATHGPU_OK || ps.dst.reserve((size_t)n * 4) != BATHGPU_OK ||
+      ps.dcounter.reserve((size_t)ng * 4) != BATHGPU_OK)
+    return fail(ctx, BATHGPU_EMEM, "device allocation failed");
+  CUDA_TRY(ctx, cudaMemcpyAsync(ps.dwins.p, hw.data(), (size_t)n * sizeof(WindowDesc), cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ps.dwprof.p, hp.data(), (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ps.dtable.p, table.data(), (size_t)ps.n * sizeof(FsSetProfile), cudaMemcpyHostToDevice, ctx->stream));
+  if (which == 5) {
+    // The 5-codon kernel writes every row of its matrix (rows nobody reads here): windows take turns in a ring of scratch matrices
+    // as large as the matrix budget allows; two windows that share a slot at the same time only overwrite each other's unread rows.
+    int maxL = 0, maxJ = 0;
+    for (int z = 0; z < n; ++z) { maxL = std::max(maxL, hw[z].L); maxJ = std::max(maxJ, ps.J[hp[z]]); }
+    const size_t rows_per = (size_t)maxL + 1, mpad = (size_t)32 * maxJ;
+    const size_t slots = std::max<size_t>(1, std::min<size_t>((size_t)n, matrix_budget() / 10 * 7 / (rows_per * kPPCells * mpad * 4)));
+    const size_t rows = slots * rows_per;
+    std::vector<long long> xo(n);
+    for (int z = 0; z < n; ++z) xo[z] = (long long)((size_t)z % slots * rows_per);
+    if (ctx->xoff.reserve((size_t)n * 8) != BATHGPU_OK || reserve_matrices(ctx, rows * kPPCells * mpad * 4, 0) != BATHGPU_OK ||
+        ctx->ddcell.reserve(rows * mpad * 4) != BATHGPU_OK || ctx->dfx.reserve(rows * 24) != BATHGPU_OK || ctx->dlsf.reserve(rows * 4) != BATHGPU_OK)
+      return fail(ctx, BATHGPU_EMEM, "device allocation failed");
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->xoff.p, xo.data(), (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  CUDA_TRY(ctx, cudaMemsetAsync(ps.dcounter.p, 0, (size_t)ng * 4, ctx->stream));
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  const int sms = ctx->prop.multiProcessorCount;
+  for (int g = 0; g < ng; ++g) {
+    const int b = grp[g], e = grp[g + 1], p0 = hp[b], J = ps.J[p0];
+    if (which == 3) {
+      FsParserArgs a{};
+      a.dna4 = ctx->S().dna4.as<uint32_t>(); a.wins = ps.dwins.as<WindowDesc>() + b; a.nwin = e - b; a.mpad = 32 * J;
+      a.fwdsc = ps.dsc.as<float>() + b; a.status = ps.dst.as<int>() + b; a.counter = ps.dcounter.as<int>() + g;
+      a.scan_steps = ps.scan_steps[p0]; a.mw_scan_steps = ps.mw_scan_steps[p0]; a.cellmw = table[p0].cellmw;
+      a.set = ps.dtable.as<FsSetProfile>(); a.wprof = ps.dwprof.as<int>() + b;
+      CUDA_TRY(ctx, dispatch_fwd_set(J, a, sms, ctx->stream));
+    } else {
+      DomainArgs a{};
+      a.dna4 = ctx->S().dna4.as<uint32_t>(); a.envs = ps.dwins.as<EnvelopeDesc>() + b; a.nenv = e - b; a.mpad = 32 * J;
+      a.fwdsc = ps.dsc.as<float>() + b; a.status = ps.dst.as<int>() + b; a.counter = ps.dcounter.as<int>() + g;
+      a.set = ps.dtable.as<FsSetProfile>(); a.wprof = ps.dwprof.as<int>() + b;
+      a.xoff = ctx->xoff.as<long long>() + b; a.pp = ctx->dpp.as<float>(); a.dcell = ctx->ddcell.as<float>(); a.fx = ctx->dfx.as<float>();
+      a.lsf = ctx->dlsf.as<float>();
+      CUDA_TRY(ctx, dispatch_fs5_set(J, a, sms, ctx->stream));
+    }
+  }
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  std::vector<float> sc(n);
+  std::vector<int> st(n);
+  CUDA_TRY(ctx, cudaMemcpyAsync(sc.data(), ps.dsc.p, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(st.data(), ps.dst.p, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, wait_stream(ctx));
+  for (int z = 0; z < n; ++z) { fwdsc[order[z]] = sc[z]; status[order[z]] = st[z]; }
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
+  ctx->last_launches = ng;
+  if (which == 5) { ctx->dom_L.clear(); ctx->dom_xoff.clear(); }        // the posterior matrices of the last bathgpu_fs_domains call are gone
   return BATHGPU_OK;
 }
 

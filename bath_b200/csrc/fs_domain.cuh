@@ -71,6 +71,8 @@ struct DomainArgs {
   float          *null2;       // [nenv][29]
   int            *status;      // [nenv]
   int            *counter;
+  const FsSetProfile *set;     // fs5_forward_kernel<J, true, true>: envelope e is scored with profile set[wprof[e]] (emis, cellf, tEM, tEL unused)
+  const int      *wprof;
 };
 
 template <int J, int VEC>
@@ -284,14 +286,22 @@ __device__ __forceinline__ void load_fwd5_consts(const float *__restrict__ cc, i
   for (int s = 0; s < 5; ++s) K.bs[s] = __ldg(cc + F5_COUNT * J * kWarp + s * kWarp + lane);
 }
 
-template <int J, bool STORE_D = false>
+// SET: the envelopes of a profile set (DomainArgs::set); constants and table re-read whenever a warp's next envelope has another
+// profile.  Everything else is the kernel bathgpu_fs_forward_matrices runs, stores included: a copy that skips them is compiled
+// into other floating-point contractions and misses the scores-only call's results by an ulp.
+template <int J, bool STORE_D = false, bool SET = false>
 __global__ void __launch_bounds__(32) fs5_forward_kernel(DomainArgs a)
 {
   constexpr int VEC = VecOf<J>::V;
   const int lane = threadIdx.x & 31;
   Fwd5Consts<J> K;
-  load_fwd5_consts<J>(a.cellf, lane, K);
-  const char    *emis_lane = reinterpret_cast<const char *>(a.emis + lane * VEC);
+  const char    *emis_lane = nullptr;
+  float          tEM = a.tEM, tEL = a.tEL;
+  int            cur = -1;
+  if constexpr (!SET) {
+    load_fwd5_consts<J>(a.cellf, lane, K);
+    emis_lane = reinterpret_cast<const char *>(a.emis + lane * VEC);
+  }
   const unsigned rowbytes  = (unsigned)a.mpad * 4u;
 
   for (;;) {
@@ -299,10 +309,20 @@ __global__ void __launch_bounds__(32) fs5_forward_kernel(DomainArgs a)
     if (lane == 0) e = atomicAdd(a.counter, 1);
     e = __shfl_sync(0xffffffffu, e, 0);
     if (e >= a.nenv) break;
+    if constexpr (SET) {
+      const int p = a.wprof[e];
+      if (p != cur) {
+        cur = p;
+        const FsSetProfile sp = a.set[p];
+        load_fwd5_consts<J>(sp.cellc, lane, K);
+        emis_lane = reinterpret_cast<const char *>(sp.emis + lane * VEC);
+        tEM = sp.tEM; tEL = sp.tEL;
+      }
+    }
     const EnvelopeDesc ed = a.envs[e];
     const int L = ed.L;
     Fwd5Ctx R;
-    R.L = L; R.ploop = ed.ploop; R.pmove = ed.pmove; R.tEL = a.tEL; R.tEM = a.tEM; R.totscale = 0.f; R.lsf = 0.f;
+    R.L = L; R.ploop = ed.ploop; R.pmove = ed.pmove; R.tEL = tEL; R.tEM = tEM; R.totscale = 0.f; R.lsf = 0.f;
     const long long xo = a.xoff[e];
     float *pprow_lane = a.pp + (size_t)xo * kPPCells * a.mpad + lane * VEC;
     float *fxrow = a.fx + (size_t)xo * 6;

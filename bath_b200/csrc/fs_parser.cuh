@@ -42,6 +42,15 @@ struct WindowDesc {      // device copy of bathgpu_window
   float     ploop;
 };
 
+// One profile of a resident profile set (bathgpu_load_fs_profile_set): the pointers a kernel otherwise takes from its arguments,
+// read per window in the kernels' SET instantiations.  Every profile of one launch has the same node count per lane J.
+struct FsSetProfile {
+  const float *emis;           // the table the kernel reads: emis_fwd (3 codon lengths) or emis (5)
+  const float *cellc;          // lane constants: cellc (3) or cellf5 (5)
+  const float *cellmw;         // multi-warp Forward constants (3, J >= 16), else null
+  float        tEM, tEL;       // E->MOVE, E->LOOP odds of this profile
+};
+
 struct FsParserArgs {
   const float    *emis;        // [nrows][mpad] permuted odds table (3-codon profile)
   const float    *cellc;       // lane-constant image
@@ -58,6 +67,8 @@ struct FsParserArgs {
   int             scan_steps;  // steps of the D->D warp scan this profile needs (5 = all; fewer when the D->D odds products die out)
   const float    *cellmw;      // lane-constant image of the multi-warp kernel (fs_parser_mw.cuh); null for models the one-warp kernels keep in registers
   int             mw_scan_steps;
+  const FsSetProfile *set;     // SET instantiations: window w is scored with profile set[wprof[w]] (emis, cellc, cellmw, tEM, tEL unused)
+  const int      *wprof;
 };
 
 template <int J> struct VecOf { static constexpr int V = (J % 4 == 0) ? 4 : ((J % 2 == 0) ? 2 : 1); };

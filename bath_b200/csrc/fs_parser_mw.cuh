@@ -162,15 +162,10 @@ __device__ __forceinline__ void mw_row_pair(int i, int lane, int warp, FwdState<
 // JW nodes per lane, NW warps per window (32 NW JW >= M).  Resident blocks per SM the kernel is compiled for.
 template <int NW, int JW> struct MwTune { static constexpr int kBlocks = (JW == 8) ? ((NW == 4) ? 2 : (NW == 3) ? 2 : 4) : ((NW >= 5) ? 2 : 4); };
 
-template <int NW, int JW, bool XMX, int NS>
-__global__ void __launch_bounds__(32 * NW, MwTune<NW, JW>::kBlocks) fs3_forward_parser_kernel_mw(FsParserArgs a)
+template <int NW, int JW>
+__device__ __forceinline__ void mw_load_consts(const float *__restrict__ cc, int vl, FwdConsts<JW> &K, float &Q, float (&PW)[NW])
 {
-  __shared__ MwShared<NW> sh;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, vl = threadIdx.x;
   constexpr int VL = 32 * NW;
-
-  FwdConsts<JW> K;
-  const float *cc = a.cellmw;
 #pragma unroll
   for (int j = 0; j < JW; ++j) {
     K.qm[j] = __ldg(cc + (0 * JW + j) * VL + vl);
@@ -181,13 +176,30 @@ __global__ void __launch_bounds__(32 * NW, MwTune<NW, JW>::kBlocks) fs3_forward_
   }
 #pragma unroll
   for (int s = 0; s < 5; ++s) K.bs[s] = __ldg(cc + (5 * JW + s) * VL + vl);
-  const float Q = __ldg(cc + (5 * JW + 5) * VL + vl);
-  float PW[NW];
+  Q = __ldg(cc + (5 * JW + 5) * VL + vl);
 #pragma unroll
   for (int v = 0; v < NW; ++v) PW[v] = __ldg(cc + (5 * JW + 6) * VL + v);
+}
+
+// SET: as in fs3_forward_parser_kernel_v3 (the block's warps share one window, hence one profile)
+template <int NW, int JW, bool XMX, int NS, bool SET = false>
+__global__ void __launch_bounds__(32 * NW, MwTune<NW, JW>::kBlocks) fs3_forward_parser_kernel_mw(FsParserArgs a)
+{
+  __shared__ MwShared<NW> sh;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, vl = threadIdx.x;
+
+  FwdConsts<JW> K;
+  float Q;
+  float PW[NW];
   // this thread's JW nodes are JW/4 consecutive float4 chunks of real lane (JW vl) / (NW JW) of the one-warp table layout
   const int node0 = JW * vl, rl = node0 / (NW * JW), c0 = (node0 % (NW * JW)) / 4;
-  const char    *emis_lane = reinterpret_cast<const char *>(a.emis + ((size_t)c0 * 32 + rl) * 4);
+  const char    *emis_lane = nullptr;
+  float          tEM = a.tEM, tEL = a.tEL;
+  int            cur = -1;
+  if constexpr (!SET) {
+    mw_load_consts<NW, JW>(a.cellmw, vl, K, Q, PW);
+    emis_lane = reinterpret_cast<const char *>(a.emis + ((size_t)c0 * 32 + rl) * 4);
+  }
   const unsigned rowbytes  = (unsigned)a.mpad * 4u;
 
   for (;;) {
@@ -196,6 +208,16 @@ __global__ void __launch_bounds__(32 * NW, MwTune<NW, JW>::kBlocks) fs3_forward_
     const int w = sh.win;
     __syncthreads();
     if (w >= a.nwin) break;
+    if constexpr (SET) {
+      const int p = a.wprof[w];
+      if (p != cur) {
+        cur = p;
+        const FsSetProfile sp = a.set[p];
+        mw_load_consts<NW, JW>(sp.cellmw, vl, K, Q, PW);
+        emis_lane = reinterpret_cast<const char *>(sp.emis + ((size_t)c0 * 32 + rl) * 4);
+        tEM = sp.tEM; tEL = sp.tEL;
+      }
+    }
 
     const WindowDesc wd = a.wins[w];
     const int   L     = wd.L;
@@ -242,8 +264,8 @@ __global__ void __launch_bounds__(32 * NW, MwTune<NW, JW>::kBlocks) fs3_forward_
         const uint32_t src = (qq < 7) ? cwl : cwn;                                                                                \
         const uint32_t n0 = __shfl_sync(0xffffffffu, src, (qq * 4 + 4) & 31);                                                     \
         const uint32_t n1 = __shfl_sync(0xffffffffu, src, (qq * 4 + 5) & 31);                                                     \
-        mw_row_pair<NW, JW, 0, XMX, NS, HEAD_>(i, lane, warp, S, K, Q, PW, sh, emis_lane, rowbytes, TA, TB, c2, c3, true, ploop, pmove, a.tEL, a.tEM, totscale, xrow); i += 2; \
-        mw_row_pair<NW, JW, 2, XMX, NS, HEAD_>(i, lane, warp, S, K, Q, PW, sh, emis_lane, rowbytes, TA, TB, n0, n1, (qq + 1 < qn) || more, ploop, pmove, a.tEL, a.tEM, totscale, xrow); i += 2; \
+        mw_row_pair<NW, JW, 0, XMX, NS, HEAD_>(i, lane, warp, S, K, Q, PW, sh, emis_lane, rowbytes, TA, TB, c2, c3, true, ploop, pmove, tEL, tEM, totscale, xrow); i += 2; \
+        mw_row_pair<NW, JW, 2, XMX, NS, HEAD_>(i, lane, warp, S, K, Q, PW, sh, emis_lane, rowbytes, TA, TB, n0, n1, (qq + 1 < qn) || more, ploop, pmove, tEL, tEM, totscale, xrow); i += 2; \
       }                                                                                                                           \
       cwl = cwn;                                                                                                                  \
     }

@@ -220,15 +220,21 @@ __device__ __forceinline__ void fwd_row_pair(int i, int lane, FwdState<J> &S, co
 #define BATHGPU_V3_RESIDENT(J) 64
 #endif
 
-template <int J, bool XMX, int NS = 5>
+// SET: the windows of a profile set (FsParserArgs::set), constants and table re-read whenever a warp's next window has another profile
+template <int J, bool XMX, int NS = 5, bool SET = false>
 __global__ void __launch_bounds__(32, BATHGPU_V3_WARPS(J)) fs3_forward_parser_kernel_v3(FsParserArgs a)
 {
   constexpr int VEC = VecOf<J>::V;
   const int lane = threadIdx.x & 31;
 
   FwdConsts<J> K;
-  load_fwd_consts<J>(a.cellc, lane, K);
-  const char    *emis_lane = reinterpret_cast<const char *>(a.emis + lane * VEC);
+  const char    *emis_lane = nullptr;
+  float          tEM = a.tEM, tEL = a.tEL;
+  int            cur = -1;
+  if constexpr (!SET) {
+    load_fwd_consts<J>(a.cellc, lane, K);
+    emis_lane = reinterpret_cast<const char *>(a.emis + lane * VEC);
+  }
   const unsigned rowbytes  = (unsigned)a.mpad * 4u;
 
   for (;;) {
@@ -236,6 +242,16 @@ __global__ void __launch_bounds__(32, BATHGPU_V3_WARPS(J)) fs3_forward_parser_ke
     if (lane == 0) w = atomicAdd(a.counter, 1);
     w = __shfl_sync(0xffffffffu, w, 0);
     if (w >= a.nwin) break;
+    if constexpr (SET) {
+      const int p = a.wprof[w];
+      if (p != cur) {
+        cur = p;
+        const FsSetProfile sp = a.set[p];
+        load_fwd_consts<J>(sp.cellc, lane, K);
+        emis_lane = reinterpret_cast<const char *>(sp.emis + lane * VEC);
+        tEM = sp.tEM; tEL = sp.tEL;
+      }
+    }
 
     const WindowDesc wd = a.wins[w];
     const int   L     = wd.L;
@@ -270,8 +286,8 @@ __global__ void __launch_bounds__(32, BATHGPU_V3_WARPS(J)) fs3_forward_parser_ke
         const uint32_t c1 = __shfl_sync(0xffffffffu, cwl, qq * 4 + 1);                                                            \
         const uint32_t c2 = __shfl_sync(0xffffffffu, cwl, qq * 4 + 2);                                                            \
         const uint32_t c3 = __shfl_sync(0xffffffffu, cwl, qq * 4 + 3);                                                            \
-        fwd_row_pair<J, VEC, 0, XMX, NS, HEAD_>(i, lane, S, K, emis_lane, rowbytes, c0, c1, ploop, pmove, a.tEL, a.tEM, totscale, xrow); i += 2; \
-        fwd_row_pair<J, VEC, 2, XMX, NS, HEAD_>(i, lane, S, K, emis_lane, rowbytes, c2, c3, ploop, pmove, a.tEL, a.tEM, totscale, xrow); i += 2; \
+        fwd_row_pair<J, VEC, 0, XMX, NS, HEAD_>(i, lane, S, K, emis_lane, rowbytes, c0, c1, ploop, pmove, tEL, tEM, totscale, xrow); i += 2; \
+        fwd_row_pair<J, VEC, 2, XMX, NS, HEAD_>(i, lane, S, K, emis_lane, rowbytes, c2, c3, ploop, pmove, tEL, tEM, totscale, xrow); i += 2; \
       }                                                                                                                           \
     }
     int q0 = 0;

@@ -271,7 +271,8 @@ __device__ __forceinline__ void fwd4_row_pair(int i, int lane, FwdState4<J> &S, 
 #define BATHGPU_V4_WARPS(J) ((J) <= 2 ? 20 : (J) == 3 ? 18 : (J) == 4 ? 16 : (J) == 5 ? 14 : (J) == 6 ? 12 : (J) == 7 ? 10 : (J) == 8 ? 9 : 8)
 #endif
 
-template <int J, bool XMX, int NS = 5>
+// SET: as in fs3_forward_parser_kernel_v3
+template <int J, bool XMX, int NS = 5, bool SET = false>
 __global__ void __launch_bounds__(32, BATHGPU_V4_WARPS(J)) fs3_forward_parser_kernel_v4(FsParserArgs a)
 {
   constexpr int VEC = VecOf<J>::V;
@@ -279,8 +280,13 @@ __global__ void __launch_bounds__(32, BATHGPU_V4_WARPS(J)) fs3_forward_parser_ke
   const int lane = threadIdx.x & 31;
 
   FwdConsts4<J> K;
-  load_fwd_consts4<J>(a.cellc, lane, K);
-  const char    *emis_lane = reinterpret_cast<const char *>(a.emis + lane * VEC);
+  const char    *emis_lane = nullptr;
+  float          tEM = a.tEM, tEL = a.tEL;
+  int            cur = -1;
+  if constexpr (!SET) {
+    load_fwd_consts4<J>(a.cellc, lane, K);
+    emis_lane = reinterpret_cast<const char *>(a.emis + lane * VEC);
+  }
   const unsigned rowbytes  = (unsigned)a.mpad * 4u;
 
   for (;;) {
@@ -288,6 +294,16 @@ __global__ void __launch_bounds__(32, BATHGPU_V4_WARPS(J)) fs3_forward_parser_ke
     if (lane == 0) w = atomicAdd(a.counter, 1);
     w = __shfl_sync(0xffffffffu, w, 0);
     if (w >= a.nwin) break;
+    if constexpr (SET) {
+      const int p = a.wprof[w];
+      if (p != cur) {
+        cur = p;
+        const FsSetProfile sp = a.set[p];
+        load_fwd_consts4<J>(sp.cellc, lane, K);
+        emis_lane = reinterpret_cast<const char *>(sp.emis + lane * VEC);
+        tEM = sp.tEM; tEL = sp.tEL;
+      }
+    }
 
     const WindowDesc wd = a.wins[w];
     const int   L     = wd.L;
@@ -318,7 +334,7 @@ __global__ void __launch_bounds__(32, BATHGPU_V4_WARPS(J)) fs3_forward_parser_ke
         {                                                                                                                         \
           const uint32_t cA = __shfl_sync(0xffffffffu, cwl, bb * 12 + (R_));                                                      \
           const uint32_t cB = __shfl_sync(0xffffffffu, cwl, bb * 12 + (R_) + 1);                                                  \
-          fwd4_row_pair<J, VEC, (R_) & 3, (R_) % 3, XMX, NS, HEAD_>(i, lane, S, K, emis_lane, rowbytes, cA, cB, ploop, pmove, a.tEL, a.tEM, totscale, xemax, xrow); \
+          fwd4_row_pair<J, VEC, (R_) & 3, (R_) % 3, XMX, NS, HEAD_>(i, lane, S, K, emis_lane, rowbytes, cA, cB, ploop, pmove, tEL, tEM, totscale, xemax, xrow); \
           i += 2;                                                                                                                 \
         }
 #define BATHGPU_V4_CHUNK(HEAD_)                                                                                                   \

@@ -68,32 +68,43 @@ template <class K> static int fwd_grid(K kernel, int J, int n, int sms)
 
 // models past the one-warp kernels' register budget (J >= 16): J/8 warps per window (fs_parser_mw.cuh); BATHGPU_FWD_MW=0 keeps the
 // one-warp kernel for comparison
-template <int NW, int JW, bool XMX> static cudaError_t run_fwd_mw(const FsParserArgs &a, int sms, cudaStream_t s)
+template <int NW, int JW, bool XMX, bool SET = false> static cudaError_t run_fwd_mw(const FsParserArgs &a, int sms, cudaStream_t s)
 {
-  if (a.mw_scan_steps <= 3) fs3_forward_parser_kernel_mw<NW, JW, XMX, 3><<<grid_for(fs3_forward_parser_kernel_mw<NW, JW, XMX, 3>, 32 * NW, 0, a.nwin, sms), 32 * NW, 0, s>>>(a);
-  else                      fs3_forward_parser_kernel_mw<NW, JW, XMX, 5><<<grid_for(fs3_forward_parser_kernel_mw<NW, JW, XMX, 5>, 32 * NW, 0, a.nwin, sms), 32 * NW, 0, s>>>(a);
+  if (a.mw_scan_steps <= 3) fs3_forward_parser_kernel_mw<NW, JW, XMX, 3, SET><<<grid_for(fs3_forward_parser_kernel_mw<NW, JW, XMX, 3, SET>, 32 * NW, 0, a.nwin, sms), 32 * NW, 0, s>>>(a);
+  else                      fs3_forward_parser_kernel_mw<NW, JW, XMX, 5, SET><<<grid_for(fs3_forward_parser_kernel_mw<NW, JW, XMX, 5, SET>, 32 * NW, 0, a.nwin, sms), 32 * NW, 0, s>>>(a);
   return cudaGetLastError();
 }
 
-template <int J, bool XMX> static cudaError_t run_fwd(int version, const FsParserArgs &a, int sms, cudaStream_t s)
+// SET: the windows of a profile set (FsParserArgs::set); a.cellmw non-null when the set's profiles have multi-warp images
+template <int J, bool XMX, bool SET = false> static cudaError_t run_fwd(int version, const FsParserArgs &a, int sms, cudaStream_t s)
 {
   if constexpr (J >= 16) {
     // BATHGPU_FWD_MW: 0 never, 1 (default) from 24 nodes per lane up -- at 16 the one-warp kernel is still ahead (800 vs 620 GCUPS
     // at M = 409) --, 2 from 16 up
     static const int mw_mode = [] { const char *e = getenv("BATHGPU_FWD_MW"); return e ? atoi(e) : 1; }();
-    if (version >= 3 && a.cellmw && (mw_mode >= 2 || (mw_mode == 1 && J >= 24))) return run_fwd_mw<J / kMwNodesPerLane, kMwNodesPerLane, XMX>(a, sms, s);
+    if (version >= 3 && a.cellmw && (mw_mode >= 2 || (mw_mode == 1 && J >= 24))) return run_fwd_mw<J / kMwNodesPerLane, kMwNodesPerLane, XMX, SET>(a, sms, s);
   }
   if (version >= 4) {                 // packed-FP32 row pairs (fs_parser_v4.cuh)
-    if (a.scan_steps <= 2)      fs3_forward_parser_kernel_v4<J, XMX, 2><<<fwd_grid(fs3_forward_parser_kernel_v4<J, XMX, 2>, J, a.nwin, sms), 32, 0, s>>>(a);
-    else if (a.scan_steps == 3) fs3_forward_parser_kernel_v4<J, XMX, 3><<<fwd_grid(fs3_forward_parser_kernel_v4<J, XMX, 3>, J, a.nwin, sms), 32, 0, s>>>(a);
-    else                        fs3_forward_parser_kernel_v4<J, XMX, 5><<<fwd_grid(fs3_forward_parser_kernel_v4<J, XMX, 5>, J, a.nwin, sms), 32, 0, s>>>(a);
+    if (a.scan_steps <= 2)      fs3_forward_parser_kernel_v4<J, XMX, 2, SET><<<fwd_grid(fs3_forward_parser_kernel_v4<J, XMX, 2, SET>, J, a.nwin, sms), 32, 0, s>>>(a);
+    else if (a.scan_steps == 3) fs3_forward_parser_kernel_v4<J, XMX, 3, SET><<<fwd_grid(fs3_forward_parser_kernel_v4<J, XMX, 3, SET>, J, a.nwin, sms), 32, 0, s>>>(a);
+    else                        fs3_forward_parser_kernel_v4<J, XMX, 5, SET><<<fwd_grid(fs3_forward_parser_kernel_v4<J, XMX, 5, SET>, J, a.nwin, sms), 32, 0, s>>>(a);
   }
   else {                              // scalar row pairs (fs_parser_v3.cuh); the first-generation one-row kernel is gone
-    if (a.scan_steps <= 2)      fs3_forward_parser_kernel_v3<J, XMX, 2><<<fwd_grid(fs3_forward_parser_kernel_v3<J, XMX, 2>, J, a.nwin, sms), 32, 0, s>>>(a);
-    else if (a.scan_steps == 3) fs3_forward_parser_kernel_v3<J, XMX, 3><<<fwd_grid(fs3_forward_parser_kernel_v3<J, XMX, 3>, J, a.nwin, sms), 32, 0, s>>>(a);
-    else                        fs3_forward_parser_kernel_v3<J, XMX, 5><<<fwd_grid(fs3_forward_parser_kernel_v3<J, XMX, 5>, J, a.nwin, sms), 32, 0, s>>>(a);
+    if (a.scan_steps <= 2)      fs3_forward_parser_kernel_v3<J, XMX, 2, SET><<<fwd_grid(fs3_forward_parser_kernel_v3<J, XMX, 2, SET>, J, a.nwin, sms), 32, 0, s>>>(a);
+    else if (a.scan_steps == 3) fs3_forward_parser_kernel_v3<J, XMX, 3, SET><<<fwd_grid(fs3_forward_parser_kernel_v3<J, XMX, 3, SET>, J, a.nwin, sms), 32, 0, s>>>(a);
+    else                        fs3_forward_parser_kernel_v3<J, XMX, 5, SET><<<fwd_grid(fs3_forward_parser_kernel_v3<J, XMX, 5, SET>, J, a.nwin, sms), 32, 0, s>>>(a);
   }
   return cudaGetLastError();
+}
+// the Forward parser over the windows of a profile set: the kernel run_fwd picks for the set's J, scan steps and version
+bool CAT(launch_fs3_forward_set_, SETNAME)(int J, int version, const FsParserArgs &a, int sms, cudaStream_t s, cudaError_t *err)
+{
+  switch (J) {
+#define X(J_) case J_: *err = run_fwd<J_, false, true>(version, a, sms, s); return true;
+  JLIST(X)
+#undef X
+  default: return false;
+  }
 }
 bool CAT(launch_fs3_forward_, SETNAME)(int J, bool xmx, int version, const FsParserArgs &a, int sms, cudaStream_t s, cudaError_t *err)
 {
@@ -184,6 +195,17 @@ bool CAT(launch_fs5_forward_matrix_, SETNAME)(int J, const DomainArgs &a, int sm
   switch (J) {
 #define X(J_) case J_: if ((*err = cudaMemsetAsync(a.counter, 0, 4, s)) != cudaSuccess) return true;                               \
                        fs5_forward_kernel<J_, true><<<grid_for(fs5_forward_kernel<J_, true>, 32, 0, a.nenv, sms), 32, 0, s>>>(a);   \
+                       *err = cudaGetLastError(); return true;
+  JLIST(X)
+#undef X
+  default: return false;
+  }
+}
+// the scores of p7_ForwardParser_Frameshift_5Codons over the envelopes of a profile set (launch_fs5_forward_matrix's kernel)
+bool CAT(launch_fs5_forward_set_, SETNAME)(int J, const DomainArgs &a, int sms, cudaStream_t s, cudaError_t *err)
+{
+  switch (J) {
+#define X(J_) case J_: fs5_forward_kernel<J_, true, true><<<grid_for(fs5_forward_kernel<J_, true, true>, 32, 0, a.nenv, sms), 32, 0, s>>>(a); \
                        *err = cudaGetLastError(); return true;
   JLIST(X)
 #undef X

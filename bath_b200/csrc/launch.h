@@ -27,6 +27,8 @@ struct FilterArgs;
   bool launch_orf_domains_##S(int J, bool full, const OrfDomainArgs &a, const TraceArgs &t, int sms, cudaStream_t s, cudaError_t *err); \
   bool launch_orf_forward_matrix_##S(int J, const OrfDomainArgs &a, int sms, cudaStream_t s, cudaError_t *err);                            \
   bool launch_orf_forward_parser_##S(int J, const OrfFwdArgs &a, int sms, cudaStream_t s, cudaError_t *err);                        \
+  bool launch_fs3_forward_set_##S(int J, int version, const FsParserArgs &a, int sms, cudaStream_t s, cudaError_t *err);            \
+  bool launch_fs5_forward_set_##S(int J, const DomainArgs &a, int sms, cudaStream_t s, cudaError_t *err);                            \
   void preload_fwd_##S(int J); void preload_bck_##S(int J); void preload_fs5_##S(int J); void preload_orf_##S(int J);
 BATHGPU_FOR_EACH_SET(BATHGPU_DECLARE_SET)
 #undef BATHGPU_DECLARE_SET

@@ -103,6 +103,18 @@ double tau_of(const std::vector<double> &x, double lambda, double tailp)     // 
   return (gmu - log(-log(1.0 - tailp)) / glam) + log(tailp) / lambda;
 }
 
+// esl_rsq_xfIID of a random protein, reverse-translated with uniformly drawn synonymous codons (src/evalues.c:634-647): n sequences
+// of 3 L nucleotides, one after the other from dst
+void draw_reverse_translated(const bathhost_model *m, const CodonTable &tbl, FastRng &rng, int L, int n, uint8_t *dst)
+{
+  std::vector<uint8_t> amino(L);
+  for (int i = 0; i < n; ++i) {
+    for (int a = 0; a < L; ++a) amino[a] = (uint8_t) rng.choose(m->bg.f, kK);
+    uint8_t *d = dst + (size_t) i * 3 * L;
+    for (int a = 0; a < L; ++a, d += 3) memcpy(d, tbl.nt[amino[a]][rng.roll(tbl.n[amino[a]])], 3);
+  }
+}
+
 float null_one(int L)      { const float p1 = (float) L / (float) (L + 1); return (float) L * log(p1) + log(1. - p1); }      // p7_bg_SetLength + p7_bg_NullOne
 float fs_null_one(int La)  { return null_one(La) + log(3.0); }                                                               // p7_bg_fs_NullOne (src/p7_bg.c:377-384)
 
@@ -210,7 +222,7 @@ extern "C" int bathhost_calibrate(const bathhost_model *m, const bathhost_backen
   // the two frameshift simulations: random proteins reverse-translated with uniformly drawn synonymous codons
   // (src/evalues.c:634-647); the length model is set from the AMINO length (:628), null model p7_bg_fs_NullOne(EfL)
   const int Ln = 3 * EfL;
-  std::vector<uint8_t> dna, amino(EfL);
+  std::vector<uint8_t> dna;
   std::vector<bathgpu_window> wins;
   auto frameshift_simulation = [&](int which, bool run, double *tau) -> int {
     xv.clear();
@@ -221,11 +233,7 @@ extern "C" int bathhost_calibrate(const bathhost_model *m, const bathhost_backen
     while (need > 0) {
       if (++rounds > 64) return BATHHOST_EFAIL;             // every score overflows: the reference would draw for ever (:649)
       dna.assign((size_t) need * Ln + 2, 255);
-      for (int i = 0; i < need; ++i) {
-        for (int a = 0; a < EfL; ++a) amino[a] = (uint8_t) rng.choose(m->bg.f, kK);
-        uint8_t *d = &dna[1 + (size_t) i * Ln];
-        for (int a = 0; a < EfL; ++a, d += 3) memcpy(d, tbl.nt[amino[a]][rng.roll(tbl.n[amino[a]])], 3);
-      }
+      draw_reverse_translated(m, tbl, rng, EfL, need, &dna[1]);
       if (!run) return 0;
       if ((st = be->select_slot(be->ctx, 0)) != 0 || (st = be->upload_block(be->ctx, dna.data(), (int64_t) need * Ln)) != 0) return st;
       sc.assign(need, 0.0f); status.assign(need, 0);
@@ -255,4 +263,26 @@ extern "C" int bathhost_calibrate(const bathhost_model *m, const bathhost_backen
   if ((st = frameshift_simulation(5, mask & 16, &evparam[EV_FTAUFS5])) != 0) return st;
   cal->rng_state = rng.x;
   return BATHHOST_OK;
+}
+
+uint32_t bathhost::calibration_generator(uint32_t seed) { return FastRng(seed ? seed : 42u).x; }
+
+bool bathhost::draw_fs_sequences(const bathhost_model *m, uint32_t *state, int n, uint8_t *dna)
+{
+  uint8_t gcode[64];
+  if (!genetic_code(m->ct, gcode)) return false;
+  const CodonTable tbl(gcode);
+  FastRng rng(42u);
+  rng.x = *state;
+  draw_reverse_translated(m, tbl, rng, kFsSimL, n, dna);
+  *state = rng.x;
+  return true;
+}
+
+double bathhost::fs_tau(const float *sc, int n, double lambda)
+{
+  const float nullsc = fs_null_one(kFsSimL);
+  std::vector<double> xv(n);
+  for (int i = 0; i < n; ++i) xv[i] = (sc[i] - nullsc) / kLog2;
+  return tau_of(xv, lambda, 0.04);
 }

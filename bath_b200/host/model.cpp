@@ -602,6 +602,22 @@ static int open_nth(const char *path, int index, CoreModel &h)
   return st;
 }
 
+// everything after reading the core model: the query set-up of bathsearch (src/bathsearch.c:761-762, :794-801)
+static int setup_model(bathhost_model *m, int ct)
+{
+  m->maxl_in_file = m->hmm.max_length;
+  if (m->hmm.max_length == -1) m->hmm.max_length = builder_max_length(m->hmm, 1e-7);      // src/bathsearch.c:761-762
+  m->ct = (ct > 0) ? ct : (m->hmm.ct > 0 ? m->hmm.ct : 1);
+  uint8_t gcode[64];
+  if (!genetic_code(m->ct, gcode) || !(m->hmm.fsprob > 0.0f)) return BATHHOST_EINVAL;
+  m->gm3.configure(m->hmm, m->bg, gcode, 3);
+  m->gm5.configure(m->hmm, m->bg, gcode, 5);
+  m->om3.convert(m->gm3);
+  m->om5.convert(m->gm5);
+  m->prot.configure(m->hmm, m->bg, m->gm5, m->om5);
+  return BATHHOST_OK;
+}
+
 extern "C" int bathhost_model_read(const char *path, int index, int ct, bathhost_model **ret_model)
 {
   if (!path || index < 0 || !ret_model) return BATHHOST_EINVAL;
@@ -609,18 +625,27 @@ extern "C" int bathhost_model_read(const char *path, int index, int ct, bathhost
   bathhost_model *m = new (std::nothrow) bathhost_model();
   if (!m) return BATHHOST_EMEM;
   int st = open_nth(path, index, m->hmm);
+  if (st == BATHHOST_OK) st = setup_model(m, ct);
   if (st != BATHHOST_OK) { delete m; return st; }
-  m->maxl_in_file = m->hmm.max_length;
-  if (m->hmm.max_length == -1) m->hmm.max_length = builder_max_length(m->hmm, 1e-7);      // src/bathsearch.c:761-762
-  m->ct = (ct > 0) ? ct : (m->hmm.ct > 0 ? m->hmm.ct : 1);
-  uint8_t gcode[64];
-  if (!genetic_code(m->ct, gcode) || !(m->hmm.fsprob > 0.0f)) { delete m; return BATHHOST_EINVAL; }
-  m->gm3.configure(m->hmm, m->bg, gcode, 3);
-  m->gm5.configure(m->hmm, m->bg, gcode, 5);
-  m->om3.convert(m->gm3);
-  m->om5.convert(m->gm5);
-  m->prot.configure(m->hmm, m->bg, m->gm5, m->om5);
   *ret_model = m;
+  return BATHHOST_OK;
+}
+
+int bathhost::model_from_record(const std::string &text, int ct, float fsprob, bathhost_model **ret)
+{
+  *ret = nullptr;
+  bathhost_model *m = new (std::nothrow) bathhost_model();
+  if (!m) return BATHHOST_EMEM;
+  std::istringstream in(text);
+  int st = read_record(in, m->hmm);
+  if (st == BATHHOST_EOF) st = BATHHOST_EFORMAT;
+  if (st == BATHHOST_OK) {
+    m->hmm.ct = ct;
+    m->hmm.fsprob = fsprob;
+    st = setup_model(m, ct);
+  }
+  if (st != BATHHOST_OK) { delete m; return st; }
+  *ret = m;
   return BATHHOST_OK;
 }
 

@@ -18,6 +18,7 @@ EXPORTS = [
     "bathhost_sample_region_segments", "bathhost_cluster_region_segments", "bathhost_sample_region_segments_protein",
     "bathhost_cluster_region_segments_protein", "bathhost_search_format_tblout",
     "bathhost_calibrate", "bathhost_model_lambda", "bathhost_search_format_report", "bathhost_search_format_output", "bathhost_search_format_fstblout",
+    "bathhost_convert", "bathhost_convert_last_error",
 ]
 
 
@@ -37,7 +38,10 @@ class Backend(C.Structure):
     """bathhost_backend: the device library as a table of function pointers (include/bathhost.h)"""
     _names = ["last_error", "load_fs_profile", "load_filter_profile", "select_slot", "upload_block", "upload_orfs", "msv_orfs", "ssv_windows",
               "vit_orfs", "fwd_orfs", "fs_fwd_windows", "fs_fwd_bck_xrows", "fs_bck_decode", "fs_domains", "fs_forward_matrices", "orf_fwd_bck_xrows", "orf_domains", "orfs_msv_screen", "orfs_fetch", "revcomp_slot", "host_alloc", "host_free", "bias_forward", "orf_forward_matrices", "upload_block_segments"]
-    _fields_ = [("ctx", C.c_void_p)] + [(n, C.c_void_p) for n in _names]
+    # the optional pair at the end of the table: left NULL by a table that fills _names only (bathhost_convert then calibrates
+    # model by model)
+    _set_names = ["load_fs_profile_set", "fs_set_scores"]
+    _fields_ = [("ctx", C.c_void_p)] + [(n, C.c_void_p) for n in _names + _set_names]
 
 
 class Options(C.Structure):
@@ -147,6 +151,10 @@ def load():
     L.bathhost_calibrate.argtypes = [vp, C.POINTER(Backend), C.POINTER(Calibration), C.POINTER(C.c_double)]
     L.bathhost_model_lambda.restype = C.c_double
     L.bathhost_model_lambda.argtypes = [vp]
+    L.bathhost_convert.restype = C.c_int
+    L.bathhost_convert.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_float, C.c_uint32, C.POINTER(Backend), C.POINTER(C.c_int)]
+    L.bathhost_convert_last_error.restype = C.c_char_p
+    L.bathhost_convert_last_error.argtypes = []
     L.bathhost_length_model.restype = None
     L.bathhost_length_model.argtypes = [C.c_int, C.c_float, fp, fp]
     _lib = L
@@ -263,7 +271,7 @@ def backend_from(gpu_lib, ctx_handle):
     """bathhost_backend over a loaded libbathgpu.so (ctypes CDLL) and a bathgpu_ctx handle"""
     be = Backend()
     be.ctx = ctx_handle
-    for n in Backend._names:
+    for n in Backend._names + Backend._set_names:
         setattr(be, n, C.cast(getattr(gpu_lib, "bathgpu_" + n), C.c_void_p))
     return be
 
@@ -282,6 +290,29 @@ def calibrate(model, gpu_ctx=None, backend=None, seed=42, lam=0.0, which=31, con
     if st != OK:
         raise RuntimeError(f"bathhost_calibrate: status {st}")
     return [float(v) for v in out], int(cal.rng_state)
+
+
+class ConvertError(RuntimeError):
+    def __init__(self, code, msg):
+        super().__init__(f"bathhost_convert: status {code}: {msg}")
+        self.code = code
+
+
+def convert(in_path, out_path, gpu_ctx=None, backend=None, ct=1, fsprob=0.01, seed=42):
+    """A HMMER3/f profile library (hmmbuild output, any number of models) as a BATH3/f one that bathsearch reads: each model's
+    text with the FS3 / FS5 Forward taus bathconvert's calibration gives, FRAMESHIFT PROB and CODON TABLE added (see bathhost_convert
+    in include/bathhost.h).  Returns the number of models; raises ConvertError (code EFORMAT = 7 for input that is not HMMER3/f,
+    EINVAL = 11 for ct / fsprob) and leaves out_path unwritten on failure."""
+    lib = load()
+    if backend is None:
+        if gpu_ctx is None:
+            raise ValueError("a device context is required: the product has no CPU path")
+        backend = backend_from(gpu_ctx.lib, gpu_ctx.h)
+    n = C.c_int(0)
+    st = lib.bathhost_convert(os.fsencode(in_path), os.fsencode(out_path), int(ct), float(fsprob), int(seed), C.byref(backend), C.byref(n))
+    if st != OK:
+        raise ConvertError(st, lib.bathhost_convert_last_error().decode())
+    return int(n.value)
 
 
 class Search:

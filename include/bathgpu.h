@@ -245,6 +245,32 @@ int bathgpu_fs_domains(bathgpu_ctx *ctx, const bathgpu_envelope *envs, int n, co
 int bathgpu_fs_forward_matrices(bathgpu_ctx *ctx, const bathgpu_envelope *regs, int n, const float xfE5[2],
                                 float *mx, float *xrows, int64_t max_rows, float *fwdsc, int32_t *status);
 
+/* ---- the frameshift Forward parsers over a resident profile set (calibration of many models at once) ------------------ */
+/* The calibration runs p7_fs_Tau_3codons / p7_fs_Tau_5codons once per model (src/evalues.c:607-680, :703-776; 200 windows of
+ * 300 nt each): a model alone fills a fraction of the device.  These two calls score the windows of MANY profiles in one launch
+ * per kernel.
+ * bathgpu_load_fs_profile_set: n profile images of one codon length (which = 3 or 5), profile p in the layout
+ * bathgpu_load_fs_profile takes (M[p], nrows[p], rfv[p], tfv[p]).  Held beside the context's single loaded profile, which stays
+ * untouched; loading a new set of the same codon length replaces the old one. */
+int bathgpu_load_fs_profile_set(bathgpu_ctx *ctx, int which, int n, const int *M, const int *nrows,
+                                const float *const *rfv, const float *const *tfv);
+
+/* A window of the selected slot's block (as bathgpu_window) scored with profile `profile` of the set. */
+typedef struct {
+  int64_t start;
+  int32_t L;
+  float   pmove;
+  float   ploop;
+  int32_t profile;
+} bathgpu_set_window;
+
+/* xfE[2 p], xfE[2 p + 1] = {E->MOVE, E->LOOP} odds of profile p.  which = 3: fwdsc[w] is what bathgpu_fs_fwd_windows returns for
+ * the window with that profile loaded alone (p7_ForwardParser_Frameshift_3Codons, call site src/evalues.c:649); which = 5: what
+ * bathgpu_fs_forward_matrices returns in its scores-only mode (p7_ForwardParser_Frameshift_5Codons, :759).  Bit-identical to those
+ * calls, status[w] = eslERANGE where they set it.  Windows of any mix of profiles and lengths, in any order. */
+int bathgpu_fs_set_scores(bathgpu_ctx *ctx, int which, const bathgpu_set_window *wins, int n, const float *xfE,
+                          float *fwdsc, int32_t *status);
+
 /* Test/diagnostic: matrices of envelope e of the last chunk of the last bathgpu_fs_domains call, in the
  * reference's cell order: pp [(L+1)][(M+1)][8] {D,I,M_C0..M_C5} (impl_sse.h:296-314; D cells are 0 after
  * decoding), oa [(L+1)][(M+1)][3] {M,D,I}, ppx / oax [(L+1)][6] {E,N,J,B,C,SCALE}.  Any pointer may be NULL. */

@@ -13,6 +13,7 @@
  *                                as bathsearch sets a query up                 src/bathsearch.c:794-801
  *   bathhost_length_model     <- p7_fs_oprofile_ReconfigLength                 src/impl_sse/p7_fs_oprofile.c:636-651
  *   bathhost_calibrate        <- p7_Calibrate / bathconvert's frameshift taus  src/evalues.c:64-183; src/bathconvert.c:128-161
+ *   bathhost_convert          <- bathconvert over a HMMER3/f library           src/bathconvert.c:128-161 per model
  */
 #ifndef BATHHOST_H
 #define BATHHOST_H
@@ -136,6 +137,10 @@ typedef struct {
   /* optional (may be NULL: a chunk made of several sequences is then concatenated in a host buffer first and goes through
    * upload_block): bathgpu_upload_block_segments */
   int (*upload_block_segments)(void *ctx, const uint8_t *const *seg, const int64_t *seg_n, int nseg);
+  /* optional pair (both NULL: bathhost_convert calibrates model by model through bathhost_calibrate):
+   * bathgpu_load_fs_profile_set and bathgpu_fs_set_scores, the frameshift Forward parsers over many profiles at once */
+  int (*load_fs_profile_set)(void *ctx, int which, int n, const int *M, const int *nrows, const float *const *rfv, const float *const *tfv);
+  int (*fs_set_scores)(void *ctx, int which, const void *wins, int n, const float *xfE, float *fwdsc, int32_t *status);
 } bathhost_backend;
 
 /* 0 / unset fields take bathsearch's defaults (src/p7_pipeline.c:145-214; src/bathsearch.c:94) */
@@ -258,6 +263,20 @@ typedef struct {
 } bathhost_calibration;
 int    bathhost_calibrate(const bathhost_model *m, const bathhost_backend *be, bathhost_calibration *cal, double evparam[8]);
 double bathhost_model_lambda(const bathhost_model *m);          /* p7_Lambda, src/evalues.c:243-250 */
+
+/* ---- HMMER3/f -> BATH3/f (convert.cpp) ----------------------------------------------------------------------------
+ * bathconvert for a library of hmmbuild models (read each model, add the frameshift parts, calibrate the two frameshift taus as
+ * src/bathconvert.c:128-161 does, write): every model of in_path, read in one pass, is written to out_path as its own text with the first line
+ * "BATH3/f", and "STATS LOCAL FS3 FORWARD", "STATS LOCAL FS5 FORWARD", "FRAMESHIFT PROB" and "CODON TABLE" lines after its
+ * "STATS LOCAL FORWARD" line; every other byte is as the input has it.  ct (0 = 1) and fsprob (0 = 0.01) apply to every model.
+ * The taus are those of bathhost_calibrate(convert_flow = 1, which_mask = FS3 | FS5) called model after model on one generator
+ * (seed; rng_state carried), with the lambda of each model's STATS LOCAL FORWARD line.  With the backend's load_fs_profile_set /
+ * fs_set_scores the simulations of many models share each device call (the output is the same).  BATHHOST_EFORMAT for anything but
+ * HMMER3/f input, EINVAL for ct or fsprob; on failure out_path is not written.  *nmodels = models converted;
+ * bathhost_convert_last_error() says why a call of this thread failed. */
+int         bathhost_convert(const char *in_path, const char *out_path, int ct, float fsprob, uint32_t seed,
+                             const bathhost_backend *be, int *nmodels);
+const char *bathhost_convert_last_error(void);
 
 #ifdef __cplusplus
 }
