@@ -69,7 +69,7 @@ _OBJ = os.path.join(_HERE, "_obj")
 
 # kernels_tu.cu is compiled once per (family, node-count set): see csrc/launch.h
 _FAMILIES = {"fwd": 1, "bck": 2, "fs5": 3, "orf": 4}
-_SETS = {"a": 0, "b": 1, "c": 2, "d": 3, "e": 4, "f": 5}
+_SETS = {"a": 0, "b": 1, "c": 2, "d": 3, "e": 4, "f": 5, "g": 6, "h": 7}
 _FILTERS = {"msv": 5, "vit_lo": 6, "vit_hi": 7}
 
 
@@ -114,7 +114,7 @@ def build_library(force=False, verbose=False, jobs=None, variant=None, extra_fla
     else:
         keep = []
     # longest first: the node-count sets with the most (or the largest) instantiations
-    units.sort(key=lambda u: (u[0].endswith(("_f", "_e", "_c", "_b")), u[0]), reverse=True)
+    units.sort(key=lambda u: (u[0].endswith(("_h", "_g", "_f", "_e", "_c", "_b")), u[0]), reverse=True)
     with ThreadPoolExecutor(max_workers=jobs or os.cpu_count() or 4) as pool:
         objs = list(pool.map(compile_one, units)) + keep
     subprocess.check_call([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-Xcompiler", "-fPIC", "-o", _SO] + objs)

@@ -10,7 +10,7 @@ OK, EMEM, EINVAL, ERANGE, ENODEVICE, ECUDA = 0, 5, 11, 16, 100, 101
 KP = 29
 
 EXPORTS = [
-    "bathgpu_create", "bathgpu_destroy", "bathgpu_last_error", "bathgpu_device_info",
+    "bathgpu_create", "bathgpu_destroy", "bathgpu_last_error", "bathgpu_device_info", "bathgpu_set_long_models",
     "bathgpu_load_fs_profile", "bathgpu_upload_block", "bathgpu_fs_fwd_windows",
     "bathgpu_stage_windows", "bathgpu_fs_fwd_staged", "bathgpu_fetch_scores",
     "bathgpu_fs_bck_decode", "bathgpu_fs_domains", "bathgpu_last_stage_timing", "bathgpu_measure_fp32_peak",
@@ -81,6 +81,8 @@ def load():
     L.bathgpu_last_error.restype = C.c_char_p
     L.bathgpu_last_error.argtypes = [vp]
     L.bathgpu_device_info.restype = C.c_int
+    L.bathgpu_set_long_models.restype = C.c_int
+    L.bathgpu_set_long_models.argtypes = [vp, C.c_int]
     L.bathgpu_device_info.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_size_t)]
     L.bathgpu_load_fs_profile.restype = C.c_int
     L.bathgpu_load_fs_profile.argtypes = [vp, C.c_int, C.c_int, C.c_int, fp, fp]
@@ -205,13 +207,16 @@ class Context:
     """One device context (one stream).  Mirrors the per-worker P7_PIPELINE ownership of the
     reference (src/bathsearch.c:814-844): one context per worker thread / per GPU."""
 
-    def __init__(self, device=0):
+    def __init__(self, device=0, long_models=False):
+        """long_models: take profiles of up to 2048 nodes (bathgpu_set_long_models); without it the context refuses profiles past 1024"""
         self.lib = load()
         h = C.c_void_p()
         st = self.lib.bathgpu_create(device, C.byref(h))
         if st != OK:
             raise BathGpuError(st, "bathgpu_create failed (no usable CUDA device?)")
         self.h = h
+        if long_models:
+            self._check(self.lib.bathgpu_set_long_models(self.h, 1))
 
     def close(self):
         if getattr(self, "h", None):

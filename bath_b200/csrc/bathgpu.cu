@@ -13,6 +13,7 @@
 #include <algorithm>
 #include <mutex>
 #include <memory>
+#include <functional>
 
 #include "../../include/bathgpu.h"
 #include "fs_parser.cuh"
@@ -79,6 +80,7 @@ struct FsProfileImage {
   int    mw_scan_steps = 5;
   DevBuf cellb;    // backward lane constants
   DevBuf cellf5;   // 5-codon full-matrix Forward lane constants (fs_domain.cuh)
+  DevBuf cellf5mw, cellb5mw;   // the Forward and Backward constants of the multi-warp envelope sweeps (fs_domain_mw.cuh; J >= 16)
   DevBuf amino;    // [20][mpad] amino-acid odds, unfolded, permuted (null2)
   DevBuf oaflags;  // [mpad] transition-allowed bits per node (optimal accuracy masks)
   DevBuf oapass;   // [5][32] D pass-through flags of the optimal-accuracy scan
@@ -128,6 +130,7 @@ struct bathgpu_ctx {
   bool          flt_loaded = false;
   bathgpu_filter_params flt{};
   int           flt_W = 0, flt_P = 0;
+  int           max_model_length = 1024;          // bathgpu_set_long_models: 2048
   DevBuf        f_rbv, f_rwv, f_twv, f_ddsum, f_nrb, orfs, fsc, fst, fwins, fnw;
   DevBuf        b_items, b_tables, b_out;      // bias filter
   DevBuf        o_tiles, o_cnt, o_base, o_blocks, o_first, o_tjb, o_null, o_meta, o_hits, o_counters;
@@ -392,7 +395,27 @@ extern "C" int bathgpu_measure_fp32_peak(bathgpu_ctx *ctx, double *tflops, doubl
 
 // ---------------------------------------------------------------------------------------------
 // profile images
-static const int kSupportedJ[] = { 1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 16, 24, 32 };   // 16, 24, 32: part of the state spills (launch.h)
+// 16, 24, 32: part of the one-warp kernels' state spills; 48, 64: multi-warp kernels only (launch.h)
+static const int kSupportedJ[] = { 1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 16, 24, 32, 48, 64 };
+constexpr int kMaxModelLength = 32 * 64;
+constexpr int kDefaultModelLength = 32 * 32;    // the one-warp kernels' reach: a context takes longer profiles once asked to
+
+// Refuses a profile longer than the context takes (the loaders' first size check).
+static int check_model_length(bathgpu_ctx *ctx, int M)
+{
+  if (M > kMaxModelLength) return fail(ctx, BATHGPU_EINVAL, "model length %d exceeds the longest supported profile (%d nodes)", M, kMaxModelLength);
+  if (M > ctx->max_model_length)
+    return fail(ctx, BATHGPU_EINVAL, "model length %d exceeds %d nodes, the limit of a context without long models (bathgpu_set_long_models "
+                "takes it to %d)", M, ctx->max_model_length, kMaxModelLength);
+  return BATHGPU_OK;
+}
+
+extern "C" int bathgpu_set_long_models(bathgpu_ctx *ctx, int on)
+{
+  if (!ctx) return BATHGPU_EINVAL;
+  ctx->max_model_length = on ? kMaxModelLength : kDefaultModelLength;
+  return BATHGPU_OK;
+}
 
 static int choose_J(int M)
 {
@@ -431,8 +454,8 @@ static int fold_profile(bathgpu_ctx *ctx, int which, int M, int nrows, const flo
   if (which != 3 && which != 5)     return fail(ctx, BATHGPU_EINVAL, "codon_lengths must be 3 or 5");
   const int want_rows = (which == 3 ? 338 : 1367) + BATHGPU_KP;
   if (nrows != want_rows)           return fail(ctx, BATHGPU_EINVAL, "nrows %d != %d for %d codon lengths", nrows, want_rows, which);
+  if (check_model_length(ctx, M) != BATHGPU_OK) return BATHGPU_EINVAL;
   const int J = choose_J(M);
-  if (J == 0) return fail(ctx, BATHGPU_EINVAL, "model length %d exceeds the single-warp kernels' limit (%d)", M, 32 * 32);
   f.M = M; f.J = J; f.mpad = 32 * J; f.ld = M + 1; f.tfv = tfv;
   const int mpad = f.mpad;
   auto T = [&](int t, int k) -> double { return f.T(t, k); };
@@ -567,8 +590,59 @@ static void forward3_tables(const Fold &f, int which, int nrows, const float *rf
   }
 }
 
-// the full-matrix 5-codon Forward lane constants (fs_domain.cuh, Fwd5Const)
-static void fs5_forward_consts(const Fold &f, std::vector<float> &cc)
+// The multi-warp envelope sweeps' image of per-node constants (fs_domain_mw.cuh): node(c, k) for each of the ncell constant kinds, laid
+// out [ncell][8][32 NW] by virtual lane v = 32 w + lane owning nodes 8 v + 1 .. 8 v + 8, then the chain products: per lane the product
+// of dd over its 8 nodes scanned inside its warp (forward: from lane l - 2^s + 1 to l, backward: from l to l + 2^s - 1), then Q / QU
+// and per warp PW / PWb, dd and vdm of its last node.  Empty below 16 nodes per lane.
+static void fs5_mw_image(const Fold &f, bool backward, int ncell, const std::function<double(int, int)> &node, const std::function<double(int)> &ddk,
+                         const std::function<double(int)> &vdmk, std::vector<float> &mw)
+{
+  mw.clear();
+  if (f.J < 16) return;
+  const int JW = kMwNodesPerLane, NW = f.J / JW, VL = 32 * NW, M = f.M;
+  mw.assign((size_t)(ncell * JW + 6) * VL + 3 * NW, 0.0f);
+  std::vector<double> lp(VL, 1.0);
+  for (int v = 0; v < VL; ++v)
+    for (int j = 0; j < JW; ++j) {
+      const int k = v * JW + j + 1;
+      if (k <= M) for (int c = 0; c < ncell; ++c) mw[(size_t)(c * JW + j) * VL + v] = (float)node(c, k);
+      lp[v] *= ddk(k);
+    }
+  for (int w = 0; w < NW; ++w) {
+    std::vector<double> b(lp.begin() + 32 * w, lp.begin() + 32 * w + 32);
+    for (int s = 0; s < 5; ++s) {
+      const int d = 1 << s;
+      std::vector<double> nb(b);
+      for (int lane = 0; lane < 32; ++lane) {
+        const bool in = backward ? (lane + d <= 31) : (lane >= d);
+        mw[(size_t)(ncell * JW + s) * VL + 32 * w + lane] = in ? (float)b[lane] : 0.0f;
+        if (in) nb[lane] = b[lane] * b[backward ? lane + d : lane - d];
+      }
+      b.swap(nb);
+    }
+    const int k_a = 32 * w * JW + 1, k_b = 32 * (w + 1) * JW;          // first and last node of the warp
+    float *q = &mw[(size_t)(ncell * JW + 5) * VL + 32 * w], *tail = &mw[(size_t)(ncell * JW + 6) * VL];
+    if (!backward) {
+      double qq = 1.0;                                                  // Q: over the lanes in front; PW: the whole warp
+      for (int lane = 0; lane < 32; ++lane) { q[lane] = (float)qq; qq *= lp[32 * w + lane]; }
+      tail[w] = (float)qq;
+    } else {
+      for (int lane = 0; lane < 31; ++lane) {                          // QU: from the first node of lane + 1 to the warp's last node but one
+        double qq = 1.0;
+        for (int k = (32 * w + lane + 1) * JW + 1; k <= k_b - 1; ++k) qq *= ddk(k);
+        q[lane] = (float)qq;
+      }
+      double pw = 1.0;                                                  // PWb: the warp's nodes but the last
+      for (int k = k_a; k <= k_b - 1; ++k) pw *= ddk(k);
+      tail[w] = (float)pw;
+      tail[NW + w] = (float)ddk(k_b);
+      tail[2 * NW + w] = (float)vdmk(k_b);
+    }
+  }
+}
+
+// the full-matrix 5-codon Forward lane constants (fs_domain.cuh, Fwd5Const) and their multi-warp image (empty below 16 nodes per lane)
+static void fs5_forward_consts(const Fold &f, std::vector<float> &cc, std::vector<float> &mw)
 {
   const int M = f.M, J = f.J;
   const std::vector<double> &sK = f.sK, &zK = f.zK;
@@ -604,6 +678,19 @@ static void fs5_forward_consts(const Fold &f, std::vector<float> &cc)
     }
     b.swap(nb);
   }
+  auto node = [&](int c, int k) -> double {
+    const double sn = sK[k + 1];
+    switch (c) {
+    case F5_MM: return T(tMM, k) / (zK[k] * sn);
+    case F5_IM: return T(tIM, k) / sn;
+    case F5_DM: return T(tDM, k) / sn;
+    case F5_MD: return T(tMD, k) / zK[k];
+    case F5_DD: return T(tDD, k);
+    case F5_MI: return T(tMI, k) / zK[k];
+    default:    return T(tII, k);
+    }
+  };
+  fs5_mw_image(f, false, F5_COUNT, node, [&](int k) { return T(tDD, k); }, [](int) { return 0.0; }, mw);
 }
 
 extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int nrows, const float *rfv, const float *tfv)
@@ -679,6 +766,27 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
     if (im.cellb.reserve(cc.size() * sizeof(float)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
     CUDA_TRY(ctx, cudaMemcpyAsync(im.cellb.p, cc.data(), cc.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(ctx, wait_stream(ctx));
+    std::vector<float> mw;
+    auto node = [&](int c, int k) -> double {
+      const double sn = sK[k + 1];
+      switch (c) {
+      case BC_VMM: return T(tMM, k) / (sn * zK[k]);
+      case BC_VIM: return T(tIM, k) / sn;
+      case BC_VDM: return T(tDM, k) / sn;
+      case BC_DD:  return T(tDD, k);
+      case BC_MD:  return T(tMD, k) / zK[k];
+      case BC_MI:  return T(tMI, k) / zK[k];
+      default:     return T(tII, k);
+      }
+    };
+    auto ddk = [&](int k) -> double { return (k >= 1 && k <= M) ? T(tDD, k) : 0.0; };
+    auto vdmk = [&](int k) -> double { return (k >= 1 && k <= M) ? T(tDM, k) / sK[k + 1] : 0.0; };
+    fs5_mw_image(f, true, BC_COUNT, node, ddk, vdmk, mw);
+    if (!mw.empty()) {
+      if (im.cellb5mw.reserve(mw.size() * sizeof(float)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
+      CUDA_TRY(ctx, cudaMemcpyAsync(im.cellb5mw.p, mw.data(), mw.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+      CUDA_TRY(ctx, wait_stream(ctx));
+    } else im.cellb5mw.release();
   }
 
   // ---- the 3-codon Backward parser's scaled constants and table copy (fs_backward.cuh, Bck3Consts)
@@ -775,8 +883,13 @@ extern "C" int bathgpu_load_fs_profile(bathgpu_ctx *ctx, int which, int M, int n
 
   // ---- full-matrix Forward constants, null2 amino rows, optimal-accuracy masks, raw transitions (fs_domain.cuh)
   {
-    std::vector<float> cc;
-    fs5_forward_consts(f, cc);
+    std::vector<float> cc, mw;
+    fs5_forward_consts(f, cc, mw);
+    if (!mw.empty()) {
+      if (im.cellf5mw.reserve(mw.size() * sizeof(float)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
+      CUDA_TRY(ctx, cudaMemcpyAsync(im.cellf5mw.p, mw.data(), mw.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+      CUDA_TRY(ctx, wait_stream(ctx));
+    } else im.cellf5mw.release();
     const int amino0 = nrows - BATHGPU_KP;
     std::vector<float> am((size_t)20 * mpad, 0.0f);
     for (int x = 0; x < 20; ++x)
@@ -1460,6 +1573,7 @@ static int domains_chunk(bathgpu_ctx *ctx, const bathgpu_envelope *envs, int n, 
 
   DomainArgs a{};
   a.emis = im.emis.as<float>(); a.amino = im.amino.as<float>(); a.cellf = im.cellf5.as<float>(); a.cellb = im.cellb.as<float>();
+  a.cellfmw = im.cellf5mw.as<float>(); a.cellbmw = im.cellb5mw.as<float>();
   a.oapass = im.oapass.as<float>(); a.oaflags = im.oaflags.as<uint32_t>(); a.dna4 = ctx->S().dna4.as<uint32_t>();
   a.envs = ctx->envs.as<EnvelopeDesc>(); a.nenv = n; a.M = M; a.mpad = mpad; a.tEM = xfE5[0]; a.tEL = xfE5[1];
   a.xoff = ctx->xoff.as<long long>(); a.pp = ctx->dpp.as<float>(); a.oa = ctx->doa.as<float>(); a.fx = ctx->dfx.as<float>();
@@ -1620,7 +1734,7 @@ extern "C" int bathgpu_fs_forward_matrices(bathgpu_ctx *ctx, const bathgpu_envel
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->envs.p, regs + e0, (size_t)m * sizeof(EnvelopeDesc), cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->xoff.p, xoff.data(), (size_t)(m + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
     DomainArgs a{};
-    a.emis = im.emis.as<float>(); a.cellf = im.cellf5.as<float>(); a.dna4 = ctx->S().dna4.as<uint32_t>();
+    a.emis = im.emis.as<float>(); a.cellf = im.cellf5.as<float>(); a.cellfmw = im.cellf5mw.as<float>(); a.dna4 = ctx->S().dna4.as<uint32_t>();
     a.envs = ctx->envs.as<EnvelopeDesc>(); a.nenv = m; a.M = M; a.mpad = mpad; a.tEM = xfE5[0]; a.tEL = xfE5[1];
     a.xoff = ctx->xoff.as<long long>(); a.pp = ctx->dpp.as<float>(); a.dcell = ctx->ddcell.as<float>(); a.fx = ctx->dfx.as<float>();
     a.lsf = ctx->dlsf.as<float>(); a.fwdsc = ctx->dfw.as<float>(); a.status = ctx->dstat.as<int>(); a.counter = ctx->counter.as<int>();
@@ -1675,7 +1789,7 @@ extern "C" int bathgpu_load_fs_profile_set(bathgpu_ctx *ctx, int which, int n, c
     const int st = fold_profile(ctx, which, M[p], nrows[p], rfv[p], tfv[p], f);
     if (st != BATHGPU_OK) return fail(ctx, st, "profile %d of the set: %s", p, std::string(ctx->err).c_str());
     if (which == 3) forward3_tables(f, 3, nrows[p], rfv[p], tab, cc, mw, ps.scan_steps[p], ps.mw_scan_steps[p]);
-    else { emission_table(f, nrows[p], rfv[p], tab); fs5_forward_consts(f, cc); mw.clear(); }
+    else { emission_table(f, nrows[p], rfv[p], tab); fs5_forward_consts(f, cc, mw); }
     ps.J[p] = f.J;
     off_emis[p] = append(tab);
     off_cc[p] = append(cc);
@@ -1862,14 +1976,15 @@ extern "C" int bathgpu_load_filter_profile(bathgpu_ctx *ctx, const bathgpu_filte
 {
   if (!ctx || !prm || !rbv || !rwv || !twv || prm->M < 1) return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_load_filter_profile");
   const int M = prm->M, ld = M + 1;
-  if (M > 1024) return fail(ctx, BATHGPU_EINVAL, "model length %d exceeds the single-warp kernels' limit (1024)", M);
+  if (check_model_length(ctx, M) != BATHGPU_OK) return BATHGPU_EINVAL;
   if (prm->cpu_lanes_u8 < 1 || prm->cpu_lanes_i16 < 1) return fail(ctx, BATHGPU_EINVAL, "cpu lane counts must be positive");
   CUDA_TRY(ctx, enter(ctx));
   ctx->flt_loaded = false;
   ctx->flt = *prm;
   int W = (M + 127) / 128, P = (M + 63) / 64;
   if (W == 5) W = 6; else if (W == 7) W = 8;             // instantiated widths (launch.h)
-  if (P > 6) P = (P <= 8) ? 8 : (P <= 12) ? 12 : 16;
+  else if (W > 8) W = (W <= 12) ? 12 : 16;
+  if (P > 6) P = (P <= 8) ? 8 : (P <= 12) ? 12 : (P <= 16) ? 16 : (P <= 24) ? 24 : 32;
   ctx->flt_W = W; ctx->flt_P = P;
   const int nb = 128 * W, nw = 64 * P;                 // nodes per padded row
   std::vector<uint8_t> hb((size_t)29 * nb, 255);

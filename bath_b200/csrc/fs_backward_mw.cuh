@@ -309,8 +309,9 @@ __device__ __forceinline__ void mw_bck_row_pair(int i, int lane, int warp, BckSt
 }
 
 // constant image (bathgpu.cu, cellbmw): [5 JW + 6][32 NW] floats (qb, dd, md, mi, ii per node; 5 scan multipliers; QU), then PWb[NW], DDL[NW]
+// two blocks a multiprocessor up to NW = 4, one from NW = 6 up (two blocks allow 170 or 128 registers a thread there: 92 and 124 bytes spilled)
 template <int NW, int JW>
-__global__ void __launch_bounds__(32 * NW, 2) fs3_backward_parser_kernel_mw(FsBackwardArgs a)
+__global__ void __launch_bounds__(32 * NW, (NW >= 5) ? 1 : 2) fs3_backward_parser_kernel_mw(FsBackwardArgs a)
 {
   __shared__ MwBckShared<NW> sh;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, vl = threadIdx.x;

@@ -52,6 +52,8 @@ struct DomainArgs {
   const float    *amino;       // amino-acid odds rows, NOT folded: [20][mpad] permuted (null2)
   const float    *cellf;       // forward lane constants  [F5_COUNT][J][32] + [5][32]
   const float    *cellb;       // backward lane constants [BC_COUNT][J][32] + [5][32]
+  const float    *cellfmw;     // the same two for the multi-warp sweeps (fs_domain_mw.cuh; J >= 16), or null
+  const float    *cellbmw;
   const float    *oapass;      // [5][32]: scan step s may carry D through the lanes it spans (all DD allowed)
   const uint32_t *oaflags;     // per node: bit t set iff transition t has positive odds, t = BM,MM,IM,DM (source k-1), MD,DD (source k-1), MI,II (k)
   const uint32_t *dna4;
@@ -71,7 +73,7 @@ struct DomainArgs {
   float          *null2;       // [nenv][29]
   int            *status;      // [nenv]
   int            *counter;
-  const FsSetProfile *set;     // fs5_forward_kernel<J, true, true>: envelope e is scored with profile set[wprof[e]] (emis, cellf, tEM, tEL unused)
+  const FsSetProfile *set;     // fs5_forward_kernel<J, true, true>: envelope e is scored with profile set[wprof[e]] (emis, cellf, cellfmw, tEM, tEL unused)
   const int      *wprof;
 };
 

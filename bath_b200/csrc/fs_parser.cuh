@@ -47,7 +47,7 @@ struct WindowDesc {      // device copy of bathgpu_window
 struct FsSetProfile {
   const float *emis;           // the table the kernel reads: emis_fwd (3 codon lengths) or emis (5)
   const float *cellc;          // lane constants: cellc (3) or cellf5 (5)
-  const float *cellmw;         // multi-warp Forward constants (3, J >= 16), else null
+  const float *cellmw;         // multi-warp Forward constants (J >= 16: fs_parser_mw.cuh for 3 codon lengths, fs_domain_mw.cuh for 5), else null
   float        tEM, tEL;       // E->MOVE, E->LOOP odds of this profile
 };
 

@@ -160,7 +160,9 @@ __device__ __forceinline__ void mw_row_pair(int i, int lane, int warp, FwdState<
 }
 
 // JW nodes per lane, NW warps per window (32 NW JW >= M).  Resident blocks per SM the kernel is compiled for.
-template <int NW, int JW> struct MwTune { static constexpr int kBlocks = (JW == 8) ? ((NW == 4) ? 2 : (NW == 3) ? 2 : 4) : ((NW >= 5) ? 2 : 4); };
+// NW = 6, 8 (M > 1024): one block, up to 255 registers a thread.  Four blocks capped them at 64 registers, two at 170 (NW = 6) or 128
+// (NW = 8), and all of these spilled (76-764 bytes a thread).
+template <int NW, int JW> struct MwTune { static constexpr int kBlocks = (JW == 8) ? ((NW >= 5) ? 1 : (NW == 4) ? 2 : (NW == 3) ? 2 : 4) : ((NW >= 5) ? 2 : 4); };
 
 template <int NW, int JW>
 __device__ __forceinline__ void mw_load_consts(const float *__restrict__ cc, int vl, FwdConsts<JW> &K, float &Q, float (&PW)[NW])

@@ -10,6 +10,7 @@
 #include "fs_backward.cuh"
 #include "fs_backward_mw.cuh"
 #include "fs_domain.cuh"
+#include "fs_domain_mw.cuh"
 #include "orf_domain.cuh"
 #include "orf_filters.cuh"
 
@@ -39,11 +40,19 @@
 #elif BATHGPU_SET == 5
 #define SETNAME f
 #define JLIST(X) X(32)
+#elif BATHGPU_SET == 6
+#define SETNAME g
+#define JLIST(X) X(48)
+#elif BATHGPU_SET == 7
+#define SETNAME h
+#define JLIST(X) X(64)
 #endif
 #define CAT2(a, b) a##b
 #define CAT(a, b) CAT2(a, b)
 
 namespace bathgpu {
+
+static_assert(kMw5NodesPerLane == kMwNodesPerLane, "the loader builds every multi-warp constant image for 8 nodes per lane");
 
 template <class K> static void touch(K kernel) { cudaFuncAttributes fa; cudaFuncGetAttributes(&fa, kernel); }
 
@@ -78,6 +87,10 @@ template <int NW, int JW, bool XMX, bool SET = false> static cudaError_t run_fwd
 // SET: the windows of a profile set (FsParserArgs::set); a.cellmw non-null when the set's profiles have multi-warp images
 template <int J, bool XMX, bool SET = false> static cudaError_t run_fwd(int version, const FsParserArgs &a, int sms, cudaStream_t s)
 {
+  if constexpr (J > 32) {             // past 32 nodes per lane the multi-warp kernel is the only one (the one-warp kernels are not built)
+    if (!a.cellmw) return cudaErrorInvalidValue;
+    return run_fwd_mw<J / kMwNodesPerLane, kMwNodesPerLane, XMX, SET>(a, sms, s);
+  } else {
   if constexpr (J >= 16) {
     // BATHGPU_FWD_MW: 0 never, 1 (default) from 24 nodes per lane up -- at 16 the one-warp kernel is still ahead (800 vs 620 GCUPS
     // at M = 409) --, 2 from 16 up
@@ -95,6 +108,7 @@ template <int J, bool XMX, bool SET = false> static cudaError_t run_fwd(int vers
     else                        fs3_forward_parser_kernel_v3<J, XMX, 5, SET><<<fwd_grid(fs3_forward_parser_kernel_v3<J, XMX, 5, SET>, J, a.nwin, sms), 32, 0, s>>>(a);
   }
   return cudaGetLastError();
+  }
 }
 // the Forward parser over the windows of a profile set: the kernel run_fwd picks for the set's J, scan steps and version
 bool CAT(launch_fs3_forward_set_, SETNAME)(int J, int version, const FsParserArgs &a, int sms, cudaStream_t s, cudaError_t *err)
@@ -115,14 +129,23 @@ bool CAT(launch_fs3_forward_, SETNAME)(int J, bool xmx, int version, const FsPar
   default: return false;
   }
 }
+template <int J> static void preload_fwd_t()
+{
+  if constexpr (J > 32) {
+    constexpr int NW = J / kMwNodesPerLane, JW = kMwNodesPerLane;
+    touch(fs3_forward_parser_kernel_mw<NW, JW, false, 3>); touch(fs3_forward_parser_kernel_mw<NW, JW, true, 3>);
+    touch(fs3_forward_parser_kernel_mw<NW, JW, false, 5>); touch(fs3_forward_parser_kernel_mw<NW, JW, true, 5>);
+  } else {
+    touch(fs3_forward_parser_kernel_v3<J, false, 2>); touch(fs3_forward_parser_kernel_v3<J, true, 2>); touch(fs3_forward_parser_kernel_v3<J, false, 3>);
+    touch(fs3_forward_parser_kernel_v3<J, true, 3>); touch(fs3_forward_parser_kernel_v3<J, false, 5>); touch(fs3_forward_parser_kernel_v3<J, true, 5>);
+    if (J == 10) { touch(fs3_forward_parser_kernel_v4<J, false, 2>); touch(fs3_forward_parser_kernel_v4<J, true, 2>); touch(fs3_forward_parser_kernel_v4<J, false, 3>);
+                   touch(fs3_forward_parser_kernel_v4<J, true, 3>); touch(fs3_forward_parser_kernel_v4<J, false, 5>); touch(fs3_forward_parser_kernel_v4<J, true, 5>); }
+  }
+}
 void CAT(preload_fwd_, SETNAME)(int J)
 {
   switch (J) {
-#define X(J_) case J_: touch(fs3_forward_parser_kernel_v3<J_, false, 2>); touch(fs3_forward_parser_kernel_v3<J_, true, 2>); touch(fs3_forward_parser_kernel_v3<J_, false, 3>); \
-                       touch(fs3_forward_parser_kernel_v3<J_, true, 3>); touch(fs3_forward_parser_kernel_v3<J_, false, 5>); touch(fs3_forward_parser_kernel_v3<J_, true, 5>); \
-                       if (J_ == 10) { touch(fs3_forward_parser_kernel_v4<J_, false, 2>); touch(fs3_forward_parser_kernel_v4<J_, true, 2>); touch(fs3_forward_parser_kernel_v4<J_, false, 3>); \
-                                       touch(fs3_forward_parser_kernel_v4<J_, true, 3>); touch(fs3_forward_parser_kernel_v4<J_, false, 5>); touch(fs3_forward_parser_kernel_v4<J_, true, 5>); } \
-                       break;
+#define X(J_) case J_: preload_fwd_t<J_>(); break;
   JLIST(X)
 #undef X
   default: break;
@@ -143,8 +166,11 @@ template <int J> static cudaError_t run_bck(const FsBackwardArgs &a, int sms, cu
       return cudaGetLastError();
     }
   }
-  fs3_backward_parser_kernel<J><<<grid_for(fs3_backward_parser_kernel<J>, BckTune<J>::kThreads, 0, a.nwin, sms), BckTune<J>::kThreads, 0, s>>>(a);
-  return cudaGetLastError();
+  if constexpr (J > 32) return cudaErrorInvalidValue;        // no one-warp kernel past 32 nodes per lane: the multi-warp image is required
+  else {
+    fs3_backward_parser_kernel<J><<<grid_for(fs3_backward_parser_kernel<J>, BckTune<J>::kThreads, 0, a.nwin, sms), BckTune<J>::kThreads, 0, s>>>(a);
+    return cudaGetLastError();
+  }
 }
 bool CAT(launch_fs3_backward_, SETNAME)(int J, const FsBackwardArgs &a, int sms, cudaStream_t s, cudaError_t *err)
 {
@@ -155,10 +181,15 @@ bool CAT(launch_fs3_backward_, SETNAME)(int J, const FsBackwardArgs &a, int sms,
   default: return false;
   }
 }
+template <int J> static void preload_bck_t()
+{
+  if constexpr (J <= 32) touch(fs3_backward_parser_kernel<J>);
+  if constexpr (J >= 16) touch(fs3_backward_parser_kernel_mw<J / kMwNodesPerLane, kMwNodesPerLane>);
+}
 void CAT(preload_bck_, SETNAME)(int J)
 {
   switch (J) {
-#define X(J_) case J_: touch(fs3_backward_parser_kernel<J_>); if constexpr (J_ >= 16) touch(fs3_backward_parser_kernel_mw<J_ / kMwNodesPerLane, kMwNodesPerLane>); break;
+#define X(J_) case J_: preload_bck_t<J_>(); break;
   JLIST(X)
 #undef X
   default: break;
@@ -167,8 +198,53 @@ void CAT(preload_bck_, SETNAME)(int J)
 #endif
 
 #if BATHGPU_FAMILY == FAM_FS5
+// J/8 warps per envelope (fs_domain_mw.cuh): always past 32 nodes per lane, where the one-warp sweeps are not built; BATHGPU_FS5_MW=2
+// from 16 up as well, to compare them with the one-warp sweeps on the models both can run
+[[maybe_unused]] static bool fs5_mw(int J)
+{
+  static const int mode = [] { const char *e = getenv("BATHGPU_FS5_MW"); return e ? atoi(e) : 1; }();
+  return J > 32 || (mode >= 2 && J >= 16);
+}
+
+template <int J> static cudaError_t run_fs5_mw(const DomainArgs &a, const TraceArgs &t, int sms, cudaStream_t s)
+{
+  constexpr int NW = J / kMw5NodesPerLane;
+  if (!a.cellfmw || !a.cellbmw) return cudaErrorInvalidValue;
+  cudaError_t e;
+  if ((e = cudaMemsetAsync(a.counter, 0, 4, s)) != cudaSuccess) return e;
+  fs5_forward_kernel_mw<NW><<<grid_for(fs5_forward_kernel_mw<NW>, 32 * NW, 0, a.nenv, sms), 32 * NW, 0, s>>>(a);
+  if ((e = cudaMemsetAsync(a.counter, 0, 4, s)) != cudaSuccess) return e;
+  fs5_backward_decode_kernel_mw<NW><<<grid_for(fs5_backward_decode_kernel_mw<NW>, 32 * NW, 0, a.nenv, sms), 32 * NW, 0, s>>>(a);
+  if ((e = cudaMemsetAsync(a.counter, 0, 4, s)) != cudaSuccess) return e;
+  fs5_optacc_kernel_mw<NW><<<grid_for(fs5_optacc_kernel_mw<NW>, 32 * NW, 0, a.nenv, sms), 32 * NW, 0, s>>>(a);
+  fs5_oatrace_kernel<<<(a.nenv + 3) / 4, 128, 0, s>>>(a, t);
+  return cudaGetLastError();
+}
+
+// the Forward sweep alone, D cells kept (SET: over the envelopes of a profile set, whose caller clears the counter)
+template <int J, bool SET> static cudaError_t run_fs5_forward_matrix(const DomainArgs &a, int sms, cudaStream_t s)
+{
+  if constexpr (!SET) { cudaError_t e = cudaMemsetAsync(a.counter, 0, 4, s); if (e != cudaSuccess) return e; }
+  if constexpr (J >= 16) {
+    if (fs5_mw(J)) {
+      constexpr int NW = J / kMw5NodesPerLane;
+      if (!SET && !a.cellfmw) return cudaErrorInvalidValue;
+      fs5_forward_kernel_mw<NW, true, SET><<<grid_for(fs5_forward_kernel_mw<NW, true, SET>, 32 * NW, 0, a.nenv, sms), 32 * NW, 0, s>>>(a);
+      return cudaGetLastError();
+    }
+  }
+  if constexpr (J <= 32) {
+    fs5_forward_kernel<J, true, SET><<<grid_for(fs5_forward_kernel<J, true, SET>, 32, 0, a.nenv, sms), 32, 0, s>>>(a);
+    return cudaGetLastError();
+  }
+  return cudaErrorInvalidValue;
+}
+
 template <int J> static cudaError_t run_fs5(const DomainArgs &a, const TraceArgs &t, int sms, cudaStream_t s)
 {
+  if constexpr (J >= 16) { if (fs5_mw(J)) return run_fs5_mw<J>(a, t, sms, s); }
+  if constexpr (J > 32) return cudaErrorInvalidValue;
+  else {
   cudaError_t e;
   if ((e = cudaMemsetAsync(a.counter, 0, 4, s)) != cudaSuccess) return e;
   fs5_forward_kernel<J><<<grid_for(fs5_forward_kernel<J>, 32, 0, a.nenv, sms), 32, 0, s>>>(a);
@@ -178,6 +254,7 @@ template <int J> static cudaError_t run_fs5(const DomainArgs &a, const TraceArgs
   fs5_optacc_kernel<J><<<grid_for(fs5_optacc_kernel<J>, 32, 0, a.nenv, sms), 32, 0, s>>>(a);
   fs5_oatrace_kernel<<<(a.nenv + 3) / 4, 128, 0, s>>>(a, t);
   return cudaGetLastError();
+  }
 }
 bool CAT(launch_fs5_domains_, SETNAME)(int J, const DomainArgs &a, const TraceArgs &t, int sms, cudaStream_t s, cudaError_t *err)
 {
@@ -193,9 +270,7 @@ bool CAT(launch_fs5_domains_, SETNAME)(int J, const DomainArgs &a, const TraceAr
 bool CAT(launch_fs5_forward_matrix_, SETNAME)(int J, const DomainArgs &a, int sms, cudaStream_t s, cudaError_t *err)
 {
   switch (J) {
-#define X(J_) case J_: if ((*err = cudaMemsetAsync(a.counter, 0, 4, s)) != cudaSuccess) return true;                               \
-                       fs5_forward_kernel<J_, true><<<grid_for(fs5_forward_kernel<J_, true>, 32, 0, a.nenv, sms), 32, 0, s>>>(a);   \
-                       *err = cudaGetLastError(); return true;
+#define X(J_) case J_: *err = run_fs5_forward_matrix<J_, false>(a, sms, s); return true;
   JLIST(X)
 #undef X
   default: return false;
@@ -205,17 +280,27 @@ bool CAT(launch_fs5_forward_matrix_, SETNAME)(int J, const DomainArgs &a, int sm
 bool CAT(launch_fs5_forward_set_, SETNAME)(int J, const DomainArgs &a, int sms, cudaStream_t s, cudaError_t *err)
 {
   switch (J) {
-#define X(J_) case J_: fs5_forward_kernel<J_, true, true><<<grid_for(fs5_forward_kernel<J_, true, true>, 32, 0, a.nenv, sms), 32, 0, s>>>(a); \
-                       *err = cudaGetLastError(); return true;
+#define X(J_) case J_: *err = run_fs5_forward_matrix<J_, true>(a, sms, s); return true;
   JLIST(X)
 #undef X
   default: return false;
   }
 }
+template <int J> static void preload_fs5_t()
+{
+  if constexpr (J <= 32) { touch(fs5_forward_kernel<J>); touch(fs5_backward_decode_kernel<J>); touch(fs5_optacc_kernel<J>); }
+  if constexpr (J >= 16) {
+    if (fs5_mw(J)) {
+      constexpr int NW = J / kMw5NodesPerLane;
+      touch(fs5_forward_kernel_mw<NW>); touch(fs5_backward_decode_kernel_mw<NW>); touch(fs5_optacc_kernel_mw<NW>);
+    }
+  }
+  touch(fs5_oatrace_kernel);
+}
 void CAT(preload_fs5_, SETNAME)(int J)
 {
   switch (J) {
-#define X(J_) case J_: touch(fs5_forward_kernel<J_>); touch(fs5_backward_decode_kernel<J_>); touch(fs5_optacc_kernel<J_>); touch(fs5_oatrace_kernel); break;
+#define X(J_) case J_: preload_fs5_t<J_>(); break;
   JLIST(X)
 #undef X
   default: break;
@@ -288,6 +373,10 @@ void CAT(preload_orf_, SETNAME)(int J)
 template <int W, int MODE> static cudaError_t run_msv(const FilterArgs &a, int sms, cudaStream_t s)
 {
   const size_t smem = (size_t)29 * 32 * W * 4;
+  if (smem > 48 * 1024) {              // W = 16 (M > 1536)
+    cudaError_t e = cudaFuncSetAttribute(msv_filter_kernel<W, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
   msv_filter_kernel<W, MODE><<<grid_for(msv_filter_kernel<W, MODE>, 128, smem, (a.norf + 3) / 4, sms), 128, smem, s>>>(a);
   return cudaGetLastError();
 }
@@ -307,14 +396,14 @@ bool launch_msv_filter(int W, int P, int mode, const FilterArgs &a, int sms, cud
   if (mode == 0) {
     switch (P) {
 #define X(P_) case P_: *err = run_msv16<P_>(a, sms, s); return true;
-    X(1) X(2) X(3) X(4) X(5) X(6) X(8) X(12) X(16)
+    X(1) X(2) X(3) X(4) X(5) X(6) X(8) X(12) X(16) X(24) X(32)
 #undef X
     default: return false;
     }
   }
   switch (W) {
 #define X(W_) case W_: *err = run_msv<W_, 1>(a, sms, s); return true;
-  X(1) X(2) X(3) X(4) X(6) X(8)
+  X(1) X(2) X(3) X(4) X(6) X(8) X(12) X(16)
 #undef X
   default: return false;
   }
@@ -323,13 +412,13 @@ void preload_msv_filter(int W, int P)
 {
   switch (W) {
 #define X(W_) case W_: touch(msv_filter_kernel<W_, 1>); break;
-  X(1) X(2) X(3) X(4) X(6) X(8)
+  X(1) X(2) X(3) X(4) X(6) X(8) X(12) X(16)
 #undef X
   default: break;
   }
   switch (P) {
 #define X(P_) case P_: touch(msv16_filter_kernel<P_>); break;
-  X(1) X(2) X(3) X(4) X(5) X(6) X(8) X(12) X(16)
+  X(1) X(2) X(3) X(4) X(5) X(6) X(8) X(12) X(16) X(24) X(32)
 #undef X
   default: break;
   }
@@ -371,7 +460,7 @@ bool launch_vit_filter_hi(int P, const FilterArgs &a, int sms, cudaStream_t s, c
 {
   switch (P) {
 #define X(P_) case P_: *err = run_vit<P_>(a, sms, s); return true;
-  X(8) X(12) X(16)
+  X(8) X(12) X(16) X(24) X(32)
 #undef X
   default: return false;
   }
@@ -380,7 +469,7 @@ void preload_vit_filter_hi(int P)
 {
   switch (P) {
 #define X(P_) case P_: touch(vit_filter_kernel<P_>); break;
-  X(8) X(12) X(16)
+  X(8) X(12) X(16) X(24) X(32)
 #undef X
   default: break;
   }

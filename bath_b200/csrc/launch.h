@@ -15,9 +15,11 @@ struct OrfDomainArgs;
 struct OrfFwdArgs;
 struct FilterArgs;
 
-// J (nodes per lane) sets: a = 1..5, b = 6..8, c = 10,12, d = 16, e = 24, f = 32 (the last three spill part of the
-// per-node state to local memory: they exist so that models up to M = 1024 run at all, at reduced speed)
-#define BATHGPU_FOR_EACH_SET(X) X(a) X(b) X(c) X(d) X(e) X(f)
+// J (nodes per lane) sets: a = 1..5, b = 6..8, c = 10,12, d = 16, e = 24, f = 32 (the one-warp kernels of the last three spill part
+// of the per-node state to local memory: they exist so that models up to M = 1024 run at all, at reduced speed), g = 48, h = 64
+// (M <= 1536, 2048: multi-warp kernels only, J/8 warps per window or envelope at 8 nodes per lane, except the standard-translation
+// branch's one-warp kernels)
+#define BATHGPU_FOR_EACH_SET(X) X(a) X(b) X(c) X(d) X(e) X(f) X(g) X(h)
 
 #define BATHGPU_DECLARE_SET(S)                                                                                                       \
   bool launch_fs3_forward_##S(int J, bool xmx, int version, const FsParserArgs &a, int sms, cudaStream_t s, cudaError_t *err);       \
@@ -39,9 +41,9 @@ BATHGPU_FOR_EACH_SET(BATHGPU_DECLARE_SET)
 constexpr int kMwNodesPerLane = 8;
 
 // integer filters: W words (4 nodes each) per lane for MSV/SSV, P words (2 nodes each) per lane for Viterbi
-bool launch_msv_filter(int W, int P, int mode, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);
+bool launch_msv_filter(int W, int P, int mode, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);   // W = 1..4, 6, 8, 12, 16
 bool launch_vit_filter_lo(int P, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);      // P = 1..6
-bool launch_vit_filter_hi(int P, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);      // P = 8, 12, 16
+bool launch_vit_filter_hi(int P, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);      // P = 8, 12, 16, 24, 32
 // Touch the kernels a profile of this size will use, so that the driver loads their code when the profile is loaded and not
 // inside the first stage call (CUDA loads kernels lazily).
 void preload_msv_filter(int W, int P); void preload_vit_filter_lo(int P); void preload_vit_filter_hi(int P);

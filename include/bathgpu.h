@@ -94,6 +94,10 @@ int         bathgpu_create(int device, bathgpu_ctx **ret_ctx);
 void        bathgpu_destroy(bathgpu_ctx *ctx);
 const char *bathgpu_last_error(const bathgpu_ctx *ctx);
 int         bathgpu_device_info(const bathgpu_ctx *ctx, int *sm_count, int *clock_khz, size_t *total_mem);
+/* Profiles of 1025 to 2048 nodes.  A context takes profiles of up to 1024 nodes and refuses longer ones with EINVAL; with on = 1 it
+ * takes up to 2048 (the frameshift stages then run 6 or 8 warps per window or envelope, DESIGN §4.3b), with on = 0 it is back at 1024.
+ * It applies to the profiles loaded after the call. */
+int         bathgpu_set_long_models(bathgpu_ctx *ctx, int on);
 
 /* Page-locked host buffers for blocks, descriptors and results (so the copies inside the stage calls run at
  * full PCIe/C2C rate).  Any host pointer is accepted by the stage calls; pinned ones are just faster. */
