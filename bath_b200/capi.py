@@ -23,6 +23,7 @@ EXPORTS = [
     "bathgpu_bias_forward", "bathgpu_orfs_stage_breakdown", "bathgpu_measure_int16_peak", "bathgpu_orf_forward_matrices",
     "bathgpu_packed4_bytes", "bathgpu_pack_dna4", "bathgpu_upload_block_packed4", "bathgpu_fs_fwd_block_packed4",
     "bathgpu_upload_block_segments", "bathgpu_load_fs_profile_set", "bathgpu_fs_set_scores",
+    "bathgpu_load_filter_profile_set", "bathgpu_orfs_msv_screen_set", "bathgpu_orfs_fetch_set",
 ]
 
 
@@ -50,6 +51,11 @@ orf_dtype = np.dtype([("offset", "<i8"), ("L", "<i4"), ("tjb_b", "u1"), ("ssv_th
 orf_window_dtype = np.dtype([("orf", "<i4"), ("n", "<i4"), ("k", "<i4"), ("length", "<i4"), ("score", "<f4")], align=True)
 bias_item_dtype = np.dtype([("start", "<i8"), ("L", "<i4"), ("table", "<i4"), ("t00", "<f4"), ("pad_", "<i4")], align=True)
 block_dtype = np.dtype([("goff", "<i8"), ("n", "<i4"), ("C", "<i4")], align=True)
+
+
+class ScreenJob(C.Structure):
+    """bathgpu_screen_job"""
+    _fields_ = [("profile", C.c_int32), ("nblocks", C.c_int32), ("blocks", C.c_void_p), ("min_bits", C.c_double)]
 orf_hit_dtype = np.dtype([("block", "<i4"), ("index", "<i4"), ("start", "<i4"), ("end", "<i4"), ("n", "<i4"), ("frame", "<i4"),
                           ("offset", "<i8"), ("usc", "<f4"), ("status", "<i4")], align=True)
 
@@ -141,6 +147,13 @@ def load():
                                           C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     L.bathgpu_orfs_fetch.restype = C.c_int
     L.bathgpu_orfs_fetch.argtypes = [vp, vp, C.POINTER(C.c_uint8)]
+    L.bathgpu_load_filter_profile_set.restype = C.c_int
+    L.bathgpu_load_filter_profile_set.argtypes = [vp, C.c_int, vp, C.POINTER(C.POINTER(C.c_uint8))]
+    L.bathgpu_orfs_msv_screen_set.restype = C.c_int
+    L.bathgpu_orfs_msv_screen_set.argtypes = [vp, vp, C.c_int, C.c_int, C.POINTER(C.c_uint8), C.c_int, C.POINTER(C.c_uint8), fp, C.c_int,
+                                              C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    L.bathgpu_orfs_fetch_set.restype = C.c_int
+    L.bathgpu_orfs_fetch_set.argtypes = [vp, vp, C.POINTER(C.c_uint8)]
     L.bathgpu_revcomp_slot.restype = C.c_int
     L.bathgpu_revcomp_slot.argtypes = [vp, C.c_int, C.c_int]
     L.bathgpu_fs_fwd_block.restype = C.c_int
@@ -499,6 +512,39 @@ class Context:
         res = np.zeros(max(nr.value, 1), np.uint8)
         self._check(self.lib.bathgpu_orfs_fetch(self.h, hits.ctypes.data, res.ctypes.data_as(u8)))
         return per, hits[: nh.value], res[: nr.value]
+
+    def load_filter_profile_set(self, profiles):
+        """bathgpu_load_filter_profile_set: profiles = [(params dict with the FilterParams fields, rbv [29][M+1] u8), ...]"""
+        n = len(profiles)
+        prm = (FilterParams * n)(*[FilterParams(**p) for p, _ in profiles])
+        rbv = [np.ascontiguousarray(r, np.uint8) for _, r in profiles]
+        u8 = C.POINTER(C.c_uint8)
+        self._check(self.lib.bathgpu_load_filter_profile_set(self.h, n, C.cast(prm, C.c_void_p), (u8 * n)(*[r.ctypes.data_as(u8) for r in rbv])))
+
+    def orfs_msv_screen_set(self, jobs, complement, gcode, min_len, tjb_of, null_of):
+        """bathgpu_orfs_msv_screen_set + bathgpu_orfs_fetch_set over jobs = [(profile, blocks (block_dtype array), min_bits), ...]:
+        per job (ORFs found per block, survivors, the residues each survivor's offset indexes -- one buffer shared by all jobs)"""
+        n = len(jobs)
+        blocks = [np.ascontiguousarray(b, block_dtype) for _, b, _ in jobs]
+        jd = (ScreenJob * n)(*[ScreenJob(int(p), len(b), b.ctypes.data, float(mb)) for (p, _, mb), b in zip(jobs, blocks)])
+        gcode = np.ascontiguousarray(gcode, np.uint8)
+        tjb_of = np.ascontiguousarray(tjb_of, np.uint8)
+        null_of = np.ascontiguousarray(null_of, np.float32)
+        nblk = [len(b) for b in blocks]
+        per = np.zeros(max(sum(nblk), 1), np.int64)
+        nh, nr = np.zeros(n, np.int64), np.zeros(n, np.int64)
+        u8, i64 = C.POINTER(C.c_uint8), C.POINTER(C.c_int64)
+        self._check(self.lib.bathgpu_orfs_msv_screen_set(self.h, C.cast(jd, C.c_void_p), n, int(complement), gcode.ctypes.data_as(u8), int(min_len),
+                                                         tjb_of.ctypes.data_as(u8), _f(null_of), len(tjb_of) - 1, per.ctypes.data_as(i64),
+                                                         nh.ctypes.data_as(i64), nr.ctypes.data_as(i64)))
+        hits = np.zeros(max(int(nh.sum()), 1), orf_hit_dtype)
+        res = np.zeros(max(int(nr.sum()), 1), np.uint8)
+        self._check(self.lib.bathgpu_orfs_fetch_set(self.h, hits.ctypes.data, res.ctypes.data_as(u8)))
+        out, z, b0 = [], 0, 0
+        for j in range(n):
+            out.append((per[b0: b0 + nblk[j]], hits[z: z + nh[j]], res[: int(nr.sum())]))
+            z += int(nh[j]); b0 += nblk[j]
+        return out
 
     def orf_fwd_bck_xrows(self, orfs, nj=1.0, xfE=(0.5, 0.5)):
         n = len(orfs)

@@ -138,6 +138,13 @@ struct bathgpu_ctx {
   cudaEvent_t   o_ev[6] = {};                      // boundaries of the kernel groups of the last bathgpu_orfs_msv_screen call
   float         o_ms[5] = {};                      // classes, count pass, emit pass, MSV, screen
   long long     o_scored = 0, o_norf = 0;          // residues and ORFs the MSV kernel scored
+  // bathgpu_load_filter_profile_set: MSV byte tables of many profiles in one block, beside the single filter profile
+  int           fset_n = 0;
+  std::vector<int> fset_P;                          // words per lane of each profile's table (what picks the kernel)
+  DevBuf        fset_arena, fset_prof;
+  // bathgpu_orfs_msv_screen_set: jobs of the last call (0: the last screen was bathgpu_orfs_msv_screen), its tiles and survivors' jobs
+  int           o_set_njobs = 0;
+  DevBuf        o_set_jobs, o_set_tiles, o_set_hitjob, o_set_jobcnt;
   // domain stage workspace (last chunk stays resident for bathgpu_fs_fetch_domain_matrices)
   DevBuf        envs, dpp, doa, dfx, dppx, doax, dlsf, dfw, dbk, doasc, dnull2, dstat, dtoff, dtlen, dsteps, ddcell, dmxout;
   std::vector<long long> dom_xoff;
@@ -1971,6 +1978,16 @@ extern "C" int bathgpu_fs_fetch_domain_matrices(bathgpu_ctx *ctx, int e, float *
 
 // ---------------------------------------------------------------------------------------------
 // ORF-stage integer filters
+// words per lane of the byte (W) and word (P) filter tables of an M-node profile: the instantiated widths (launch.h)
+static void filter_widths(int M, int *Wp, int *Pp)
+{
+  int W = (M + 127) / 128, P = (M + 63) / 64;
+  if (W == 5) W = 6; else if (W == 7) W = 8;
+  else if (W > 8) W = (W <= 12) ? 12 : 16;
+  if (P > 6) P = (P <= 8) ? 8 : (P <= 12) ? 12 : (P <= 16) ? 16 : (P <= 24) ? 24 : 32;
+  *Wp = W; *Pp = P;
+}
+
 extern "C" int bathgpu_load_filter_profile(bathgpu_ctx *ctx, const bathgpu_filter_params *prm,
                                            const uint8_t *rbv, const int16_t *rwv, const int16_t *twv)
 {
@@ -1981,10 +1998,8 @@ extern "C" int bathgpu_load_filter_profile(bathgpu_ctx *ctx, const bathgpu_filte
   CUDA_TRY(ctx, enter(ctx));
   ctx->flt_loaded = false;
   ctx->flt = *prm;
-  int W = (M + 127) / 128, P = (M + 63) / 64;
-  if (W == 5) W = 6; else if (W == 7) W = 8;             // instantiated widths (launch.h)
-  else if (W > 8) W = (W <= 12) ? 12 : 16;
-  if (P > 6) P = (P <= 8) ? 8 : (P <= 12) ? 12 : (P <= 16) ? 16 : (P <= 24) ? 24 : 32;
+  int W, P;
+  filter_widths(M, &W, &P);
   ctx->flt_W = W; ctx->flt_P = P;
   const int nb = 128 * W, nw = 64 * P;                 // nodes per padded row
   std::vector<uint8_t> hb((size_t)29 * nb, 255);
@@ -2557,7 +2572,7 @@ extern "C" int bathgpu_orfs_msv_screen(bathgpu_ctx *ctx, const bathgpu_block *bl
   for (int b = 0; b < nblocks; ++b) sum_block_n += blocks[b].n;
   const int ntiles = (int)tile_block.size();
   *nhits = 0; *nres = 0;
-  ctx->o_nhits = 0; ctx->o_nres = 0; S.nres = 0;
+  ctx->o_nhits = 0; ctx->o_nres = 0; S.nres = 0; ctx->o_set_njobs = 0;
   if (norfs_per_block) for (int b = 0; b < nblocks; ++b) norfs_per_block[b] = 0;
   if (ntiles == 0) return BATHGPU_OK;
   CUDA_TRY(ctx, enter(ctx));
@@ -2627,7 +2642,7 @@ extern "C" int bathgpu_orfs_msv_screen(bathgpu_ctx *ctx, const bathgpu_block *bl
   ra.cls = S.cls.as<uint8_t>(); ra.descs = ctx->orfs.as<OrfDesc>(); ra.meta = ctx->o_meta.as<OrfMeta>(); ra.usc = ctx->fsc.as<float>();
   ra.status = ctx->fst.as<int>(); ra.norf = N; ra.null_of = ctx->o_null.as<float>(); ra.max_len = max_len; ra.min_bits = min_bits;
   ra.hits = ctx->o_hits.as<OrfHit>(); ra.residues = S.residues.as<uint8_t>(); ra.counters = ctx->o_counters.as<unsigned long long>();
-  orf_screen_kernel<<<(unsigned)((N + 255) / 256), 256, 0, ctx->stream>>>(ra);
+  orf_screen_kernel<false><<<(unsigned)((N + 255) / 256), 256, 0, ctx->stream>>>(ra);
   CUDA_TRY(ctx, cudaGetLastError());
   CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
   unsigned long long hc[3] = { 0, 0, 0 };
@@ -2659,6 +2674,7 @@ extern "C" int bathgpu_orfs_stage_breakdown(bathgpu_ctx *ctx, float ms[5], int64
 extern "C" int bathgpu_orfs_fetch(bathgpu_ctx *ctx, bathgpu_orf_hit *hits, uint8_t *residues)
 {
   if (!ctx || (ctx->o_nhits > 0 && (!hits || !residues))) return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_orfs_fetch");
+  if (ctx->o_set_njobs > 0) return fail(ctx, BATHGPU_EINVAL, "the last screen was a profile-set screen: fetch it with bathgpu_orfs_fetch_set");
   if (ctx->o_nhits == 0) return BATHGPU_OK;
   CUDA_TRY(ctx, enter(ctx));
   CUDA_TRY(ctx, cudaMemcpyAsync(hits, ctx->o_hits.p, (size_t)ctx->o_nhits * sizeof(OrfHit), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2666,5 +2682,295 @@ extern "C" int bathgpu_orfs_fetch(bathgpu_ctx *ctx, bathgpu_orf_hit *hits, uint8
   CUDA_TRY(ctx, wait_stream(ctx));
   std::sort(hits, hits + ctx->o_nhits, [](const bathgpu_orf_hit &x, const bathgpu_orf_hit &y) {
     return x.block != y.block ? x.block < y.block : x.index < y.index; });
+  return BATHGPU_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// f1 over a profile set (bathgpu_load_filter_profile_set, bathgpu_orfs_msv_screen_set, bathgpu_orfs_fetch_set)
+extern "C" int bathgpu_load_filter_profile_set(bathgpu_ctx *ctx, int n, const bathgpu_filter_params *prm, const uint8_t *const *rbv)
+{
+  if (!ctx || n < 1 || !prm || !rbv) return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_load_filter_profile_set");
+  for (int p = 0; p < n; ++p) {
+    if (!rbv[p] || prm[p].M < 1) return fail(ctx, BATHGPU_EINVAL, "profile %d of the filter set: bad arguments", p);
+    if (check_model_length(ctx, prm[p].M) != BATHGPU_OK) return BATHGPU_EINVAL;
+  }
+  CUDA_TRY(ctx, enter(ctx));
+  ctx->fset_n = 0;
+  ctx->fset_P.assign((size_t)n, 0);
+  std::vector<size_t> off((size_t)n + 1, 0);             // int16 entries before each profile's table
+  for (int p = 0; p < n; ++p) {
+    int W, P;
+    filter_widths(prm[p].M, &W, &P);
+    ctx->fset_P[p] = P;
+    off[p + 1] = off[p] + (size_t)29 * 64 * P;
+  }
+  if (ctx->fset_arena.reserve(off[n] * 2) != BATHGPU_OK || ctx->fset_prof.reserve((size_t)n * sizeof(MsvSetProfile)) != BATHGPU_OK)
+    return fail(ctx, BATHGPU_EMEM, "a filter profile set of %d profiles (%zu bytes) does not fit on the device", n, off[n] * 2);
+  // the table bathgpu_load_filter_profile builds for msv16_filter_kernel (f_nrb), profile after profile
+  std::vector<int16_t> hn(off[n], -255);
+  std::vector<MsvSetProfile> prof((size_t)n);
+  for (int p = 0; p < n; ++p) {
+    const int M = prm[p].M, ld = M + 1, nw = 64 * ctx->fset_P[p];
+    for (int x = 0; x < 29; ++x)
+      for (int k = 1; k <= M; ++k) hn[off[p] + (size_t)x * nw + (k - 1)] = (int16_t)(-(int)rbv[p][(size_t)x * ld + k]);
+    MsvSetProfile &q = prof[p];
+    q.nrb = reinterpret_cast<const uint32_t *>(ctx->fset_arena.as<int16_t>() + off[p]); q.P = ctx->fset_P[p];
+    q.tbm_b = prm[p].tbm_b; q.tec_b = prm[p].tec_b; q.base_b = prm[p].base_b; q.bias_b = prm[p].bias_b; q.scale_b = prm[p].scale_b;
+  }
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->fset_arena.p, hn.data(), off[n] * 2, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->fset_prof.p, prof.data(), (size_t)n * sizeof(MsvSetProfile), cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, wait_stream(ctx));
+  ctx->fset_n = n;
+  for (int p = 0; p < n; ++p) preload_msv_filter(0, ctx->fset_P[p]);
+  return BATHGPU_OK;
+}
+
+extern "C" int bathgpu_orfs_msv_screen_set(bathgpu_ctx *ctx, const bathgpu_screen_job *jobs, int njobs, int complement, const uint8_t gcode[64],
+                                           int min_len, const uint8_t *tjb_of, const float *null_of, int max_len,
+                                           int64_t *norfs_per_block, int64_t *nhits, int64_t *nres)
+{
+  if (!ctx || !jobs || njobs < 1 || !gcode || min_len < 1 || !tjb_of || !null_of || max_len < 1 || !nhits || !nres)
+    return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_orfs_msv_screen_set");
+  if (njobs > BATHGPU_SCREEN_SET_MAX_JOBS) return fail(ctx, BATHGPU_EINVAL, "%d jobs in one call: at most %d", njobs, BATHGPU_SCREEN_SET_MAX_JOBS);
+  if (ctx->fset_n == 0) return fail(ctx, BATHGPU_EINVAL, "filter profile set not loaded");
+  TargetSlot &S = ctx->S();
+  if (S.block_n == 0) return fail(ctx, BATHGPU_EINVAL, "no block uploaded");
+  for (int j = 0; j < njobs; ++j) {
+    if (jobs[j].profile < 0 || jobs[j].profile >= ctx->fset_n || jobs[j].nblocks < 1 || !jobs[j].blocks)
+      return fail(ctx, BATHGPU_EINVAL, "job %d: profile %d of %d, %d blocks", j, jobs[j].profile, ctx->fset_n, jobs[j].nblocks);
+    for (int b = 0; b < jobs[j].nblocks; ++b) {
+      const bathgpu_block &bk = jobs[j].blocks[b];
+      if (bk.n < 0 || bk.goff < 0 || bk.goff + bk.n > S.block_n)
+        return fail(ctx, BATHGPU_EINVAL, "job %d block %d (offset %lld, n %d) is outside the uploaded sequence (n=%lld)", j, b, (long long)bk.goff, bk.n, (long long)S.block_n);
+    }
+  }
+  BulkScope bulk(ctx);
+  // the distinct block layouts among the jobs: ORFs are found once per layout
+  struct Layout { int job, nblocks; long long blk0, tile0, ntiles, sum_n, desc0 = 0, norf = 0; int njobs = 0; };
+  std::vector<Layout> lay;
+  std::vector<int> layout_of((size_t)njobs);
+  std::vector<int> tile_block, tile_p0;
+  std::vector<long long> first_tile;                     // per concatenated block, + one past the last block of each layout
+  std::vector<BlockDesc> blocks;
+  for (int j = 0; j < njobs; ++j) {
+    int l = 0;
+    for (; l < (int)lay.size(); ++l) {
+      const bathgpu_screen_job &r = jobs[lay[l].job];
+      if (r.nblocks == jobs[j].nblocks && memcmp(r.blocks, jobs[j].blocks, (size_t)r.nblocks * sizeof(bathgpu_block)) == 0) break;
+    }
+    layout_of[j] = l;
+    if (l < (int)lay.size()) { lay[l].njobs++; continue; }
+    Layout L; L.job = j; L.nblocks = jobs[j].nblocks; L.blk0 = (long long)blocks.size(); L.tile0 = (long long)tile_block.size(); L.sum_n = 0; L.njobs = 1;
+    for (int b = 0; b < L.nblocks; ++b) {
+      const bathgpu_block &bk = jobs[j].blocks[b];
+      blocks.push_back(BlockDesc{ bk.goff, bk.n, bk.C });
+      first_tile.push_back((long long)tile_block.size() - L.tile0);
+      if (bk.n >= 3)
+        for (int p0 = 1; p0 <= bk.n + 1; p0 += kOrfTile) { tile_block.push_back(b); tile_p0.push_back(p0); }
+      L.sum_n += bk.n;
+    }
+    L.ntiles = (long long)tile_block.size() - L.tile0;
+    lay.push_back(L);
+  }
+  long long nblk_out = 0;
+  for (int j = 0; j < njobs; ++j) { nhits[j] = 0; nres[j] = 0; nblk_out += jobs[j].nblocks; }
+  if (norfs_per_block) for (long long b = 0; b < nblk_out; ++b) norfs_per_block[b] = 0;
+  ctx->o_nhits = 0; ctx->o_nres = 0; S.nres = 0; ctx->o_set_njobs = njobs;
+  const int ntiles = (int)tile_block.size(), nl = (int)lay.size();
+  if (ntiles == 0) return BATHGPU_OK;
+  CUDA_TRY(ctx, enter(ctx));
+  const long long n = S.block_n;
+  if (S.cls.reserve((size_t)n + 64) != BATHGPU_OK || ctx->o_tiles.reserve((size_t)ntiles * 8) != BATHGPU_OK || ctx->o_cnt.reserve((size_t)ntiles * 4) != BATHGPU_OK ||
+      ctx->o_base.reserve((size_t)ntiles * 8) != BATHGPU_OK || ctx->o_blocks.reserve(blocks.size() * sizeof(BlockDesc)) != BATHGPU_OK ||
+      ctx->o_first.reserve(blocks.size() * 8) != BATHGPU_OK || ctx->o_tjb.reserve((size_t)max_len + 1) != BATHGPU_OK ||
+      ctx->o_null.reserve(((size_t)max_len + 1) * 4) != BATHGPU_OK || ctx->o_counters.reserve((size_t)(4 + nl) * 8) != BATHGPU_OK ||
+      ctx->counter.reserve(64) != BATHGPU_OK || ctx->o_set_jobcnt.reserve((size_t)njobs * 16) != BATHGPU_OK ||
+      ctx->o_set_jobs.reserve((size_t)njobs * sizeof(ScreenSetJob)) != BATHGPU_OK)
+    return fail(ctx, BATHGPU_EMEM, "device allocation failed");
+  int *d_tile_block = ctx->o_tiles.as<int>(), *d_tile_p0 = ctx->o_tiles.as<int>() + ntiles;
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_tile_block, tile_block.data(), (size_t)ntiles * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_tile_p0, tile_p0.data(), (size_t)ntiles * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->o_blocks.p, blocks.data(), blocks.size() * sizeof(BlockDesc), cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->o_tjb.p, tjb_of, (size_t)max_len + 1, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->o_null.p, null_of, ((size_t)max_len + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  if (!ctx->o_ev[0]) for (auto &e : ctx->o_ev) CUDA_TRY(ctx, cudaEventCreate(&e));
+  for (float &m : ctx->o_ms) m = 0.f;
+  ctx->o_scored = 0; ctx->o_norf = 0;
+  GeneticCode gc;
+  memcpy(gc.aa, gcode, 64);
+  // codon classes once for every job
+  CUDA_TRY(ctx, cudaEventRecord(ctx->o_ev[0], ctx->stream));
+  {
+    const long long nthreads = (n + 7) / 8;
+    codon_class_kernel<<<(unsigned)((nthreads + 255) / 256), 256, 0, ctx->stream>>>(S.dna4.as<uint32_t>(), n, gc, S.cls.as<uint8_t>());
+  }
+  CUDA_TRY(ctx, cudaEventRecord(ctx->o_ev[1], ctx->stream));
+  auto scan_args = [&](const Layout &L) {
+    OrfScanArgs sa{};
+    sa.cls = S.cls.as<uint8_t>(); sa.blocks = ctx->o_blocks.as<BlockDesc>() + L.blk0; sa.tile_block = d_tile_block + L.tile0; sa.tile_p0 = d_tile_p0 + L.tile0;
+    sa.ntiles = (int)L.ntiles; sa.min_len = min_len; sa.complement = complement; sa.tile_cnt = ctx->o_cnt.as<int>() + L.tile0;
+    return sa;
+  };
+  for (const Layout &L : lay) {                           // ORF count pass, once per layout
+    if (L.ntiles == 0) continue;
+    OrfScanArgs sa = scan_args(L);
+    orf_scan_kernel<false><<<(unsigned)L.ntiles, kOrfTileThreads, 0, ctx->stream>>>(sa);
+    CUDA_TRY(ctx, cudaGetLastError());
+  }
+  CUDA_TRY(ctx, cudaEventRecord(ctx->o_ev[2], ctx->stream));
+  std::vector<int> cnt((size_t)ntiles);
+  CUDA_TRY(ctx, cudaMemcpyAsync(cnt.data(), ctx->o_cnt.p, (size_t)ntiles * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, wait_stream(ctx));
+  std::vector<long long> base((size_t)ntiles, 0), bfirst(blocks.size(), 0);   // per layout, from 0
+  long long Nd = 0;
+  for (Layout &L : lay) {
+    long long acc = 0;
+    for (long long t = 0; t < L.ntiles; ++t) { base[(size_t)(L.tile0 + t)] = acc; acc += cnt[(size_t)(L.tile0 + t)]; }
+    for (int b = 0; b < L.nblocks; ++b) {
+      const long long ft = first_tile[(size_t)(L.blk0 + b)];
+      bfirst[(size_t)(L.blk0 + b)] = (ft < L.ntiles) ? base[(size_t)(L.tile0 + ft)] : acc;
+    }
+    L.desc0 = Nd; L.norf = acc; Nd += acc;
+  }
+  // ORFs per block of each job, and the (job, ORF) items in job order
+  std::vector<long long> item0((size_t)njobs + 1, 0);
+  {
+    long long ob = 0;
+    for (int j = 0; j < njobs; ++j) {
+      const Layout &L = lay[(size_t)layout_of[j]];
+      if (norfs_per_block)
+        for (int b = 0; b < L.nblocks; ++b) {
+          const long long hi = (b + 1 < L.nblocks) ? bfirst[(size_t)(L.blk0 + b + 1)] : L.norf;
+          norfs_per_block[ob + b] = hi - bfirst[(size_t)(L.blk0 + b)];
+        }
+      ob += L.nblocks;
+      item0[(size_t)j + 1] = item0[(size_t)j] + L.norf;
+    }
+  }
+  const long long items = item0[(size_t)njobs];
+  if (Nd == 0) return BATHGPU_OK;
+  if (Nd > 0x7fffffffLL) return fail(ctx, BATHGPU_EINVAL, "%lld ORFs in one call: split the sequence", Nd);
+  if (items > BATHGPU_SCREEN_SET_MAX_ITEMS)
+    return fail(ctx, BATHGPU_EMEM, "%lld (job, ORF) pairs in one call: at most %lld; split the jobs", items, (long long)BATHGPU_SCREEN_SET_MAX_ITEMS);
+  if (ctx->orfs.reserve((size_t)Nd * sizeof(OrfDesc)) != BATHGPU_OK || ctx->o_meta.reserve((size_t)Nd * sizeof(OrfMeta)) != BATHGPU_OK ||
+      ctx->fsc.reserve((size_t)items * 4) != BATHGPU_OK || ctx->fst.reserve((size_t)items * 4) != BATHGPU_OK)
+    return fail(ctx, BATHGPU_EMEM, "device allocation failed for %lld ORFs of %d jobs", Nd, njobs);
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->o_base.p, base.data(), (size_t)ntiles * 8, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->o_first.p, bfirst.data(), bfirst.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, cudaMemsetAsync(ctx->o_counters.p, 0, (size_t)(4 + nl) * 8, ctx->stream));
+  CUDA_TRY(ctx, cudaEventRecord(ctx->o_ev[5], ctx->stream));
+  for (int l = 0; l < nl; ++l) {                          // ORF emit pass, once per layout
+    const Layout &L = lay[(size_t)l];
+    if (L.norf == 0) continue;
+    OrfScanArgs sa = scan_args(L);
+    sa.tile_base = ctx->o_base.as<long long>() + L.tile0; sa.block_first = ctx->o_first.as<long long>() + L.blk0; sa.tjb_of = ctx->o_tjb.as<uint8_t>();
+    sa.max_len = max_len; sa.descs = ctx->orfs.as<OrfDesc>() + L.desc0; sa.meta = ctx->o_meta.as<OrfMeta>() + L.desc0;
+    sa.scored = ctx->o_counters.as<unsigned long long>() + 4 + l;
+    orf_scan_kernel<true><<<(unsigned)L.ntiles, kOrfTileThreads, 0, ctx->stream>>>(sa);
+    CUDA_TRY(ctx, cudaGetLastError());
+  }
+  CUDA_TRY(ctx, cudaEventRecord(ctx->o_ev[3], ctx->stream));
+  // MSV: one launch per table width over every (job, ORF) pair of the jobs whose profile has that width
+  std::vector<MsvSetTile> tiles;
+  std::vector<std::pair<int, std::pair<size_t, size_t>>> groups;      // P, tile range
+  {
+    std::vector<int> widths;
+    for (int j = 0; j < njobs; ++j) widths.push_back(ctx->fset_P[jobs[j].profile]);
+    std::sort(widths.begin(), widths.end());
+    widths.erase(std::unique(widths.begin(), widths.end()), widths.end());
+    for (int P : widths) {
+      const size_t t0 = tiles.size();
+      for (int j = 0; j < njobs; ++j) {
+        if (ctx->fset_P[jobs[j].profile] != P) continue;
+        const Layout &L = lay[(size_t)layout_of[j]];
+        for (long long o0 = 0; o0 < L.norf; o0 += kMsvSetTileOrfs)
+          tiles.push_back(MsvSetTile{ jobs[j].profile, (int)std::min<long long>(kMsvSetTileOrfs, L.norf - o0), L.desc0 + o0, item0[(size_t)j] + o0 });
+      }
+      if (tiles.size() > t0) groups.push_back({ P, { t0, tiles.size() } });
+    }
+  }
+  if (ctx->o_set_tiles.reserve(tiles.size() * sizeof(MsvSetTile)) != BATHGPU_OK) return fail(ctx, BATHGPU_EMEM, "device allocation failed");
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->o_set_tiles.p, tiles.data(), tiles.size() * sizeof(MsvSetTile), cudaMemcpyHostToDevice, ctx->stream));
+  for (const auto &g : groups) {
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->counter.p, 0, 4, ctx->stream));
+    FilterArgs fa{};
+    fa.residues = S.cls.as<uint8_t>(); fa.res_stride = 3; fa.orfs = ctx->orfs.as<OrfDesc>(); fa.norf = 0;
+    fa.sc = ctx->fsc.as<float>(); fa.status = ctx->fst.as<int>(); fa.counter = ctx->counter.as<int>();
+    fa.set_tiles = ctx->o_set_tiles.as<MsvSetTile>() + g.second.first; fa.set_ntiles = (int)(g.second.second - g.second.first);
+    fa.set_profiles = ctx->fset_prof.as<MsvSetProfile>();
+    cudaError_t e = cudaErrorInvalidValue;
+    if (!launch_msv16_set(g.first, fa, ctx->prop.multiProcessorCount, ctx->stream, &e)) return fail(ctx, BATHGPU_EINVAL, "no MSV kernel for %d words per lane", g.first);
+    CUDA_TRY(ctx, e);
+  }
+  CUDA_TRY(ctx, cudaEventRecord(ctx->o_ev[4], ctx->stream));
+  // F1 screen + residue gather over every item in one launch; the survivor buffers start at what one profile would need and grow once
+  // if the jobs together keep more
+  std::vector<ScreenSetJob> sj((size_t)njobs);
+  for (int j = 0; j < njobs; ++j) sj[(size_t)j] = ScreenSetJob{ item0[(size_t)j], lay[(size_t)layout_of[j]].desc0, jobs[j].min_bits };
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->o_set_jobs.p, sj.data(), sj.size() * sizeof(ScreenSetJob), cudaMemcpyHostToDevice, ctx->stream));
+  long long max_sum_n = 0;
+  for (const Layout &L : lay) max_sum_n = std::max(max_sum_n, L.sum_n);
+  unsigned long long cap_hits = (unsigned long long)std::max<long long>(Nd, 1), cap_res = (unsigned long long)(max_sum_n / 3 * 3);
+  unsigned long long hc[3] = { 0, 0, 0 };
+  for (int pass = 0; pass < 2; ++pass) {
+    if (ctx->o_hits.reserve((size_t)cap_hits * sizeof(OrfHit)) != BATHGPU_OK || ctx->o_set_hitjob.reserve((size_t)cap_hits * 4) != BATHGPU_OK ||
+        S.residues.reserve((size_t)cap_res + 64) != BATHGPU_OK)
+      return fail(ctx, BATHGPU_EMEM, "device allocation failed for the survivors of %d jobs", njobs);
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->o_counters.p, 0, 16, ctx->stream));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->o_set_jobcnt.p, 0, (size_t)njobs * 16, ctx->stream));
+    OrfScreenArgs ra{};
+    ra.cls = S.cls.as<uint8_t>(); ra.descs = ctx->orfs.as<OrfDesc>(); ra.meta = ctx->o_meta.as<OrfMeta>(); ra.usc = ctx->fsc.as<float>();
+    ra.status = ctx->fst.as<int>(); ra.norf = items; ra.null_of = ctx->o_null.as<float>(); ra.max_len = max_len;
+    ra.hits = ctx->o_hits.as<OrfHit>(); ra.residues = S.residues.as<uint8_t>(); ra.counters = ctx->o_counters.as<unsigned long long>();
+    ra.jobs = ctx->o_set_jobs.as<ScreenSetJob>(); ra.njobs = njobs; ra.hit_job = ctx->o_set_hitjob.as<int>();
+    ra.job_counters = ctx->o_set_jobcnt.as<unsigned long long>(); ra.max_hits = cap_hits; ra.max_res = cap_res;
+    orf_screen_kernel<true><<<(unsigned)((items + 255) / 256), 256, 0, ctx->stream>>>(ra);
+    CUDA_TRY(ctx, cudaGetLastError());
+    CUDA_TRY(ctx, cudaMemcpyAsync(hc, ctx->o_counters.p, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, wait_stream(ctx));
+    if (hc[0] <= cap_hits && hc[1] <= cap_res) break;
+    if (pass == 1) return fail(ctx, BATHGPU_ECUDA, "survivor count changed between two runs of the screen");
+    cap_hits = std::max(cap_hits, hc[0]); cap_res = std::max(cap_res, hc[1]);
+  }
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  std::vector<unsigned long long> jc((size_t)njobs * 2), scored((size_t)nl);
+  CUDA_TRY(ctx, cudaMemcpyAsync(jc.data(), ctx->o_set_jobcnt.p, jc.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(scored.data(), ctx->o_counters.as<unsigned long long>() + 4, (size_t)nl * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, wait_stream(ctx));
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ctx->o_ms[0], ctx->o_ev[0], ctx->o_ev[1]));
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ctx->o_ms[1], ctx->o_ev[1], ctx->o_ev[2]));
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ctx->o_ms[2], ctx->o_ev[5], ctx->o_ev[3]));
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ctx->o_ms[3], ctx->o_ev[3], ctx->o_ev[4]));
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ctx->o_ms[4], ctx->o_ev[4], ctx->ev1));
+  for (int l = 0; l < nl; ++l) ctx->o_scored += (long long)scored[(size_t)l] * lay[(size_t)l].njobs;
+  ctx->o_norf = items;
+  ctx->last_launches = 1 + 2 * nl + (int)groups.size() + 1;
+  ctx->o_nhits = (long long)hc[0]; ctx->o_nres = (long long)hc[1];
+  S.nres = (int64_t)hc[1];
+  for (int j = 0; j < njobs; ++j) { nhits[j] = (int64_t)jc[(size_t)2 * j]; nres[j] = (int64_t)jc[(size_t)2 * j + 1]; }
+  return BATHGPU_OK;
+}
+
+extern "C" int bathgpu_orfs_fetch_set(bathgpu_ctx *ctx, bathgpu_orf_hit *hits, uint8_t *residues)
+{
+  if (!ctx || ctx->o_set_njobs == 0) return fail(ctx, BATHGPU_EINVAL, "no profile-set screen to fetch");
+  if (ctx->o_nhits > 0 && (!hits || !residues)) return fail(ctx, BATHGPU_EINVAL, "bad arguments to bathgpu_orfs_fetch_set");
+  if (ctx->o_nhits == 0) return BATHGPU_OK;
+  CUDA_TRY(ctx, enter(ctx));
+  const size_t nh = (size_t)ctx->o_nhits;
+  std::vector<bathgpu_orf_hit> h(nh);
+  std::vector<int> job(nh);
+  CUDA_TRY(ctx, cudaMemcpyAsync(h.data(), ctx->o_hits.p, nh * sizeof(OrfHit), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(job.data(), ctx->o_set_hitjob.p, nh * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaMemcpyAsync(residues, ctx->S().residues.p, (size_t)ctx->o_nres, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, wait_stream(ctx));
+  std::vector<uint32_t> ord(nh);
+  for (size_t z = 0; z < nh; ++z) ord[z] = (uint32_t)z;
+  std::sort(ord.begin(), ord.end(), [&](uint32_t x, uint32_t y) {
+    if (job[x] != job[y]) return job[x] < job[y];
+    return h[x].block != h[y].block ? h[x].block < h[y].block : h[x].index < h[y].index; });
+  for (size_t z = 0; z < nh; ++z) hits[z] = h[ord[z]];
   return BATHGPU_OK;
 }

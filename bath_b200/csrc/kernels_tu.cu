@@ -380,14 +380,15 @@ template <int W, int MODE> static cudaError_t run_msv(const FilterArgs &a, int s
   msv_filter_kernel<W, MODE><<<grid_for(msv_filter_kernel<W, MODE>, 128, smem, (a.norf + 3) / 4, sms), 128, smem, s>>>(a);
   return cudaGetLastError();
 }
-template <int P> static cudaError_t run_msv16(const FilterArgs &a, int sms, cudaStream_t s)
+template <int P, bool SET = false> static cudaError_t run_msv16(const FilterArgs &a, int sms, cudaStream_t s)
 {
   const size_t smem = (size_t)29 * 32 * P * 4;
   if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(msv16_filter_kernel<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(msv16_filter_kernel<P, SET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
-  msv16_filter_kernel<P><<<grid_for(msv16_filter_kernel<P>, 128, smem, (a.norf + 3) / 4, sms), 128, smem, s>>>(a);
+  const int need = SET ? a.set_ntiles : (a.norf + 3) / 4;
+  msv16_filter_kernel<P, SET><<<grid_for(msv16_filter_kernel<P, SET>, 128, smem, need, sms), 128, smem, s>>>(a);
   return cudaGetLastError();
 }
 // mode 0: MSV scores (16-bit lanes, P words per lane); mode 1: SSV windows (byte lanes, W words per lane)
@@ -408,6 +409,16 @@ bool launch_msv_filter(int W, int P, int mode, const FilterArgs &a, int sms, cud
   default: return false;
   }
 }
+// MSV scores over the tiles of a profile-set screen (a.set_tiles), all of whose profiles have P words per lane
+bool launch_msv16_set(int P, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err)
+{
+  switch (P) {
+#define X(P_) case P_: *err = run_msv16<P_, true>(a, sms, s); return true;
+  X(1) X(2) X(3) X(4) X(5) X(6) X(8) X(12) X(16) X(24) X(32)
+#undef X
+  default: return false;
+  }
+}
 void preload_msv_filter(int W, int P)
 {
   switch (W) {
@@ -417,7 +428,7 @@ void preload_msv_filter(int W, int P)
   default: break;
   }
   switch (P) {
-#define X(P_) case P_: touch(msv16_filter_kernel<P_>); break;
+#define X(P_) case P_: touch(msv16_filter_kernel<P_, false>); touch(msv16_filter_kernel<P_, true>); break;
   X(1) X(2) X(3) X(4) X(5) X(6) X(8) X(12) X(16) X(24) X(32)
 #undef X
   default: break;

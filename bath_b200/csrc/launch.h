@@ -42,6 +42,7 @@ constexpr int kMwNodesPerLane = 8;
 
 // integer filters: W words (4 nodes each) per lane for MSV/SSV, P words (2 nodes each) per lane for Viterbi
 bool launch_msv_filter(int W, int P, int mode, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);   // W = 1..4, 6, 8, 12, 16
+bool launch_msv16_set(int P, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);                   // P as launch_msv_filter's
 bool launch_vit_filter_lo(int P, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);      // P = 1..6
 bool launch_vit_filter_hi(int P, const FilterArgs &a, int sms, cudaStream_t s, cudaError_t *err);      // P = 8, 12, 16, 24, 32
 // Touch the kernels a profile of this size will use, so that the driver loads their code when the profile is loaded and not

@@ -37,6 +37,8 @@ struct OrfDesc {           // device copy of bathgpu_orf
 };
 
 struct WindowRec { int orf, n, k, length; float score; };
+struct MsvSetProfile;
+struct MsvSetTile;
 
 struct FilterArgs {
   const uint8_t  *residues;
@@ -66,6 +68,10 @@ struct FilterArgs {
   int            *nwins;
   int             max_wins;
   int            *counter;
+  // msv16_filter_kernel<P, true>: the tiles of a profile-set screen and the set's profiles
+  const MsvSetTile    *set_tiles;
+  int                  set_ntiles;
+  const MsvSetProfile *set_profiles;
 };
 
 __device__ __forceinline__ unsigned bytemax(unsigned v) { v = __vmaxu4(v, v >> 16); v = __vmaxu4(v, v >> 8); return v & 0xffu; }
@@ -248,34 +254,35 @@ __device__ __forceinline__ void msv16_row(const uint32_t *__restrict__ s_nrb_lan
   }
 }
 
+// A profile of a resident set (bathgpu_load_filter_profile_set): its MSV cost table and the byte parameters the recurrence reads.
+struct MsvSetProfile {
+  const uint32_t *nrb;       // [29][32*P] words, as FilterArgs::nrb
+  int             P;
+  int             tbm_b, tec_b, base_b, bias_b;
+  float           scale_b;
+};
+// A run of consecutive ORFs of one job of bathgpu_orfs_msv_screen_set, all scored with one profile: descriptors orfs[desc0 ..
+// desc0 + n - 1], scores written to sc[out0 ..].
+struct MsvSetTile { int profile, n; long long desc0, out0; };
+constexpr int kMsvSetTileOrfs = 256;
+
+// One ORF of the MSV recurrence on 16-bit lanes: its score and status (meaningful in lane 0).
 // Rows are taken 32 at a time (one residue per lane).  While the J state is out of reach -- E never exceeds base + tEC, so B keeps
 // its initial value -- the per-row maximum is not needed row by row: a chunk runs without any reduction and its overall maximum is
 // reduced once (this is the reference's SSV shortcut, ssvfilter.c:14-210, taken per chunk).  A chunk whose maximum shows that J
 // became reachable or that a cell overflowed is re-run from its saved first row with the exact per-row recurrence (msvfilter.c:145-201).
 template <int P>
-__global__ void __launch_bounds__(128) msv16_filter_kernel(FilterArgs a)
+__device__ __forceinline__ void msv16_orf(const FilterArgs &a, const OrfDesc &od, const uint32_t *__restrict__ s_nrb_lane, int lane,
+                                          float &sc_out, int &st_out)
 {
-  extern __shared__ uint32_t smem[];
-  uint32_t *s_nrb = smem;                                  // [29][32*P] words: -cost of node k at half k-1
   const int rowwords = 32 * P;
-  for (int t = threadIdx.x; t < 29 * rowwords; t += blockDim.x) s_nrb[t] = a.nrb[t];
-  __syncthreads();
-
-  const int lane = threadIdx.x & 31;
   const unsigned full = 0xffffffffu;
   const unsigned biasv = (unsigned)a.bias_b * 0x00010001u;
-  const uint32_t *s_nrb_lane = s_nrb + lane * P;
-
-  for (;;) {
-    int o = 0;
-    if (lane == 0) o = atomicAdd(a.counter, 1);
-    o = __shfl_sync(full, o, 0);
-    if (o >= a.norf) break;
-    const OrfDesc od = a.orfs[o];
+  {
     const int L = od.L;
     if (od.flags & 2) {                                    // wholly inside the block's overlap context: not scored (p7_pipeline.c:1634-1637)
-      if (lane == 0) { a.sc[o] = -INFINITY; a.status[o] = 0; }
-      continue;
+      sc_out = -INFINITY; st_out = 0;
+      return;
     }
     const int tjbm = (int)(uint8_t)((int8_t)od.tjb_b + (int8_t)a.tbm_b);      // set1_epi8 of the 8-bit sum (:120)
     uint32_t m[P];
@@ -314,17 +321,72 @@ __global__ void __launch_bounds__(128) msv16_filter_kernel(FilterArgs a)
         xBv = (unsigned)xB * 0x00010001u;
       }
     }
-    if (lane == 0) {
-      float sc;
-      if (st) sc = INFINITY;
-      else {                                                 // (:203-205), with the SSV shortcut's floor (see msv_filter_kernel)
-        const int floorJ = a.base_b - (int)od.tjb_b - a.tbm_b - a.tec_b;
-        if ((int)od.tjb_b + a.tbm_b + a.tec_b + a.bias_b < 127 && xJ <= a.base_b && floorJ >= 0) xJ = max(xJ, floorJ);
-        sc = ((float)(xJ - (int)od.tjb_b) - (float)a.base_b);
-        sc /= a.scale_b;
-        sc -= 3.0f;
+    float sc;
+    if (st) sc = INFINITY;
+    else {                                                   // (:203-205), with the SSV shortcut's floor (see msv_filter_kernel)
+      const int floorJ = a.base_b - (int)od.tjb_b - a.tbm_b - a.tec_b;
+      if ((int)od.tjb_b + a.tbm_b + a.tec_b + a.bias_b < 127 && xJ <= a.base_b && floorJ >= 0) xJ = max(xJ, floorJ);
+      sc = ((float)(xJ - (int)od.tjb_b) - (float)a.base_b);
+      sc /= a.scale_b;
+      sc -= 3.0f;
+    }
+    sc_out = sc; st_out = st;
+  }
+}
+
+// MSV scores of the ORFs a.orfs[0 .. norf-1] with the loaded profile (SET = false), or of the (job, ORF) runs a.set_tiles with the
+// profiles of a resident set (SET = true): a block takes a tile, stages the tile's profile table unless it holds it already, and its
+// warps take the tile's ORFs one at a time.  Both run the same recurrence (msv16_orf) on the same tables, so the scores are the same.
+template <int P, bool SET>
+__global__ void __launch_bounds__(128) msv16_filter_kernel(FilterArgs a)
+{
+  extern __shared__ uint32_t smem[];
+  uint32_t *s_nrb = smem;                                  // [29][32*P] words: -cost of node k at half k-1
+  const int rowwords = 32 * P;
+  const int lane = threadIdx.x & 31;
+  const unsigned full = 0xffffffffu;
+  const uint32_t *s_nrb_lane = s_nrb + lane * P;
+  if constexpr (!SET) {
+    for (int t = threadIdx.x; t < 29 * rowwords; t += blockDim.x) s_nrb[t] = a.nrb[t];
+    __syncthreads();
+    for (;;) {
+      int o = 0;
+      if (lane == 0) o = atomicAdd(a.counter, 1);
+      o = __shfl_sync(full, o, 0);
+      if (o >= a.norf) break;
+      const OrfDesc od = a.orfs[o];
+      float sc; int st;
+      msv16_orf<P>(a, od, s_nrb_lane, lane, sc, st);
+      if (lane == 0) { a.sc[o] = sc; a.status[o] = st; }
+    }
+  } else {
+    __shared__ int s_tile, s_next;
+    int staged = -1;
+    for (;;) {
+      if (threadIdx.x == 0) { s_tile = atomicAdd(a.counter, 1); s_next = 0; }
+      __syncthreads();
+      const int t = s_tile;
+      if (t >= a.set_ntiles) break;
+      const MsvSetTile tl = a.set_tiles[t];
+      const MsvSetProfile pr = a.set_profiles[tl.profile];
+      if (tl.profile != staged) {                          // every thread sees the same tiles: the block agrees on `staged`
+        for (int z = threadIdx.x; z < 29 * rowwords; z += blockDim.x) s_nrb[z] = pr.nrb[z];
+        staged = tl.profile;
       }
-      a.sc[o] = sc; a.status[o] = st;
+      __syncthreads();
+      FilterArgs pa = a;
+      pa.tbm_b = pr.tbm_b; pa.tec_b = pr.tec_b; pa.base_b = pr.base_b; pa.bias_b = pr.bias_b; pa.scale_b = pr.scale_b;
+      for (;;) {
+        int j = 0;
+        if (lane == 0) j = atomicAdd(&s_next, 1);
+        j = __shfl_sync(full, j, 0);
+        if (j >= tl.n) break;
+        const OrfDesc od = a.orfs[tl.desc0 + j];
+        float sc; int st;
+        msv16_orf<P>(pa, od, s_nrb_lane, lane, sc, st);
+        if (lane == 0) { a.sc[tl.out0 + j] = sc; a.status[tl.out0 + j] = st; }
+      }
+      __syncthreads();                                     // the tile and the table stay until every warp is done with them
     }
   }
 }

@@ -187,6 +187,8 @@ __global__ void __launch_bounds__(kOrfTileThreads) orf_scan_kernel(OrfScanArgs a
   }
 }
 
+struct ScreenSetJob { long long item0, desc0; double min_bits; };    // one job of bathgpu_orfs_msv_screen_set, in item order
+
 struct OrfScreenArgs {
   const uint8_t  *cls;
   const OrfDesc  *descs;
@@ -200,23 +202,47 @@ struct OrfScreenArgs {
   OrfHit         *hits;
   uint8_t        *residues;     // unit stride, survivors only
   unsigned long long *counters; // [0] hits, [1] residues
+  // orf_screen_kernel<true> (bathgpu_orfs_msv_screen_set): item r is ORF r - item0 of job j's layout, whose descriptors start at
+  // desc0; survivors past max_hits / max_res are counted, not written (the caller grows the buffers and runs the kernel again)
+  const ScreenSetJob *jobs;
+  int             njobs;
+  int            *hit_job;      // [max_hits] job of each survivor
+  unsigned long long *job_counters;   // [2 njobs] survivors and residues per job
+  unsigned long long max_hits, max_res;
 };
 
+template <bool SET>
 __global__ void __launch_bounds__(256) orf_screen_kernel(OrfScreenArgs a)
 {
   const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= a.norf) return;
-  const OrfDesc d = a.descs[r];
+  long long di = r;
+  int job = 0;
+  double min_bits = a.min_bits;
+  if constexpr (SET) {
+    int lo = 0, hi = a.njobs - 1;                         // last job whose first item is <= r
+    while (lo < hi) { const int mid = (lo + hi + 1) / 2; if (a.jobs[mid].item0 <= r) lo = mid; else hi = mid - 1; }
+    job = lo;
+    di = a.jobs[job].desc0 + (r - a.jobs[job].item0);
+    min_bits = a.jobs[job].min_bits;
+  }
+  const OrfDesc d = a.descs[di];
   if (d.flags & 2) return;
   const int st = a.status[r];
   const float usc = a.usc[r];
   if (st == 0) {
     const double bits = ((double)usc - (double)a.null_of[min(d.L, a.max_len)]) / 0.69314718055994529;
-    if (!(bits >= a.min_bits)) return;
+    if (!(bits >= min_bits)) return;
   }
   const unsigned long long slot = atomicAdd(&a.counters[0], 1ull);
   const unsigned long long off  = atomicAdd(&a.counters[1], (unsigned long long)d.L);
-  const OrfMeta m = a.meta[r];
+  if constexpr (SET) {
+    atomicAdd(&a.job_counters[2 * job], 1ull);
+    atomicAdd(&a.job_counters[2 * job + 1], (unsigned long long)d.L);
+    if (slot >= a.max_hits || off + d.L > a.max_res) return;
+    a.hit_job[slot] = job;
+  }
+  const OrfMeta m = a.meta[di];
   OrfHit h;
   h.block = m.block; h.index = m.index; h.start = m.start; h.end = m.end; h.n = d.L; h.frame = m.frame;
   h.offset = (long long)off; h.usc = usc; h.status = st;

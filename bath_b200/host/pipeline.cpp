@@ -677,6 +677,118 @@ const uint8_t *oriented(const SeqRef &sq, const BlockInfo &blk, bool complement,
   return buf.data() + pad;
 }
 
+// Stage 1 of one unit for one model, as a library search's set screen left it: ORFs per block, the survivors (sorted by block and
+// rank), and the residue buffer their offsets index (shared by the models of the screen)
+struct ScreenOut {
+  std::vector<int64_t> norfs;
+  std::vector<bathgpu_orf_hit> hits;
+  std::shared_ptr<std::vector<uint8_t>> res;
+};
+
+// The reference's blocks of a batch of sequences (src/bathsearch.c:1060-1105) for a model of C context nucleotides, and the residue
+// count as each block-strand is reached (nres: the count before the batch, then after it).  Block starts depend on W only.
+std::vector<BlockInfo> cut_blocks(const std::vector<SeqRef> &seqs, int C, const Options &opt, long long &nres)
+{
+  std::vector<BlockInfo> blocks;
+  const int W = opt.block_length;
+  for (size_t sq = 0; sq < seqs.size(); ++sq) {
+    const int64_t n = seqs[sq].n;
+    int64_t pos = 1;
+    bool first = true;
+    while (pos <= n) {
+      const int64_t ctx = first ? 0 : std::min<int64_t>(C, pos - 1);
+      BlockInfo b;
+      b.b0 = pos - ctx; b.b1 = std::min<int64_t>(n, pos + W - 1);
+      b.n = (int) (b.b1 - b.b0 + 1); b.C = (int) ctx; b.bw = (int) (b.b1 - pos + 1);
+      b.seq = (int) sq; b.coff = 0;
+      b.nres_at[0] = b.nres_at[1] = nres;
+      if (b.n >= 15) {
+        if (opt.top)    { nres += b.bw; b.nres_at[0] = nres; }
+        if (opt.bottom) { nres += b.bw; b.nres_at[1] = nres; }
+      }
+      blocks.push_back(b);
+      pos = b.b1 + 1;
+      first = false;
+    }
+  }
+  return blocks;
+}
+
+// chunks: runs of consecutive blocks; a chunk's nucleotides are the concatenation of its SEGMENTS (one per sequence it touches: first
+// block's b0 .. last block's b1), so blocks of one sequence keep their overlap and nothing is stored twice.  Sets blocks[].coff.
+struct ChunkSeg { int seq; long long from, to, off; };     // sequence coordinates from..to at chunk offset off (0-based)
+struct Chunk { int blk0, blk1; long long n; std::vector<ChunkSeg> segs; };
+std::vector<Chunk> cut_chunks(std::vector<BlockInfo> &blocks, long long target)
+{
+  std::vector<Chunk> chunks;
+  for (size_t b = 0; b < blocks.size(); ++b) {
+    const BlockInfo &blk = blocks[b];
+    const bool same_seq = !chunks.empty() && chunks.back().blk1 == (int) b && !chunks.back().segs.empty() && chunks.back().segs.back().seq == blk.seq;
+    const long long grow = same_seq ? blk.b1 - chunks.back().segs.back().to : blk.n;
+    if (chunks.empty() || chunks.back().n + grow > target) { chunks.push_back(Chunk{ (int) b, (int) b, 0, {} }); }
+    Chunk &c = chunks.back();
+    if (!c.segs.empty() && c.segs.back().seq == blk.seq && c.blk1 == (int) b) {      // the sequence's next block: extend its segment
+      blocks[b].coff = c.segs.back().off + (blk.b0 - c.segs.back().from);
+      c.n += blk.b1 - c.segs.back().to;
+      c.segs.back().to = blk.b1;
+    } else {
+      c.segs.push_back(ChunkSeg{ blk.seq, blk.b0, blk.b1, c.n });
+      blocks[b].coff = c.n;
+      c.n += blk.n;
+    }
+    c.blk1 = (int) b + 1;
+  }
+  return chunks;
+}
+
+// Chunk positions of the blocks of one model in chunks cut for a library (cut_chunks over the blocks of its largest context): every
+// block starts at or behind the segment's first nucleotide, so it lies inside the resident chunk.
+void place_blocks(std::vector<BlockInfo> &blocks, const std::vector<Chunk> &chunks)
+{
+  for (const Chunk &c : chunks)
+    for (int b = c.blk0; b < c.blk1; ++b)
+      for (const ChunkSeg &g : c.segs)
+        if (g.seq == blocks[(size_t) b].seq) { blocks[(size_t) b].coff = g.off + (blocks[(size_t) b].b0 - g.from); break; }
+}
+
+// The top strand of a chunk into slot_top, and its reverse complement made on the device in slot_bottom (bottom >= 0)
+int upload_chunk(bathhost_search *s, const bathhost_backend &BE, const std::vector<SeqRef> &seqs, const Chunk &ch, int slot_top, int slot_bottom,
+                 HostBuf &stage)
+{
+  BE_TRY(s, BE.select_slot(BE.ctx, slot_top), "bathgpu_select_slot");
+  if (ch.segs.size() == 1) {                               // the caller's buffer as it is (the byte before and the one after are not read)
+    const ChunkSeg &g = ch.segs[0];
+    BE_TRY(s, BE.upload_block(BE.ctx, seqs[(size_t) g.seq].dsq + (g.from - 1), ch.n), "bathgpu_upload_block");
+  } else if (BE.upload_block_segments) {                 // every piece crosses the link from the caller's buffer: no host copy of the chunk
+    std::vector<const uint8_t *> sp(ch.segs.size());
+    std::vector<int64_t> sn(ch.segs.size());
+    for (size_t g = 0; g < ch.segs.size(); ++g) { sp[g] = seqs[(size_t) ch.segs[g].seq].dsq + ch.segs[g].from; sn[g] = ch.segs[g].to - ch.segs[g].from + 1; }
+    BE_TRY(s, BE.upload_block_segments(BE.ctx, sp.data(), sn.data(), (int) sp.size()), "bathgpu_upload_block_segments");
+  } else {
+    uint8_t *buf = reinterpret_cast<uint8_t *>(stage.get(BE, ((size_t) ch.n + 2 + 3) / 4));
+    if (!buf) return fail(s, BATHHOST_EMEM, "host allocation failed");
+    buf[0] = 255; buf[ch.n + 1] = 255;
+    parallel_chunks(ch.segs.size(), 1, [&](size_t ga, size_t gb) {
+      for (size_t g = ga; g < gb; ++g) memcpy(buf + 1 + ch.segs[g].off, seqs[(size_t) ch.segs[g].seq].dsq + ch.segs[g].from, (size_t) (ch.segs[g].to - ch.segs[g].from + 1));
+    });
+    BE_TRY(s, BE.upload_block(BE.ctx, buf, ch.n), "bathgpu_upload_block");
+  }
+  if (slot_bottom >= 0) BE_TRY(s, BE.revcomp_slot(BE.ctx, slot_top, slot_bottom), "bathgpu_revcomp_slot");
+  return 0;
+}
+
+// the default chunk length of a batch of total nucleotides over nbe device contexts
+long long chunk_target(const bathhost_search *s, long long total)
+{
+  long long target = s->chunk_nt;
+  if (target <= 0) {
+    static const long long env_mbp = [] { const char *e = getenv("BATHHOST_CHUNK_MBP"); return e ? atoll(e) : 0LL; }();
+    target = env_mbp > 0 ? env_mbp * 1000000LL
+                         : std::max<long long>(4000000LL, std::min<long long>(128000000LL, total / (long long) s->bes.size() + 1));
+  }
+  return target;
+}
+
 struct Unit {                               // one strand of one chunk
   bool complement = false;
   int  sidx = 0, chunk = 0, be = 0, slot = 0;
@@ -687,6 +799,8 @@ struct Unit {                               // one strand of one chunk
   std::vector<int> orf_blk;                 // block of each ORF
   std::vector<int> orf_begin;               // [nblocks+1] range of each block's ORFs (index: block - blk0)
   std::vector<uint8_t> residues;
+  const uint8_t *sres = nullptr;            // the survivors' residues, indexed by bathgpu_orf_hit.offset (residues, or a library screen's buffer)
+  const ScreenOut *pre = nullptr;           // stage 1 of this unit already run by a library search's set screen (nullptr: run it here)
   std::vector<double> P_orf;
   std::vector<float>  fwdsc_orf;
   std::vector<std::vector<OrfWin>> wins_of_orf;     // windows of ORFs that reached the Forward stage, id = block-local ORF index
@@ -775,14 +889,20 @@ int filter_unit(bathhost_search *s, Unit &S, const std::vector<BlockInfo> &block
   // margin of x1 or above it, the exact tail is evaluated here for those
   const double x1 = gumbel_invsurv(opt.F1, ev[EV_MMU], ev[EV_MLAMBDA]);
   std::vector<int64_t> norfs_blk(nblk, 0);
-  int64_t nsurv = 0, nsres = 0;
-  BE_TRY(s, BE.orfs_msv_screen(BE.ctx, bdesc.data(), (int) nblk, S.complement ? 1 : 0, s->gcode, opt.min_orf, tjb_of.data(), null_of.data(),
-                                   maxlen, x1 - 0.02, norfs_blk.data(), &nsurv, &nsres), "bathgpu_orfs_msv_screen");
+  std::vector<bathgpu_orf_hit> surv;
+  if (S.pre) {
+    norfs_blk = S.pre->norfs; surv = S.pre->hits; S.sres = S.pre->res->data();
+  } else {
+    int64_t nsurv = 0, nsres = 0;
+    BE_TRY(s, BE.orfs_msv_screen(BE.ctx, bdesc.data(), (int) nblk, S.complement ? 1 : 0, s->gcode, opt.min_orf, tjb_of.data(), null_of.data(),
+                                     maxlen, x1 - 0.02, norfs_blk.data(), &nsurv, &nsres), "bathgpu_orfs_msv_screen");
+    surv.resize((size_t) nsurv);
+    S.residues.resize((size_t) nsres);
+    BE_TRY(s, BE.orfs_fetch(BE.ctx, surv.data(), S.residues.data()), "bathgpu_orfs_fetch");
+    S.sres = S.residues.data();
+  }
   for (size_t b = 0; b < nblk; ++b) S.st.n_orfs += norfs_blk[b];
-  std::vector<bathgpu_orf_hit> surv((size_t) nsurv);
-  S.residues.resize((size_t) nsres);
-  BE_TRY(s, BE.orfs_fetch(BE.ctx, surv.data(), S.residues.data()), "bathgpu_orfs_fetch");
-  const int norf = (int) nsurv;
+  const int norf = (int) surv.size();
   S.orfs.resize((size_t) norf); S.orf_blk.resize((size_t) norf);
   {
     size_t z = 0;
@@ -805,10 +925,10 @@ int filter_unit(bathhost_search *s, Unit &S, const std::vector<BlockInfo> &block
   if (norf == 0) return 0;
 
   std::vector<Orf> &orfs = S.orfs;
-  const std::vector<uint8_t> &residues = S.residues;
+  const uint8_t *residues = S.sres;
   auto orf_dsq = [&](const Orf &o, std::vector<uint8_t> &buf) {      // 1-based with sentinels, for the bias filter
     buf.assign((size_t) o.n + 2, 255);
-    memcpy(buf.data() + 1, residues.data() + o.offset, (size_t) o.n);
+    memcpy(buf.data() + 1, residues + o.offset, (size_t) o.n);
   };
   std::vector<int> live((size_t) norf);
   std::vector<float> usc((size_t) norf);
@@ -1128,9 +1248,34 @@ void add_stats(bathhost_stats &a, const bathhost_stats &b)
   a.us_decode += b.us_decode; a.us_score += b.us_score;
 }
 
+// The per-length tables of the filters (filter_unit: tjb byte cost and null1 score by ORF length), grown to the longest block
+void grow_length_tables(bathhost_search *s, const std::vector<BlockInfo> &blocks)
+{
+  const ProteinProfile &q = s->model->prot;
+  int maxlen = 1;
+  for (const BlockInfo &blk : blocks) maxlen = std::max(maxlen, blk.n / 3 + 1);
+  const size_t have = s->tjb_tab.size();
+  if (have < (size_t) maxlen + 1) {
+    s->tjb_tab.resize((size_t) maxlen + 1); s->null_tab.resize((size_t) maxlen + 1);
+    if (have == 0) { s->tjb_tab[0] = q.tjb_for_length(1); s->null_tab[0] = 0.0f; }
+    const size_t from = std::max<size_t>(have, 1);
+    parallel_chunks((size_t) maxlen + 1 - from, 4096, [&](size_t a0, size_t a1) {
+      Background lbg = s->bg;
+      for (size_t L = from + a0; L < from + a1; ++L) { s->tjb_tab[L] = q.tjb_for_length((int) L); lbg.set_length((int) L); s->null_tab[L] = lbg.null_one((int) L); }
+    });
+  }
+}
+
 // Every queued sequence, both strands.  Stage times in the statistics are summed over units (device contexts work side by side,
 // so with several of them the sum exceeds the wall time).
-int run_batch(bathhost_search *s)
+// A target already resident for the models of a library search (bathhost_library_search): the chunks cut once with the library's
+// largest context and uploaded once per device context, dealt as run_batch deals them; screen[2 c + strand] = this model's stage 1.
+struct SharedTarget {
+  std::vector<Chunk> chunks;
+  const std::vector<ScreenOut> *screen = nullptr;
+};
+
+int run_batch(bathhost_search *s, const SharedTarget *shared = nullptr)
 {
   const bathhost_model *m = s->model;
   const ProteinProfile &q = m->prot;
@@ -1144,65 +1289,19 @@ int run_batch(bathhost_search *s)
   PhaseTrace trace;
 
   // ---- the reference's blocks (src/bathsearch.c:1060-1105) and the residue count as each block-strand is reached
-  std::vector<BlockInfo> blocks;
-  {
-    const int C = q.max_length * 3, W = opt.block_length;
-    long long nres = s->st.nres;
-    for (size_t sq = 0; sq < seqs.size(); ++sq) {
-      const int64_t n = seqs[sq].n;
-      int64_t pos = 1;
-      bool first = true;
-      while (pos <= n) {
-        const int64_t ctx = first ? 0 : std::min<int64_t>(C, pos - 1);
-        BlockInfo b;
-        b.b0 = pos - ctx; b.b1 = std::min<int64_t>(n, pos + W - 1);
-        b.n = (int) (b.b1 - b.b0 + 1); b.C = (int) ctx; b.bw = (int) (b.b1 - pos + 1);
-        b.seq = (int) sq; b.coff = 0;
-        b.nres_at[0] = b.nres_at[1] = nres;
-        if (b.n >= 15) {
-          if (opt.top)    { nres += b.bw; b.nres_at[0] = nres; }
-          if (opt.bottom) { nres += b.bw; b.nres_at[1] = nres; }
-        }
-        blocks.push_back(b);
-        pos = b.b1 + 1;
-        first = false;
-      }
-    }
-    s->st.nres = nres;
-  }
+  long long nres = s->st.nres;
+  std::vector<BlockInfo> blocks = cut_blocks(seqs, q.max_length * 3, opt, nres);
+  s->st.nres = nres;
   const size_t nb = blocks.size();
 
-  // ---- chunks: runs of consecutive blocks; a chunk's nucleotides are the concatenation of its SEGMENTS (one per sequence it
-  // touches: first block's b0 .. last block's b1), so blocks of one sequence keep their overlap and nothing is stored twice
-  struct ChunkSeg { int seq; long long from, to, off; };     // sequence coordinates from..to at chunk offset off (0-based)
-  struct Chunk { int blk0, blk1; long long n; std::vector<ChunkSeg> segs; };
   std::vector<Chunk> chunks;
-  {
+  if (shared) {
+    chunks = shared->chunks;
+    place_blocks(blocks, chunks);
+  } else {
     long long total = 0;
     for (const BlockInfo &b : blocks) total += b.n;
-    long long target = s->chunk_nt;
-    if (target <= 0) {
-      static const long long env_mbp = [] { const char *e = getenv("BATHHOST_CHUNK_MBP"); return e ? atoll(e) : 0LL; }();
-      target = env_mbp > 0 ? env_mbp * 1000000LL
-                           : std::max<long long>(4000000LL, std::min<long long>(128000000LL, total / (long long) s->bes.size() + 1));
-    }
-    for (size_t b = 0; b < nb; ++b) {
-      const BlockInfo &blk = blocks[b];
-      const bool same_seq = !chunks.empty() && chunks.back().blk1 == (int) b && !chunks.back().segs.empty() && chunks.back().segs.back().seq == blk.seq;
-      const long long grow = same_seq ? blk.b1 - chunks.back().segs.back().to : blk.n;
-      if (chunks.empty() || chunks.back().n + grow > target) { chunks.push_back(Chunk{ (int) b, (int) b, 0, {} }); }
-      Chunk &c = chunks.back();
-      if (!c.segs.empty() && c.segs.back().seq == blk.seq && c.blk1 == (int) b) {      // the sequence's next block: extend its segment
-        blocks[b].coff = c.segs.back().off + (blk.b0 - c.segs.back().from);
-        c.n += blk.b1 - c.segs.back().to;
-        c.segs.back().to = blk.b1;
-      } else {
-        c.segs.push_back(ChunkSeg{ blk.seq, blk.b0, blk.b1, c.n });
-        blocks[b].coff = c.n;
-        c.n += blk.n;
-      }
-      c.blk1 = (int) b + 1;
-    }
+    chunks = cut_chunks(blocks, chunk_target(s, total));
   }
 
   // ---- units: the two strands of a chunk live in two slots of the same device context (the bottom strand is made from the top
@@ -1221,6 +1320,7 @@ int run_batch(bathhost_search *s)
       Unit &U = *units[2 * c + sidx];
       U.complement = (sidx == 1); U.sidx = sidx; U.chunk = (int) c; U.be = be; U.slot = 2 * nth + sidx;
       U.blk0 = chunks[c].blk0; U.blk1 = chunks[c].blk1; U.n_total = chunks[c].n;
+      if (shared && shared->screen) U.pre = &(*shared->screen)[2 * c + sidx];
     }
   }
   auto unit_of = [&](size_t c, int sidx) -> Unit & { return *units[2 * c + sidx]; };
@@ -1228,20 +1328,7 @@ int run_batch(bathhost_search *s)
   for (size_t c = 0; c < chunks.size(); ++c) for (int b = chunks[c].blk0; b < chunks[c].blk1; ++b) chunk_of_block[(size_t) b] = (int) c;
 
   if (s->compo_term.empty()) s->compo_term = compo_terms(m, bg);
-  {                                                           // length tables of the filters (filter_unit), up to the longest block
-    int maxlen = 1;
-    for (const BlockInfo &blk : blocks) maxlen = std::max(maxlen, blk.n / 3 + 1);
-    const size_t have = s->tjb_tab.size();
-    if (have < (size_t) maxlen + 1) {
-      s->tjb_tab.resize((size_t) maxlen + 1); s->null_tab.resize((size_t) maxlen + 1);
-      if (have == 0) { s->tjb_tab[0] = q.tjb_for_length(1); s->null_tab[0] = 0.0f; }
-      const size_t from = std::max<size_t>(have, 1);
-      parallel_chunks((size_t) maxlen + 1 - from, 4096, [&](size_t a0, size_t a1) {
-        Background lbg = bg;
-        for (size_t L = from + a0; L < from + a1; ++L) { s->tjb_tab[L] = q.tjb_for_length((int) L); lbg.set_length((int) L); s->null_tab[L] = lbg.null_one((int) L); }
-      });
-    }
-  }
+  grow_length_tables(s, blocks);
   // ---- stages 1-3 per unit, device contexts side by side: upload (top) / reverse complement on the device (bottom), ORFs, filters
   // (Letting searches that run at the same time take this phase one after the other -- it holds the throughput-bound translation + MSV
   // pass -- was measured and lost 5-9 % on one B200: 4.07-4.39 against 4.46-4.54 Gbp/s; a search's filter phase does not fill the device.)
@@ -1249,28 +1336,12 @@ int run_batch(bathhost_search *s)
     const bathhost_backend &BE = s->bes[(size_t) be];
     HostBuf stage;                                             // concatenation buffer for chunks of several sequences
     for (int c : chunks_of_be[(size_t) be]) {
-      const Chunk &ch = chunks[(size_t) c];
       Unit &T = unit_of((size_t) c, 0), &B = unit_of((size_t) c, 1);
       StageTimer tm0;
-      BE_TRY(s, BE.select_slot(BE.ctx, T.slot), "bathgpu_select_slot");
-      if (ch.segs.size() == 1) {                               // the caller's buffer as it is (the byte before and the one after are not read)
-        const ChunkSeg &g = ch.segs[0];
-        BE_TRY(s, BE.upload_block(BE.ctx, seqs[(size_t) g.seq].dsq + (g.from - 1), ch.n), "bathgpu_upload_block");
-      } else if (BE.upload_block_segments) {                 // every piece crosses the link from the caller's buffer: no host copy of the chunk
-        std::vector<const uint8_t *> sp(ch.segs.size());
-        std::vector<int64_t> sn(ch.segs.size());
-        for (size_t g = 0; g < ch.segs.size(); ++g) { sp[g] = seqs[(size_t) ch.segs[g].seq].dsq + ch.segs[g].from; sn[g] = ch.segs[g].to - ch.segs[g].from + 1; }
-        BE_TRY(s, BE.upload_block_segments(BE.ctx, sp.data(), sn.data(), (int) sp.size()), "bathgpu_upload_block_segments");
-      } else {
-        uint8_t *buf = reinterpret_cast<uint8_t *>(stage.get(BE, ((size_t) ch.n + 2 + 3) / 4));
-        if (!buf) return fail(s, BATHHOST_EMEM, "host allocation failed");
-        buf[0] = 255; buf[ch.n + 1] = 255;
-        parallel_chunks(ch.segs.size(), 1, [&](size_t ga, size_t gb) {
-          for (size_t g = ga; g < gb; ++g) memcpy(buf + 1 + ch.segs[g].off, seqs[(size_t) ch.segs[g].seq].dsq + ch.segs[g].from, (size_t) (ch.segs[g].to - ch.segs[g].from + 1));
-        });
-        BE_TRY(s, BE.upload_block(BE.ctx, buf, ch.n), "bathgpu_upload_block");
+      if (!shared) {                                           // a library search's target is resident already
+        const int st = upload_chunk(s, BE, seqs, chunks[(size_t) c], T.slot, opt.bottom ? B.slot : -1, stage);
+        if (st != 0) return st;
       }
-      if (opt.bottom) BE_TRY(s, BE.revcomp_slot(BE.ctx, T.slot, B.slot), "bathgpu_revcomp_slot");
       tm0.lap(T.st.us_upload);
       for (int sidx : active) {
         Unit &S = unit_of((size_t) c, sidx);
@@ -2029,7 +2100,7 @@ int run_batch(bathhost_search *s)
             if (rst[r] != 0) continue;                       // Forward out of range: no clusters, no envelope
             const ForwardMatrix F{ mxbuf.data() + (size_t) off[r] * (M + 1) * 4, xrbuf.data() + (size_t) off[r] * 6, M, regs[r].L };
             const SpecialOdds X{ regs[r].pmove, regs[r].ploop, xfEmh[0], xfEmh[1] };
-            const uint8_t *rres = S.residues.data() + od[mregs[r].z].offset + se.i - 2;       // rres[p] = residue p of the region
+            const uint8_t *rres = S.sres + od[mregs[r].z].offset + se.i - 2;       // rres[p] = residue p of the region
             std::vector<Segment> sp;
             std::vector<float> n2r;
             if (!sample_region_segments_protein(F, m->om3.tfv.data(), rf_amino, X, 42u, 200, se.i, rres, sp, n2r)) continue;
@@ -2086,7 +2157,7 @@ int run_batch(bathhost_search *s)
       const long long win_e = (it.w >= 0) ? win_n + S.dwin[it.w].length - 1 : o.end;
       const long long lo0 = std::min<long long>(win_n, o.start) - 1, hi0 = std::max<long long>(win_e, o.end);
       const uint8_t *wdsq = oriented(sq, binfo, S.complement, lo0, (int) (hi0 - lo0), wbuf) + (lo0 - (win_n - 1));    // wdsq[p] = block position win_n - 1 + p
-      const uint8_t *res_o = S.residues.data() + o.offset - 1;           // ORF residue p is res_o[p]
+      const uint8_t *res_o = S.sres + o.offset - 1;           // ORF residue p is res_o[p]
       const int i = envs[e].i, j = envs[e].j;
       Domain dom;
       dom.tr.assign(traces.begin() + r.trace_offset, traces.begin() + r.trace_offset + r.trace_len);
@@ -2235,6 +2306,33 @@ int run_batch(bathhost_search *s)
   return 0;
 }
 
+bathgpu_filter_params filter_params(const bathhost_search *s)
+{
+  const ProteinProfile &q = s->model->prot;
+  bathgpu_filter_params fp;
+  fp.M = s->model->hmm.M; fp.tbm_b = q.tbm_b; fp.tec_b = q.tec_b; fp.base_b = q.base_b; fp.bias_b = q.bias_b; fp.scale_b = q.scale_b;
+  fp.base_w = q.base_w; fp.ddbound_w = q.ddbound_w; fp.xw_E_move = q.xw_E_move; fp.xw_E_loop = q.xw_E_loop; fp.scale_w = q.scale_w;
+  fp.cpu_lanes_u8 = s->opt.lanes_u8; fp.cpu_lanes_i16 = s->opt.lanes_i16;
+  return fp;
+}
+
+// device images: the three profiles of a query, replicated on every device context
+int load_images(bathhost_search *s)
+{
+  const bathhost_model *m = s->model;
+  const int M = m->hmm.M;
+  const bathgpu_filter_params fp = filter_params(s);
+  const ProteinProfile &q = m->prot;
+  return for_each_backend(s, [&](int k) -> int {
+    const bathhost_backend &BE = s->bes[(size_t) k];
+    int rc;
+    if ((rc = BE.load_fs_profile(BE.ctx, 3, M, m->om3.nrows, m->om3.rfv.data(), m->om3.tfv.data())) != 0 ||
+        (rc = BE.load_fs_profile(BE.ctx, 5, M, m->om5.nrows, m->om5.rfv.data(), m->om5.tfv.data())) != 0 ||
+        (rc = BE.load_filter_profile(BE.ctx, &fp, q.rbv.data(), q.rwv.data(), q.twv.data())) != 0) return rc;
+    return 0;
+  });
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------
@@ -2266,21 +2364,7 @@ extern "C" int bathhost_search_create_multi(const bathhost_model *m, const bathh
   s->compo.assign(m->hmm.compo, m->hmm.compo + kK);
   s->bg.set_filter(m->hmm.M, s->compo.data());           // p7_pli_NewModel -> p7_bg_SetFilter(bg, om->M, om->compo)
 
-  // device images: the three profiles of a query, replicated on every device context
-  const int M = m->hmm.M;
-  bathgpu_filter_params fp;
-  const ProteinProfile &q = m->prot;
-  fp.M = M; fp.tbm_b = q.tbm_b; fp.tec_b = q.tec_b; fp.base_b = q.base_b; fp.bias_b = q.bias_b; fp.scale_b = q.scale_b;
-  fp.base_w = q.base_w; fp.ddbound_w = q.ddbound_w; fp.xw_E_move = q.xw_E_move; fp.xw_E_loop = q.xw_E_loop; fp.scale_w = q.scale_w;
-  fp.cpu_lanes_u8 = s->opt.lanes_u8; fp.cpu_lanes_i16 = s->opt.lanes_i16;
-  const int st = for_each_backend(s, [&](int k) -> int {
-    const bathhost_backend &BE = s->bes[(size_t) k];
-    int rc;
-    if ((rc = BE.load_fs_profile(BE.ctx, 3, M, m->om3.nrows, m->om3.rfv.data(), m->om3.tfv.data())) != 0 ||
-        (rc = BE.load_fs_profile(BE.ctx, 5, M, m->om5.nrows, m->om5.rfv.data(), m->om5.tfv.data())) != 0 ||
-        (rc = BE.load_filter_profile(BE.ctx, &fp, q.rbv.data(), q.rwv.data(), q.twv.data())) != 0) return rc;
-    return 0;
-  });
+  const int st = load_images(s);
   if (st != 0) { delete s; return st; }
   *ret = s;
   return BATHHOST_OK;
@@ -2741,4 +2825,203 @@ extern "C" int bathhost_search_get_stats(const bathhost_search *s, bathhost_stat
   if (!s || !st) return BATHHOST_EINVAL;
   *st = s->st;
   return BATHHOST_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// A profile library against one target (bathhost.h): one search per model over shared device contexts and a target made resident once.
+struct bathhost_library_search {
+  std::vector<bathhost_search *> s;
+  std::vector<SeqRef> queue;
+  std::string err;
+  ~bathhost_library_search() { for (bathhost_search *x : s) delete x; }
+};
+
+namespace {
+
+thread_local std::string g_library_err;
+
+// The ORF screen of models i0 .. i0+g-1 over every unit of the resident target, one set call per unit: out[k][2 c + strand]
+int screen_group(bathhost_library_search *ls, const std::vector<SeqRef> &seqs, const std::vector<Chunk> &chunks, const std::vector<BlockInfo> &lib_blocks,
+                 size_t i0, size_t g, std::vector<std::vector<ScreenOut>> &out)
+{
+  bathhost_search *s0 = ls->s[i0];
+  const Options &opt = s0->opt;
+  std::vector<std::vector<BlockInfo>> mb(g);
+  std::vector<double> min_bits(g);
+  std::vector<bathgpu_filter_params> prm(g);
+  std::vector<const uint8_t *> rbv(g);
+  for (size_t k = 0; k < g; ++k) {
+    bathhost_search *s = ls->s[i0 + k];
+    long long nres = s->st.nres;
+    mb[k] = cut_blocks(seqs, s->model->prot.max_length * 3, opt, nres);
+    place_blocks(mb[k], chunks);
+    grow_length_tables(s, lib_blocks);                      // the library's blocks are the longest any model has
+    const float *ev = s->model->hmm.evparam;
+    min_bits[k] = gumbel_invsurv(s->opt.F1, ev[EV_MMU], ev[EV_MLAMBDA]) - 0.02;      // as filter_unit asks of bathgpu_orfs_msv_screen
+    prm[k] = filter_params(s); rbv[k] = s->model->prot.rbv.data();
+  }
+  std::vector<int> active;
+  if (opt.top)    active.push_back(0);
+  if (opt.bottom) active.push_back(1);
+  out.assign(g, std::vector<ScreenOut>(chunks.size() * 2));
+  return for_each_backend(s0, [&](int be) -> int {
+    bathhost_search *s = s0;
+    const bathhost_backend &BE = s0->bes[(size_t) be];
+    BE_TRY(s, BE.load_filter_profile_set(BE.ctx, (int) g, prm.data(), rbv.data()), "bathgpu_load_filter_profile_set");
+    int nth = 0;
+    for (size_t c = (size_t) be; c < chunks.size(); c += s0->bes.size(), ++nth) {
+      const Chunk &ch = chunks[c];
+      const size_t nblk = (size_t) (ch.blk1 - ch.blk0);
+      for (int sidx : active) {
+        std::vector<std::vector<bathgpu_block>> bd(g, std::vector<bathgpu_block>(nblk));
+        std::vector<bathgpu_screen_job> jobs(g);
+        int maxlen = 1;
+        for (size_t k = 0; k < g; ++k) {
+          for (size_t b = 0; b < nblk; ++b) {
+            const BlockInfo &blk = mb[k][(size_t) ch.blk0 + b];
+            bd[k][b].goff = sidx ? ch.n - (blk.coff + blk.n) : blk.coff; bd[k][b].n = (blk.n >= 15) ? blk.n : 0; bd[k][b].C = blk.C;
+            maxlen = std::max(maxlen, blk.n / 3 + 1);
+          }
+          jobs[k] = bathgpu_screen_job{ (int32_t) k, (int32_t) nblk, bd[k].data(), min_bits[k] };
+        }
+        std::vector<int64_t> norfs(g * nblk), nh(g), nr(g);
+        BE_TRY(s, BE.select_slot(BE.ctx, 2 * nth + sidx), "bathgpu_select_slot");
+        BE_TRY(s, BE.orfs_msv_screen_set(BE.ctx, jobs.data(), (int) g, sidx, s0->gcode, opt.min_orf, s0->tjb_tab.data(), s0->null_tab.data(), maxlen,
+                                         norfs.data(), nh.data(), nr.data()), "bathgpu_orfs_msv_screen_set");
+        int64_t tot_h = 0, tot_r = 0;
+        for (size_t k = 0; k < g; ++k) { tot_h += nh[k]; tot_r += nr[k]; }
+        std::vector<bathgpu_orf_hit> hits((size_t) tot_h);
+        auto res = std::make_shared<std::vector<uint8_t>>((size_t) tot_r);
+        BE_TRY(s, BE.orfs_fetch_set(BE.ctx, hits.data(), res->data()), "bathgpu_orfs_fetch_set");
+        size_t z = 0;
+        for (size_t k = 0; k < g; ++k) {
+          ScreenOut &o = out[k][2 * c + (size_t) sidx];
+          o.norfs.assign(norfs.begin() + (long) (k * nblk), norfs.begin() + (long) ((k + 1) * nblk));
+          o.hits.assign(hits.begin() + (long) z, hits.begin() + (long) (z + (size_t) nh[k]));
+          o.res = res;
+          z += (size_t) nh[k];
+        }
+      }
+    }
+    return 0;
+  });
+}
+
+int library_fail(bathhost_library_search *ls, int code, const std::string &msg) { ls->err = msg; return code; }
+
+int library_run(bathhost_library_search *ls)
+{
+  std::vector<SeqRef> seqs;
+  seqs.swap(ls->queue);
+  if (seqs.empty()) return 0;
+  bathhost_search *s0 = ls->s[0];
+  const Options &opt = s0->opt;
+  // chunks cut once, at block starts, each resident range reaching back by the largest context of the library
+  int Cmax = 0;
+  for (bathhost_search *s : ls->s) Cmax = std::max(Cmax, s->model->prot.max_length * 3);
+  long long nres_unused = 0, total = 0;
+  std::vector<BlockInfo> lib_blocks = cut_blocks(seqs, Cmax, opt, nres_unused);
+  for (const BlockInfo &b : lib_blocks) total += b.n;
+  SharedTarget shared;
+  shared.chunks = cut_chunks(lib_blocks, chunk_target(s0, total));
+  // each chunk uploaded (and its bottom strand made) once, on the context and in the slots run_batch deals it to
+  int rc = for_each_backend(s0, [&](int be) -> int {
+    HostBuf stage;
+    int nth = 0;
+    for (size_t c = (size_t) be; c < shared.chunks.size(); c += s0->bes.size(), ++nth) {
+      const int st = upload_chunk(s0, s0->bes[(size_t) be], seqs, shared.chunks[c], 2 * nth, opt.bottom ? 2 * nth + 1 : -1, stage);
+      if (st != 0) return st;
+    }
+    return 0;
+  });
+  if (rc != 0) return library_fail(ls, rc, s0->err);
+  auto run_model = [&](size_t i, const std::vector<ScreenOut> *screen) -> int {
+    bathhost_search *s = ls->s[i];
+    int st = load_images(s);
+    if (st != 0) return library_fail(ls, st, "model " + std::to_string(i) + ": loading its profiles failed: " +
+                                             (s->bes[0].last_error ? s->bes[0].last_error(s->bes[0].ctx) : "?"));
+    for (size_t k = 0; k < seqs.size(); ++k) {
+      SeqRef r;
+      r.name = seqs[k].name; r.dsq = seqs[k].dsq; r.n = seqs[k].n; r.seqidx = s->nseqs + (int64_t) k;
+      s->queue.push_back(std::move(r));
+    }
+    s->finished = false;
+    SharedTarget sh;
+    sh.chunks = shared.chunks; sh.screen = screen;
+    st = run_batch(s, &sh);
+    return st != 0 ? library_fail(ls, st, "model " + std::to_string(i) + ": " + s->err) : 0;
+  };
+  bool set_screen = true;
+  for (const bathhost_backend &BE : s0->bes) set_screen = set_screen && BE.load_filter_profile_set && BE.orfs_msv_screen_set && BE.orfs_fetch_set;
+  const size_t n = ls->s.size();
+  if (!set_screen) {
+    for (size_t i = 0; i < n; ++i) if ((rc = run_model(i, nullptr)) != 0) return rc;
+    return 0;
+  }
+  size_t group = std::min<size_t>(n, BATHGPU_SCREEN_SET_MAX_JOBS);
+  for (size_t i0 = 0; i0 < n;) {
+    const size_t g = std::min(group, n - i0);
+    std::vector<std::vector<ScreenOut>> screens;
+    rc = screen_group(ls, seqs, shared.chunks, lib_blocks, i0, g, screens);
+    if (rc == BATHHOST_EMEM && g > 1) { group = g / 2; continue; }       // the device cannot hold this many at once: half the group
+    if (rc != 0) return library_fail(ls, rc, ls->s[i0]->err);
+    for (size_t k = 0; k < g; ++k) if ((rc = run_model(i0 + k, &screens[k])) != 0) return rc;
+    i0 += g;
+  }
+  return 0;
+}
+
+}  // namespace
+
+extern "C" int bathhost_search_create_library(const bathhost_model *const *models, int n, const bathhost_backend *be, int nbackends,
+                                              const bathhost_options *opt, bathhost_library_search **ret)
+{
+  g_library_err.clear();
+  if (!ret) return BATHHOST_EINVAL;
+  *ret = nullptr;
+  if (!models || n < 1 || !be || nbackends < 1) { g_library_err = "bad arguments to bathhost_search_create_library"; return BATHHOST_EINVAL; }
+  std::unique_ptr<bathhost_library_search> ls(new (std::nothrow) bathhost_library_search());
+  if (!ls) return BATHHOST_EMEM;
+  for (int i = 0; i < n; ++i) {
+    bathhost_search *s = nullptr;
+    const int st = models[i] ? bathhost_search_create_multi(models[i], be, nbackends, opt, &s) : BATHHOST_EINVAL;
+    if (st != BATHHOST_OK) {
+      bathhost_model_info info;
+      const bool named = models[i] && bathhost_model_get_info(models[i], &info) == BATHHOST_OK;
+      g_library_err = "model " + std::to_string(i) + (named ? std::string(" (") + info.name + ")" : std::string()) + " refused: " +
+                      (be[0].last_error ? be[0].last_error(be[0].ctx) : "status " + std::to_string(st));
+      return st;
+    }
+    ls->s.push_back(s);
+  }
+  *ret = ls.release();
+  return BATHHOST_OK;
+}
+
+extern "C" void bathhost_library_search_destroy(bathhost_library_search *ls) { delete ls; }
+extern "C" const char *bathhost_library_search_last_error(const bathhost_library_search *ls) { return ls ? ls->err.c_str() : g_library_err.c_str(); }
+
+extern "C" int bathhost_library_search_queue(bathhost_library_search *ls, const char *name, const uint8_t *dsq, int64_t n)
+{
+  if (!ls || !dsq || n < 1) return BATHHOST_EINVAL;
+  SeqRef r;
+  r.name = name ? name : ""; r.dsq = dsq; r.n = n;
+  ls->queue.push_back(std::move(r));
+  return BATHHOST_OK;
+}
+
+extern "C" int bathhost_library_search_run(bathhost_library_search *ls) { return ls ? library_run(ls) : BATHHOST_EINVAL; }
+
+extern "C" int bathhost_library_search_finish(bathhost_library_search *ls)
+{
+  if (!ls) return BATHHOST_EINVAL;
+  int st = library_run(ls);
+  for (size_t i = 0; st == BATHHOST_OK && i < ls->s.size(); ++i)
+    if ((st = bathhost_search_finish(ls->s[i])) != BATHHOST_OK) ls->err = "model " + std::to_string(i) + ": " + ls->s[i]->err;
+  return st;
+}
+
+extern "C" bathhost_search *bathhost_library_search_get(bathhost_library_search *ls, int i)
+{
+  return (ls && i >= 0 && (size_t) i < ls->s.size()) ? ls->s[(size_t) i] : nullptr;
 }

@@ -19,6 +19,8 @@ EXPORTS = [
     "bathhost_cluster_region_segments_protein", "bathhost_search_format_tblout",
     "bathhost_calibrate", "bathhost_model_lambda", "bathhost_search_format_report", "bathhost_search_format_output", "bathhost_search_format_fstblout",
     "bathhost_convert", "bathhost_convert_last_error",
+    "bathhost_search_create_library", "bathhost_library_search_destroy", "bathhost_library_search_last_error", "bathhost_library_search_queue",
+    "bathhost_library_search_run", "bathhost_library_search_finish", "bathhost_library_search_get",
 ]
 
 
@@ -38,9 +40,9 @@ class Backend(C.Structure):
     """bathhost_backend: the device library as a table of function pointers (include/bathhost.h)"""
     _names = ["last_error", "load_fs_profile", "load_filter_profile", "select_slot", "upload_block", "upload_orfs", "msv_orfs", "ssv_windows",
               "vit_orfs", "fwd_orfs", "fs_fwd_windows", "fs_fwd_bck_xrows", "fs_bck_decode", "fs_domains", "fs_forward_matrices", "orf_fwd_bck_xrows", "orf_domains", "orfs_msv_screen", "orfs_fetch", "revcomp_slot", "host_alloc", "host_free", "bias_forward", "orf_forward_matrices", "upload_block_segments"]
-    # the optional pair at the end of the table: left NULL by a table that fills _names only (bathhost_convert then calibrates
-    # model by model)
-    _set_names = ["load_fs_profile_set", "fs_set_scores"]
+    # the optional entries at the end of the table: left NULL by a table that fills _names only (bathhost_convert then calibrates
+    # model by model; a library search screens model by model)
+    _set_names = ["load_fs_profile_set", "fs_set_scores", "load_filter_profile_set", "orfs_msv_screen_set", "orfs_fetch_set"]
     _fields_ = [("ctx", C.c_void_p)] + [(n, C.c_void_p) for n in _names + _set_names]
 
 
@@ -155,6 +157,19 @@ def load():
     L.bathhost_convert.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_float, C.c_uint32, C.POINTER(Backend), C.POINTER(C.c_int)]
     L.bathhost_convert_last_error.restype = C.c_char_p
     L.bathhost_convert_last_error.argtypes = []
+    L.bathhost_search_create_library.restype = C.c_int
+    L.bathhost_search_create_library.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Backend), C.c_int, C.POINTER(Options), C.POINTER(vp)]
+    L.bathhost_library_search_destroy.restype = None
+    L.bathhost_library_search_destroy.argtypes = [vp]
+    L.bathhost_library_search_last_error.restype = C.c_char_p
+    L.bathhost_library_search_last_error.argtypes = [vp]
+    L.bathhost_library_search_queue.restype = C.c_int
+    L.bathhost_library_search_queue.argtypes = [vp, C.c_char_p, u8p, C.c_int64]
+    for name in ("bathhost_library_search_run", "bathhost_library_search_finish"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = [vp]
+    L.bathhost_library_search_get.restype = vp
+    L.bathhost_library_search_get.argtypes = [vp, C.c_int]
     L.bathhost_length_model.restype = None
     L.bathhost_length_model.argtypes = [C.c_int, C.c_float, fp, fp]
     _lib = L
@@ -441,6 +456,99 @@ class Search:
         s = Stats()
         self.lib.bathhost_search_get_stats(self.h, C.byref(s))
         return {n: getattr(s, n) for n, _ in Stats._fields_}
+
+
+class LibraryError(RuntimeError):
+    def __init__(self, code, msg):
+        super().__init__(f"bathhost library search: status {code}: {msg}")
+        self.code = code
+
+
+class _LibraryMember(Search):
+    """Model i's search of a LibrarySearch: every reader of Search over a handle the library search owns."""
+
+    def __init__(self, lib, h, model):
+        self.lib, self.h, self.model, self._keep = lib, h, model, []
+
+    def close(self):
+        self.h = None
+
+
+class LibrarySearch:
+    """Every profile of a library against one target (bathsearch with a query file, src/bathsearch.c:737): the target is uploaded and
+    translated once per device context, the ORF screen of many profiles runs in one device call, and each model's results are those
+    of a Search of that model alone (see bathhost_search_create_library in include/bathhost.h).  path_or_models: a .bhmm path (every
+    model, in file order) or a list of QueryModel; gpu_ctx / backend / options as Search takes them."""
+
+    def __init__(self, path_or_models, gpu_ctx=None, backend=None, **options):
+        self.lib = load()
+        if isinstance(path_or_models, (str, bytes, os.PathLike)):
+            n = self.lib.bathhost_model_count(os.fsencode(path_or_models))
+            if n < 1:
+                raise IOError(f"no models in {path_or_models}")
+            self.models = [QueryModel(path_or_models, i) for i in range(n)]
+        else:
+            self.models = list(path_or_models)
+        self.gpu_ctx = gpu_ctx
+        if backend is None:
+            if gpu_ctx is None:
+                raise ValueError("a device context is required: the product has no CPU path")
+            ctxs = gpu_ctx if isinstance(gpu_ctx, (list, tuple)) else [gpu_ctx]
+            backend = [backend_from(c.lib, c.h) for c in ctxs]
+        backends = list(backend) if isinstance(backend, (list, tuple)) else [backend]
+        self.backend = (Backend * len(backends))(*backends)
+        self._keep = []
+        opt = Options(**options)
+        arr = (C.c_void_p * len(self.models))(*[m.h for m in self.models])
+        h = C.c_void_p()
+        st = self.lib.bathhost_search_create_library(arr, len(self.models), self.backend, len(backends), C.byref(opt), C.byref(h))
+        if st != OK:
+            raise LibraryError(st, self.lib.bathhost_library_search_last_error(None).decode())
+        self.h = h
+        self.searches = [_LibraryMember(self.lib, self.lib.bathhost_library_search_get(h, i), m) for i, m in enumerate(self.models)]
+
+    def close(self):
+        if getattr(self, "h", None):
+            for s in self.searches:
+                s.close()
+            self.lib.bathhost_library_search_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _check(self, st, what):
+        if st != OK:
+            raise LibraryError(st, f"{what}: {self.lib.bathhost_library_search_last_error(self.h).decode()}")
+
+    def queue_sequence(self, name, dsq):
+        """one more target for the next run() or finish()"""
+        dsq = np.ascontiguousarray(dsq, np.uint8)
+        self._keep.append(dsq)
+        self._check(self.lib.bathhost_library_search_queue(self.h, name.encode(), dsq.ctypes.data_as(C.POINTER(C.c_uint8)), len(dsq) - 2),
+                    "queue")
+
+    def run(self):
+        st = self.lib.bathhost_library_search_run(self.h)
+        self._keep = []
+        self._check(st, "run")
+
+    def finish(self):
+        """everything still queued is searched, then every model's search is finished (bathhost_search_finish)"""
+        st = self.lib.bathhost_library_search_finish(self.h)
+        self._keep = []
+        self._check(st, "finish")
+
+    def tblout(self):
+        """the one --tblout table bathsearch writes for a query file: the header once, then each model's hit lines in file order"""
+        return "".join(s.tblout(header=(i == 0)) for i, s in enumerate(self.searches))
+
+    def output(self, textw=150):
+        """each model's section of bathsearch's output, each followed by the "//" line that ends it"""
+        return "".join(s.output(textw) + "//\n" for s in self.searches)
 
 
 def sample_region_segments(mx, xrows, tfv, odds, ireg, seed=42, nsamples=200):

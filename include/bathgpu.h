@@ -306,6 +306,41 @@ int bathgpu_orfs_fetch(bathgpu_ctx *ctx, bathgpu_orf_hit *hits, uint8_t *residue
  * MSV kernel scored (its DP cells = residues x M). */
 int bathgpu_orfs_stage_breakdown(bathgpu_ctx *ctx, float ms[5], int64_t *norfs, int64_t *residues_scored);
 
+/* ---- f1 over a profile set: the screen of many profiles against one resident strand (bathsearch's query loop, src/bathsearch.c:737) --- */
+/* bathgpu_load_filter_profile_set: the MSV byte tables of n profiles (prm[p], rbv[p] as bathgpu_load_filter_profile takes them; the
+ * Viterbi tables are not needed) in one device block.  Held beside the context's single filter profile, which stays untouched; a new
+ * set replaces the old one.  EMEM when the device cannot hold the set (the caller then loads fewer profiles at a time). */
+int bathgpu_load_filter_profile_set(bathgpu_ctx *ctx, int n, const bathgpu_filter_params *prm, const uint8_t *const *rbv);
+
+/* One job of a set screen: profile `profile` of the set over the blocks blocks[0 .. nblocks-1] of the selected slot's strand, with its
+ * own min_bits.  Each job has its blocks because the overlap context C = 3 MAXL depends on the model. */
+typedef struct {
+  int32_t profile;
+  int32_t nblocks;
+  const bathgpu_block *blocks;
+  double  min_bits;
+} bathgpu_screen_job;
+
+/* Device budget of one bathgpu_orfs_msv_screen_set call: at most BATHGPU_SCREEN_SET_MAX_JOBS jobs (EINVAL beyond), and at most
+ * BATHGPU_SCREEN_SET_MAX_ITEMS (job, ORF) pairs -- 8 bytes of MSV score and status each, 1 GiB -- found after the ORF count
+ * (EMEM beyond: the caller splits its jobs).  ORF descriptors are stored once per distinct block layout, not per job. */
+#define BATHGPU_SCREEN_SET_MAX_JOBS  64
+#define BATHGPU_SCREEN_SET_MAX_ITEMS ((int64_t) 1 << 27)
+
+/* bathgpu_orfs_msv_screen for every job in one call: codon classes once, the ORF count and emit passes once per distinct block layout,
+ * MSV in one launch per table width over all (job, ORF) pairs, and the F1 screen + residue gather in one launch.  tjb_of / null_of depend
+ * on the ORF length only and serve every job.  Outputs: norfs_per_block, the jobs' block counts concatenated in job order; nhits[j],
+ * nres[j] per job.  For every job the ORF counts, survivors, ranks, coordinates, usc, status and residues are those
+ * bathgpu_orfs_msv_screen returns with that profile loaded alone and the same blocks.  All survivors' residues stay in the slot's
+ * residue buffer, so each survivor's offset is valid there for the later stage calls of its job. */
+int bathgpu_orfs_msv_screen_set(bathgpu_ctx *ctx, const bathgpu_screen_job *jobs, int njobs, int complement, const uint8_t gcode[64],
+                                int min_len, const uint8_t *tjb_of, const float *null_of, int max_len,
+                                int64_t *norfs_per_block, int64_t *nhits, int64_t *nres);
+/* The survivors of the last set screen: those of job 0 first, then job 1, ..., each job's sorted by block and rank as
+ * bathgpu_orfs_fetch sorts them (sum of nhits[] entries); residues = the slot's whole residue buffer (sum of nres[] bytes), which
+ * each survivor's offset indexes.  bathgpu_orfs_stage_breakdown reports the kernel groups of the set call as of a single one. */
+int bathgpu_orfs_fetch_set(bathgpu_ctx *ctx, bathgpu_orf_hit *hits, uint8_t *residues);
+
 /* ---- a5: the bias-composition filter ---------------------------------------------------------------------------------- */
 /* esl_hmm_Forward over the 2-state filter HMM of p7_bg_SetFilter (src/p7_bg.c:449-471), batched: what p7_bg_FilterScore computes
  * for an ORF (:491-500; call sites src/p7_pipeline.c:1659, :1697) and p7_bg_fs_FilterScore for each of the three reading frames of a

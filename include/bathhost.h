@@ -141,6 +141,12 @@ typedef struct {
    * bathgpu_load_fs_profile_set and bathgpu_fs_set_scores, the frameshift Forward parsers over many profiles at once */
   int (*load_fs_profile_set)(void *ctx, int which, int n, const int *M, const int *nrows, const float *const *rfv, const float *const *tfv);
   int (*fs_set_scores)(void *ctx, int which, const void *wins, int n, const float *xfE, float *fwdsc, int32_t *status);
+  /* optional trio (all NULL: a library search screens its models one at a time through orfs_msv_screen, on the target it made resident
+   * once): bathgpu_load_filter_profile_set, bathgpu_orfs_msv_screen_set and bathgpu_orfs_fetch_set, the ORF screen of many profiles */
+  int (*load_filter_profile_set)(void *ctx, int n, const void *prm, const uint8_t *const *rbv);
+  int (*orfs_msv_screen_set)(void *ctx, const void *jobs, int njobs, int complement, const uint8_t gcode[64], int min_len,
+                             const uint8_t *tjb_of, const float *null_of, int max_len, int64_t *norfs_per_block, int64_t *nhits, int64_t *nres);
+  int (*orfs_fetch_set)(void *ctx, void *hits, uint8_t *residues);
 } bathhost_backend;
 
 /* 0 / unset fields take bathsearch's defaults (src/p7_pipeline.c:145-214; src/bathsearch.c:94) */
@@ -222,6 +228,28 @@ int  bathhost_search_finish(bathhost_search *s);
  * returns the hit list it returns alone, and one search's serial host phases run under the others' device stages.  First non-zero
  * status, BATHHOST_EINVAL for a null or repeated search or two searches over the same device context. */
 int  bathhost_search_finish_many(bathhost_search *const *searches, int n);
+/* ---- a profile library against one target (bathsearch with a query file of several profiles, src/bathsearch.c:737) ------------------
+ * One search per model, over the same device contexts, fed the same target: each model's hit list, statistics and formatted output
+ * are those of a bathhost_search_create_multi search of that model alone (bathhost_library_search_get returns model i's search, which
+ * every bathhost_search_* reader and formatter takes).  What the models share: the target's chunks are cut once (cut at block starts,
+ * which do not depend on the model; each resident range reaches back by the largest context of the library), uploaded and
+ * reverse-complemented once per device context; and with the backend's set trio, the ORF screen of up to BATHGPU_SCREEN_SET_MAX_JOBS
+ * models per unit runs as one device call (a group the device cannot hold is halved).  The models of a group then run the rest of
+ * the pipeline one after the other.  A model a device context refuses (e.g. longer than it accepts) fails the creation with its status
+ * and a message naming the model's index; nothing is searched.  bathhost_library_search_last_error(NULL) is this thread's last
+ * creation error. */
+typedef struct bathhost_library_search bathhost_library_search;
+int  bathhost_search_create_library(const bathhost_model *const *models, int n, const bathhost_backend *be, int nbackends,
+                                    const bathhost_options *opt, bathhost_library_search **ret);
+void bathhost_library_search_destroy(bathhost_library_search *ls);
+const char *bathhost_library_search_last_error(const bathhost_library_search *ls);
+/* as bathhost_search_queue / _run / _finish, for every model of the library */
+int  bathhost_library_search_queue(bathhost_library_search *ls, const char *name, const uint8_t *dsq, int64_t n);
+int  bathhost_library_search_run(bathhost_library_search *ls);
+int  bathhost_library_search_finish(bathhost_library_search *ls);
+/* model i's search (owned by the library search), NULL if i is out of range */
+bathhost_search *bathhost_library_search_get(bathhost_library_search *ls, int i);
+
 int  bathhost_search_nhits(const bathhost_search *s);
 int  bathhost_search_get_hit(const bathhost_search *s, int idx, bathhost_hit *hit);
 int  bathhost_search_get_stats(const bathhost_search *s, bathhost_stats *st);
